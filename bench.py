@@ -75,7 +75,16 @@ def parse():
     ap.add_argument("--no-traffic", action="store_true", help="skip the ncu child that measures roofline.traffic")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step handed its caller to DIR/<name>.npy "
+                         "(float32 / float64, at most 64 MB in all: larger arrays keep a fixed, seeded sample of their "
+                         "rows, listed in DIR/<name>_rows.npy); rank 0 only")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "graft":
+        ap.error("--dump-outputs writes the outputs of the CUDA path (--impl graft)")
+    return args
 
 
 def lanes_of(args):
@@ -148,14 +157,16 @@ def cpu_port_run(args, n_envs, prime, timed_steps, warmup_steps, n_threads, seed
         per_step.append(time.perf_counter() - t0)
         agent_steps += len(o["reward"])
     elapsed = float(sum(per_step))
-    return {"agent_steps": agent_steps, "elapsed": elapsed, "n_envs": n_envs}
+    return {"agent_steps": agent_steps, "elapsed": elapsed, "n_envs": n_envs, "prime": prime, "threads": n_threads,
+            "port": "oracle/scene_oracle.c (C port of the reference scene, persistent thread pool)"}
 
 
 def cpu_port_run_lane4(args, n_envs, prime, timed_steps, warmup_steps, seed):
-    """lane_num=4 / 8: the pure-Python oracles (oracle/scene4_oracle.py, scene8_oracle.py), one thread, a few intersections."""
+    """lane_num=4 / 8: the pure-Python oracles (oracle/scene4_oracle.py, scene8_oracle.py), one thread, a few intersections
+    (the sample of intersections and the priming are bounded; every one of the `timed_steps` ticks is timed)."""
     from oracle.scene4_oracle import Scene4Oracle
     from oracle.scene8_oracle import Scene8Oracle
-    n_envs, prime, timed_steps = min(n_envs, 4), min(prime, 200), min(timed_steps, 50)
+    n_envs, prime = min(n_envs, 4), min(prime, 200)
     tabs = make_tables(args, n_envs, seed, (prime + warmup_steps + timed_steps) * 0.1 + 30.0)
     if args.workload == "lane4":
         orcs = [Scene4Oracle(vm=VM) for _ in range(n_envs)]
@@ -177,7 +188,8 @@ def cpu_port_run_lane4(args, n_envs, prime, timed_steps, warmup_steps, seed):
             if t >= prime + warmup_steps:
                 elapsed += time.perf_counter() - t0
                 agent_steps += len(out["ids"])
-    return {"agent_steps": agent_steps, "elapsed": elapsed, "n_envs": n_envs}
+    return {"agent_steps": agent_steps, "elapsed": elapsed, "n_envs": n_envs, "prime": prime, "threads": 1,
+            "port": "oracle/scene%d_oracle.py (Python port of the reference scene with lane_num=%d)" % ((lanes_of(args),) * 2)}
 
 
 def reference_arm(args, rank):
@@ -188,16 +200,16 @@ def reference_arm(args, rank):
     r = cpu_port_run(args, n_envs, PRIME_TICKS, args.steps, args.warmup, cores)
     value = r["agent_steps"] / r["elapsed"]
     sample = ("each step = one tick of %d intersections (bounded sample of the workload) on %d host threads, "
-              "after %d priming ticks" % (n_envs, cores, PRIME_TICKS))
+              "after %d priming ticks" % (r["n_envs"], r["threads"], r["prime"]))
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus,
         "steps": args.steps, "warmup": args.warmup, "ms_per_step": 1e3 * r["elapsed"] / args.steps,
         "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
-        "config": {"workload": workload_name(args), "reference_sample_envs": n_envs,
-                   "same_config": n_envs == args.envs,
+        "config": {"workload": workload_name(args), "reference_sample_envs": r["n_envs"],
+                   "same_config": r["n_envs"] == args.envs,
                    "note": "agent-steps/s is a per-agent-step rate: the sample has the workload's density, actions and "
                            "occupancy but fewer intersections per step than the CUDA arm"},
-        "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "port", "sample": sample,
+        "cpu_baseline": {"value": value, "unit": UNIT, "cores": r["threads"], "kind": "port", "sample": sample,
                          "python_reference": python_reference_rate(args)},
         "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
         "gpu_launches": 0,
@@ -387,6 +399,49 @@ class ClockSampler(threading.Thread):
 
 
 # ---------------------------------------------------------------------------------------------
+# --dump-outputs: what the last timed tick computed, for comparing two builds output for output
+# ---------------------------------------------------------------------------------------------
+DUMP_BYTES = 64 * 10**6          # decimal MB; sample_outputs leaves 1 MiB of it for the .npy headers
+
+
+def last_outputs(scene, out, actions, folder):
+    """name -> host array of what the last timed tick handed its caller: the step's outputs (``StepOutputs``: the
+    reference's 9-tuple), in a rollout the policy's actions, in a training rollout the replay records its push
+    appended.  None when the scene overflowed: that run is discarded and repeated in the next capacity class."""
+    import torch
+    if scene.stats()["overflow"]:
+        return None
+    n = out.n_agents
+    got = {f: getattr(out, f) for f in ("agent_offset", "env_collisions", "env_lock", "env_removed")}
+    got.update({f: getattr(out, f)[:n] for f in ("obs", "reward", "ids", "cpv", "status", "jerk_sum")})
+    if actions is not None:
+        got["actions"] = actions
+    if folder is not None:
+        c = folder.counters()
+        pos = torch.arange(c["num_experiences"] - c["last_added"], c["num_experiences"], device=out.obs.device)
+        got.update({"replay_" + k: v[pos % folder.capacity] for k, v in folder.arrays().items()})
+    return sample_outputs({k: v.cpu().numpy() for k, v in got.items()})
+
+
+def sample_outputs(arrays, budget=DUMP_BYTES - (1 << 20)):
+    """float32 arrays stay float32, integer ones become float64 (exact).  Whatever does not fit ``budget`` bytes in
+    all: the smallest arrays are kept whole, each larger one keeps an equal share of what is left as a seeded sample
+    of its rows (``<name>_rows``: the row numbers, ascending).  Same shapes in, same rows out."""
+    arrays = {k: v if v.dtype == np.float32 else v.astype(np.float64) for k, v in arrays.items()}
+    out, left = {}, budget
+    for i, name in enumerate(sorted(arrays, key=lambda k: (arrays[k].nbytes, k))):
+        v, share = arrays[name], left // (len(arrays) - i)
+        if v.nbytes <= share:
+            out[name] = v
+        else:
+            keep = share // (v.nbytes // len(v) + 8)
+            rows = np.sort(np.random.default_rng(0).permutation(len(v))[:keep])
+            out[name], out[name + "_rows"] = v[rows], rows.astype(np.float64)
+        left -= out[name].nbytes + (out[name + "_rows"].nbytes if name + "_rows" in out else 0)
+    return out
+
+
+# ---------------------------------------------------------------------------------------------
 # the GPU arm
 # ---------------------------------------------------------------------------------------------
 def graft_arm(args, rank, world, local_rank, veh_cap, agent_cap):
@@ -499,13 +554,17 @@ def graft_arm(args, rank, world, local_rank, veh_cap, agent_cap):
     ev = [(torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)) for _ in range(K)]
     barrier()
     wall0 = time.perf_counter()
+    out = None
     for t in range(K):                         # the K timed ticks -> value
         flush.fill_(t & 0xFF)                  # L2 flush between timed iterations (not timed)
         ev[t][0].record()
-        tick(actions(t))
+        out = tick(actions(t))
         ev[t][1].record()
     barrier()
     wall1 = time.perf_counter()
+    # copied to the host now: the ticks below reuse the output buffers
+    dumped = (last_outputs(scene, out, act_buf if actor is not None else None, folder)
+              if args.dump_outputs and rank == 0 and out is not None else None)
     step_ms = [e0.elapsed_time(e1) for e0, e1 in ev]
     first_timed = 1 + PRIME_TICKS + W          # index of the first timed step since reset
     order_launches = sum(1 for t in range(first_timed, first_timed + K) if t % 32 == 0) if B >= 1024 else 0
@@ -697,14 +756,19 @@ def graft_arm(args, rank, world, local_rank, veh_cap, agent_cap):
             r = cpu_port_run(args, n_envs, PRIME_TICKS, 100, 5, cores)
             r1 = cpu_port_run(args, 32, PRIME_TICKS, 100, 5, 1)
             line["cpu_baseline"] = {
-                "value": r["agent_steps"] / r["elapsed"], "unit": UNIT, "cores": cores, "kind": "port",
+                "value": r["agent_steps"] / r["elapsed"], "unit": UNIT, "cores": r["threads"], "kind": "port",
                 "single_thread_value": r1["agent_steps"] / r1["elapsed"],
                 "python_reference": python_reference_rate(args),
                 "same_config": False,
-                "sample": "oracle/scene_oracle.c (C port of the reference scene, persistent thread pool): %d intersections "
-                          "x 100 ticks after %d priming ticks on %d threads (a per-agent-step rate on a bounded sample of the "
-                          "workload, not the 4096-intersection batch); single-thread figure on 32 intersections"
-                          % (n_envs, PRIME_TICKS, cores)}
+                "sample": "%s: %d intersections x 100 ticks after %d priming ticks on %d threads (a per-agent-step rate "
+                          "on a bounded sample of the workload, not the 4096-intersection batch); single-thread figure on "
+                          "%d intersections" % (r["port"], r["n_envs"], r["prime"], r["threads"], r1["n_envs"])}
+        if dumped is not None:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in dumped.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
+            print("dump-outputs: %d arrays, %.1f MB in %s" % (len(dumped), sum(a.nbytes for a in dumped.values()) / 1e6,
+                                                             args.dump_outputs), file=sys.stderr)
         print(json.dumps(line), flush=True)
     return True
 

@@ -7,10 +7,9 @@ import pytest
 import parity  # noqa: F401  (sys.path)
 from oracle import actor_oracle
 from pve_mcc_for_unsignalized_intersection_b200.actor import ACTOR_FLOATS, PARAM_SPECS, ActorWeights
-from pve_mcc_for_unsignalized_intersection_b200.checkpoint import read_bundle_index
+from pve_mcc_for_unsignalized_intersection_b200.checkpoint import read_bundle, read_bundle_index
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
-REF_CKPT = "/root/reference/model_data/baseline"
 
 
 def test_weight_fixture_layout():
@@ -56,17 +55,95 @@ def test_policy_actions_zero_for_uncontrolled():
     assert np.all(a[~ctrl] == 0) and np.all(a[ctrl] != 0)
 
 
-@pytest.mark.skipif(not os.path.isdir(REF_CKPT), reason="reference checkpoint only exists in the build container")
-def test_checkpoint_reader_against_the_shipped_bundle():
-    index = read_bundle_index(os.path.join(REF_CKPT, "66.cptk.index"))
-    assert len(index) == 152
-    assert sum(int(np.prod(e["shape"])) for e in index.values()) == 79412     # SURVEY.md section 2 #20
-    assert index["agent1actor/dense/kernel"] == {"dtype": 1, "shape": (28, 64), "shard": 0, "offset": 245412,
-                                                 "size": 7168}
-    w = ActorWeights.from_checkpoint(REF_CKPT)
+def _varint(n):
+    out = bytearray()
+    while True:
+        out.append((n & 0x7F) | (0x80 if n > 0x7F else 0))
+        n >>= 7
+        if not n:
+            return bytes(out)
+
+
+def _table_block(entries, restart_interval=4):
+    """A LevelDB table block of (key, value) pairs: prefix-compressed keys, restart array, then the 5-byte trailer
+    (type 0 = uncompressed, CRC left 0: the reader does not verify it)."""
+    body, restarts, prev = bytearray(), [], b""
+    for k, (key, val) in enumerate(entries):
+        shared = 0
+        if k % restart_interval:
+            while shared < min(len(key), len(prev)) and key[shared] == prev[shared]:
+                shared += 1
+        else:
+            restarts.append(len(body))
+        body += _varint(shared) + _varint(len(key) - shared) + _varint(len(val)) + key[shared:] + val
+        prev = key
+    for r in restarts or [0]:
+        body += r.to_bytes(4, "little")
+    body += len(restarts or [0]).to_bytes(4, "little")
+    return bytes(body) + b"\0" * 5
+
+
+def _bundle_entry(dtype, shape, offset, size):
+    """BundleEntryProto; proto3 leaves zero-valued fields out, the reader must default them."""
+    dims = b"".join(b"\x12" + _varint(len(d)) + d for d in (b"\x08" + _varint(n) for n in shape))
+    out = b"\x08" + _varint(dtype) + b"\x12" + _varint(len(dims)) + dims
+    out += (b"\x20" + _varint(offset) if offset else b"") + b"\x28" + _varint(size)
+    return out + b"\x35" + b"\x5a\x5a\x5a\x5a"          # field 6, crc32c (fixed32)
+
+
+def write_bundle(prefix, tensors, per_block=5):
+    """``tf.train.Saver`` layout of ``tensors`` (name -> array): ``prefix.index`` (sorted table, several data
+    blocks, index block, empty metaindex, 48-byte footer) + ``prefix.data-00000-of-00001``."""
+    data, entries = bytearray(), [(b"", b"\x08\x01")]        # header entry: BundleHeaderProto, num_shards 1
+    for name in sorted(tensors):
+        arr = np.asarray(tensors[name])
+        dtype = {np.dtype("<f4"): 1, np.dtype("<i8"): 9}[arr.dtype]
+        entries.append((name.encode(), _bundle_entry(dtype, arr.shape, len(data), arr.nbytes)))
+        data += arr.tobytes()
+    index_file, handles = bytearray(), []
+    for k in range(0, len(entries), per_block):
+        chunk = entries[k:k + per_block]
+        block = _table_block(chunk)
+        handles.append((chunk[-1][0], _varint(len(index_file)) + _varint(len(block) - 5)))
+        index_file += block
+    footer = bytearray()
+    for block in (_table_block([]), _table_block(handles, restart_interval=1)):       # metaindex, index
+        footer += _varint(len(index_file)) + _varint(len(block) - 5)
+        index_file += block
+    index_file += bytes(footer) + b"\0" * (40 - len(footer)) + (0xDB4775248B80FB57).to_bytes(8, "little")
+    with open(prefix + ".index", "wb") as f:
+        f.write(index_file)
+    with open(prefix + ".data-00000-of-00001", "wb") as f:
+        f.write(data)
+
+
+def test_checkpoint_reader_on_a_written_bundle(tmp_path):
+    """The reader on a bundle in the reference's checkpoint format (model_data/baseline/66.cptk), written here from
+    the stored agent-1 tensors: two actor scopes, a critic tensor and the int64 global step the reader must skip."""
     f = ActorWeights.from_npz(os.path.join(GOLD, "actor_agent1.npz"))
+    tensors = {"global_step": np.array(66, "<i8"), "agent1_critic/dense/kernel": np.full((30, 64), 0.5, np.float32)}
+    for n, _ in PARAM_SPECS:
+        tensors["agent1actor/" + n] = f.tensors[n]
+        tensors["agent1_target_actor/" + n] = f.tensors[n] * np.float32(2)
+    write_bundle(str(tmp_path / "66.cptk"), tensors)
+    (tmp_path / "checkpoint").write_text('model_checkpoint_path: "66.cptk"\nall_model_checkpoint_paths: "66.cptk"\n')
+
+    index = read_bundle_index(str(tmp_path / "66.cptk.index"))
+    assert sorted(index) == sorted(tensors)
+    assert sum(int(np.prod(e["shape"])) for e in index.values()) == 2 * ACTOR_FLOATS + 30 * 64 + 1
+    assert index["agent1_critic/dense/kernel"] == {"dtype": 1, "shape": (30, 64), "shard": 0, "offset": 0, "size": 7680}
+    assert index["global_step"] == {"dtype": 9, "shape": (), "shard": 0, "offset": 4 * (2 * ACTOR_FLOATS + 30 * 64),
+                                    "size": 8}
+    assert index["agent1actor/dense/kernel"]["dtype"] == 1 and index["agent1actor/dense/kernel"]["shape"] == (28, 64)
+    assert index["agent1actor/dense/kernel"]["size"] == 7168 and index["agent1actor/dense/kernel"]["shard"] == 0
+    w = ActorWeights.from_checkpoint(str(tmp_path))
+    t = ActorWeights.from_checkpoint(str(tmp_path / "66.cptk"), scope="agent1_target_actor")
     for n, _ in PARAM_SPECS:
         assert np.array_equal(w.tensors[n], f.tensors[n]), n
+        assert np.array_equal(t.tensors[n], f.tensors[n] * np.float32(2)), n
+    assert "global_step" not in read_bundle(str(tmp_path / "66.cptk"))
+    with pytest.raises(KeyError):
+        ActorWeights.from_checkpoint(str(tmp_path), scope="agent2actor")
 
 
 def test_actor_needs_a_gpu_and_says_so():
