@@ -219,7 +219,12 @@ const pve_env_header *pve_hdr_dev(const pve_scene *s);
 int32_t pve_stats(pve_scene *s, pve_counters *out_dev, void *stream);
 /* the same statistics PER INTERSECTION, as the step kernel accumulates them on the device: double [B][PVE_ENV_NSTAT] in
  * the order agent_steps, vehicle_steps, collided_agent_steps (MAIN:569-571), lock_events (MAIN:568), passed_jerk_sum
- * (MAIN:567), reward_sum, reward_sq_sum, removed, env_steps, q5_undefined.  Valid after the stream has drained. */
+ * (MAIN:567), reward_sum, reward_sq_sum, removed, env_steps, q5_undefined.  Valid after the stream has drained.
+ * What they count: vehicle_steps adds the vehicles present when a tick starts, before that tick's arrivals spawn (the
+ * vehicles the tick steps); reward_sum / reward_sq_sum add the fp32 rewards of the rows, overrides included, in float64.
+ * pve_reset zeroes them, and its warm-up tick (warmup != 0) counts as one env step and nothing else.  pve_set_state
+ * leaves them alone: teacher-forced ticks keep adding to the episode's totals.  They describe the simulation, not the
+ * emitted rows: the rows of intersections that out_cap left out (overflow) are counted all the same. */
 #define PVE_ENV_NSTAT 10
 const double *pve_env_stats_dev(const pve_scene *s);
 
