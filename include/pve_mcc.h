@@ -143,6 +143,22 @@ typedef struct pve_outputs {
      * what a host-side consumer needs of reward / ids / cpv / status / jerk_sum at 16 instead of 29 bytes per agent
      * (the intersection index is implied by agent_offset).  pve_step_host_async delivers these records. */
     void *packed;
+    /* optional (may be null), the FACTORED observation: every observation row is a copy (Q3), so the 7 x 28 block of
+     * an agent is determined by two 28-float rows per agent of the same tick and 8 codes.  For output row
+     * r = agent_offset[b] + g:
+     *   row0_out[r]  = obs[r][0], this tick's row 0 of agent g;
+     *   prev_row0[r] = the row 0 stored for agent g's vehicle when the tick started (its actor input; zeros for a
+     *                  vehicle that spawned last tick);
+     *   obs_src[r][q], q < 7: where obs[r][q] comes from: -1 = the all-zero row; g' (0 .. 0x3FFF) =
+     *                  row0_out[agent_offset[b] + g']; 0x4000 | g' = prev_row0[agent_offset[b] + g'].  Entry 0 is g,
+     *                  entry 7 is padding (-1).
+     * Codes are relative to the agent's own intersection and never refer to another tick's buffers (a neighbour is
+     * always an agent of the same tick).  Set all three or none; `obs` may then be null, and the 784 B block of every
+     * agent is not written at all.  pve_expand_obs / pve_expand_obs_host rebuild `obs` bit for bit.  lane_num = 12
+     * only: with lane_num 4 / 8 pve_step returns PVE_EINVAL when any of them is set. */
+    float *row0_out;        /* [out_cap][28] */
+    float *prev_row0;       /* [out_cap][28] */
+    int16_t *obs_src;       /* [out_cap][8]  */
 } pve_outputs;
 
 typedef struct pve_agent_record {
@@ -184,6 +200,21 @@ int32_t pve_set_intention_draws(pve_scene *s, const uint8_t *draws_dev);
  * delete_vehicle() (TIS:435).  actions_dev: float [B][veh_cap]. */
 int32_t pve_step(pve_scene *s, const float *actions_dev, const pve_outputs *out_dev, void *stream);
 
+/* Rebuild obs[r] (float [7][28]) from the factored outputs of one tick (pve_outputs.row0_out / prev_row0 / obs_src),
+ * bit for bit, for the rows of intersections [b0, b1): rows agent_offset[b0] .. agent_offset[b1] - 1 (agent_offset
+ * [b1 + 1] entries).  Like the step, an intersection whose rows do not all fit below `out_cap` is skipped (the step
+ * wrote none of its rows).  Plain C on host memory; disjoint intersection ranges may be expanded from different threads
+ * at once.  Every code is checked against its own intersection's row count: a row with an invalid code becomes NaN
+ * instead of being read out of range.  Returns the number of invalid codes (0 for the output of a step; a negative
+ * agent_offset or a decreasing pair of offsets counts as one and skips that intersection), or PVE_EINVAL for a null
+ * pointer or b1 < b0. */
+int64_t pve_expand_obs_host(const int32_t *agent_offset, int32_t b0, int32_t b1, int64_t out_cap, const float *row0_out,
+                            const float *prev_row0, const int16_t *obs_src, float *obs_out);
+/* The same for all B intersections on the device: one CUDA kernel on `stream` that reads agent_offset_dev[0 .. B] on
+ * the device (nothing waits).  Invalid codes yield NaN rows as above; nothing is counted. */
+int32_t pve_expand_obs(const int32_t *agent_offset_dev, int32_t B, int64_t out_cap, const float *row0_out_dev,
+                       const float *prev_row0_dev, const int16_t *obs_src_dev, float *obs_dev, void *stream);
+
 /* Same tick through HOST buffers; synchronises.  `copy_mask` bit0: reward/ids/cpv/status/jerk_sum/
  * agent_offset/env_* ; bit1: obs.  `out_host` arrays need `pve_next_agent_total()` rows.
  * Pinned host memory (cudaHostAlloc / cudaHostRegister, torch pin_memory()) is used in place: the kernel reads
@@ -194,8 +225,10 @@ int32_t pve_step_host(pve_scene *s, const float *actions_host, const pve_outputs
 
 /* Pipelined host path: the same tick, but nothing waits.  Actions travel by DMA from `actions_host` (pinned), the
  * kernel runs on `stream`, and agent_offset + the per-intersection counters + the 16-byte agent records
- * (out_dev->packed, required) -- with copy_mask bit1 also the observations -- travel by DMA into `out_host` on an
- * internal copy stream while the caller already enqueues the next ticks.  Three ticks may be in flight: give
+ * (out_dev->packed, required) -- with copy_mask bit1 also the observations, with bit2 the factored observation
+ * (row0_out, prev_row0, obs_src: 240 B per agent; required in both sets, and out_dev->obs may then be null so that the
+ * step does not write the 784 B block at all) -- travel by DMA into `out_host` on an internal copy stream while the
+ * caller already enqueues the next ticks.  Three ticks may be in flight: give
  * consecutive calls different `out_dev` / `out_host` buffer sets (three of them, used in turn) and call
  * pve_host_wait() for tick t before the call for tick t + 3.  The call itself only waits for the previous tick's KERNEL
  * (it needs that tick's row count to size the copies). */

@@ -39,7 +39,7 @@ class PveStateView(C.Structure):
 class PveOutputs(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in
                 ("agent_offset", "obs", "reward", "ids", "cpv", "status", "jerk_sum",
-                 "env_collisions", "env_lock", "env_removed", "nbr_src", "packed")]
+                 "env_collisions", "env_lock", "env_removed", "nbr_src", "packed", "row0_out", "prev_row0", "obs_src")]
 
 
 class PveReplayView(C.Structure):
@@ -72,6 +72,9 @@ def load_library(path=None):
     lib.pve_step.argtypes = [vp, vp, C.POINTER(PveOutputs), vp]
     lib.pve_step_host.argtypes = [vp, vp, C.POINTER(PveOutputs), C.POINTER(PveOutputs), i32, vp]
     lib.pve_step_host_async.argtypes = [vp, vp, C.POINTER(PveOutputs), C.POINTER(PveOutputs), i32, vp]
+    lib.pve_expand_obs_host.argtypes = [vp, i32, i32, i64, vp, vp, vp, vp]
+    lib.pve_expand_obs_host.restype = i64
+    lib.pve_expand_obs.argtypes = [vp, i32, i64, vp, vp, vp, vp, vp]
     lib.pve_host_wait.argtypes = [vp]
     lib.pve_host_wait.restype = i64
     lib.pve_next_agent_total.argtypes = [vp, vp]

@@ -138,6 +138,16 @@ static int rt_host_alloc(void **p, size_t n) { return rt_alloc(p, n); }
 static void rt_host_free(void *p) { free(p); }
 #endif
 
+/* the source of one observation row under its factored code (pve_outputs.obs_src) in an intersection of A rows:
+ * 0 = the zero row, 1 = row0_out row `idx`, 2 = prev_row0 row `idx` (relative to the intersection), -1 = invalid */
+PVE_HD int pve_obs_src_decode(int16_t c, int64_t A, int64_t *idx) {
+    if (c == -1) return 0;
+    if (c < 0 || (int64_t)(c & 0x3FFF) >= A) return -1;
+    *idx = c & 0x3FFF;
+    return (c & 0x4000) ? 2 : 1;
+}
+#define PVE_NAN_BITS 0x7FC00000u      /* an observation row behind an invalid code */
+
 /* =============================================================================================
  * kernels
  * =========================================================================================== */
@@ -331,6 +341,27 @@ pve_stats_kernel(PveState S, int B, double *out) {
     }
 }
 
+/* pve_expand_obs: one CTA per intersection; consecutive threads store consecutive 16-byte pieces of its block (the
+ * code of a row is read by the 7 threads of its pieces) */
+__global__ void __launch_bounds__(128)
+pve_expand_obs_kernel(const int32_t *__restrict__ off, int64_t out_cap, const pve_v4 *__restrict__ r0,
+                      const pve_v4 *__restrict__ pr, const int16_t *__restrict__ src, pve_v4 *__restrict__ obs) {
+    const int b = (int)blockIdx.x;
+    const int64_t o0 = off[b], o1 = off[b + 1];
+    if (o0 < 0 || o1 < o0 || o1 > out_cap) return;           /* rows the step did not write (out_cap) */
+    const int64_t n = (o1 - o0) * (PVE_OBS_H * 7);
+    for (int64_t it = threadIdx.x; it < n; it += blockDim.x) {
+        const int64_t g = it / (PVE_OBS_H * 7);
+        const int rem = (int)(it - g * (PVE_OBS_H * 7)), q = rem / 7, piece = rem - q * 7;
+        int64_t idx = 0;
+        const int k = pve_obs_src_decode(src[(o0 + g) * 8 + q], o1 - o0, &idx);
+        pve_v4 v;
+        if (k > 0) v = (k == 1 ? r0 : pr)[(o0 + idx) * 7 + piece];
+        else { const uint32_t w = k == 0 ? 0u : PVE_NAN_BITS; v.x = w; v.y = w; v.z = w; v.w = w; }
+        obs[(o0 + g) * (PVE_OBS_H * 7) + rem] = v;
+    }
+}
+
 #else  /* ------------------------------- host emulation ------------------------------------ */
 
 static void emul_gsum(const int32_t *n_ctrl, int32_t *gs_now, int32_t *gs_a, int32_t *gs_b, int B, int G) {
@@ -505,10 +536,12 @@ static cudaError_t launch_dual(pve_scene *s, const float *actions, const pve_out
     return cudaStreamWaitEvent(stream, s->ev_join, 0);
 }
 
-/* the instantiation that also writes pve_outputs.nbr_src only when the caller asks for that output */
+/* the instantiation that also writes pve_outputs.nbr_src and the factored observation only when the caller asks for
+ * one of them */
+static bool wants_src(const pve_outputs &O) { return O.nbr_src != nullptr || O.obs_src != nullptr; }
 template <int NT, int VC, int AC>
 static cudaError_t launch_one(pve_scene *s, const float *actions, const pve_outputs &O, pve_stream_t stream) {
-    return O.nbr_src ? launch_variant<NT, VC, AC, true>(s, actions, O, stream)
+    return wants_src(O) ? launch_variant<NT, VC, AC, true>(s, actions, O, stream)
                      : launch_variant<NT, VC, AC, false>(s, actions, O, stream);
 }
 #endif
@@ -563,9 +596,26 @@ static int32_t launch_step4(pve_scene *s, const float *actions, const pve_output
     return PVE_OK;
 }
 
+/* the factored observation (pve_outputs.row0_out / prev_row0 / obs_src): all three fields or none, 12-lane only */
+static int32_t check_factored(pve_scene *s, const pve_outputs &O) {
+    const int n = (O.row0_out != nullptr) + (O.prev_row0 != nullptr) + (O.obs_src != nullptr);
+    if (n != 0 && n != 3) {
+        snprintf(s->err, sizeof s->err, "the factored observation needs all of row0_out, prev_row0 and obs_src (%d of 3 set)", n);
+        return PVE_EINVAL;
+    }
+    if (n != 0 && s->lane_num != 12) {
+        snprintf(s->err, sizeof s->err, "lane_num = %d: the factored observation (row0_out / prev_row0 / obs_src) exists for "
+                                        "the 12-lane intersection only", s->lane_num);
+        return PVE_EINVAL;
+    }
+    return PVE_OK;
+}
+
 static int32_t launch_step(pve_scene *s, const float *actions, const pve_outputs &O_in, pve_stream_t stream) {
     const int VCc = s->prm.VC, ACc = s->prm.AC;
     pve_outputs O = O_in;
+    const int32_t rc = check_factored(s, O);
+    if (rc != PVE_OK) return rc;
     if (s->lane_num != 12) return launch_step4(s, actions, O, stream);
     if (s->exp_no_obs) O.obs = nullptr;          /* experiment knob (env PVE_EXPERIMENT_NO_OBS): what the observation traffic costs */
 #ifndef PVE_HOST_EMULATION
@@ -584,9 +634,9 @@ static int32_t launch_step(pve_scene *s, const float *actions, const pve_outputs
     bool done = false;
     if (s->dual) {
         done = true;
-        if (VCc == 192) RT_CHECK(s, (O.nbr_src ? launch_dual<192, 128, true>(s, actions, O, stream) : launch_dual<192, 128, false>(s, actions, O, stream)));
-        else if (ACc == 96) RT_CHECK(s, (O.nbr_src ? launch_dual<128, 96, true>(s, actions, O, stream) : launch_dual<128, 96, false>(s, actions, O, stream)));
-        else RT_CHECK(s, (O.nbr_src ? launch_dual<128, 80, true>(s, actions, O, stream) : launch_dual<128, 80, false>(s, actions, O, stream)));
+        if (VCc == 192) RT_CHECK(s, (wants_src(O) ? launch_dual<192, 128, true>(s, actions, O, stream) : launch_dual<192, 128, false>(s, actions, O, stream)));
+        else if (ACc == 96) RT_CHECK(s, (wants_src(O) ? launch_dual<128, 96, true>(s, actions, O, stream) : launch_dual<128, 96, false>(s, actions, O, stream)));
+        else RT_CHECK(s, (wants_src(O) ? launch_dual<128, 80, true>(s, actions, O, stream) : launch_dual<128, 80, false>(s, actions, O, stream)));
     }
 #define X(vc, ac)                                                                              \
     if (!done && VCc == vc && ACc == ac) {                                                     \
@@ -1102,6 +1152,11 @@ static int32_t async_copy_out(pve_scene *s, int64_t seq) {
     }
     D2HA(packed, sizeof(pve_agent_record) * a);
     if (s->a_mask[slot] & 2) D2HA(obs, sizeof(float) * PVE_OBS_H * PVE_OBS_W * a);
+    if (s->a_mask[slot] & 4) {                 /* the factored observation: 240 instead of 784 bytes per agent */
+        D2HA(row0_out, sizeof(float) * PVE_OBS_W * a);
+        D2HA(prev_row0, sizeof(float) * PVE_OBS_W * a);
+        D2HA(obs_src, sizeof(int16_t) * 8 * a);
+    }
 #undef D2HA
     RT_CHECK(s, cudaEventRecord(s->a_done[slot], s->s_out));
     s->a_copied = seq + 1;
@@ -1122,6 +1177,12 @@ int32_t pve_step_host_async(pve_scene *s, const float *actions_host, const pve_o
         snprintf(s->err, sizeof s->err, "pve_step_host_async needs packed + agent_offset (and obs with bit1) in out_dev and out_host");
         return PVE_EINVAL;
     }
+    if ((copy_mask & 4) && (!out_dev->obs_src || !out_host->row0_out || !out_host->prev_row0 || !out_host->obs_src)) {
+        snprintf(s->err, sizeof s->err, "pve_step_host_async: copy_mask bit2 needs row0_out, prev_row0 and obs_src in out_dev "
+                                        "and out_host");
+        return PVE_EINVAL;
+    }
+    if (check_factored(s, *out_dev) != PVE_OK) return PVE_EINVAL;
     const int inflight = (int)(s->a_seq - s->a_waited);
     if (inflight >= PVE_ASYNC_SLOTS) {
         snprintf(s->err, sizeof s->err, "%d ticks are in flight: call pve_host_wait first", inflight);
@@ -1260,6 +1321,49 @@ int32_t pve_stats(pve_scene *s, pve_counters *out_dev, void *stream_) {
 #endif
     RT_CHECK(s, rt_copy(out_dev, s->counters_dev, sizeof(double) * 16, stream));
     return PVE_OK;
+}
+
+/* ---- factored observation -> obs ------------------------------------------------------------ */
+int64_t pve_expand_obs_host(const int32_t *off, int32_t b0, int32_t b1, int64_t out_cap, const float *r0,
+                            const float *pr, const int16_t *src, float *obs) {
+    if (!off || !r0 || !pr || !src || !obs || b0 < 0 || b1 < b0) return PVE_EINVAL;
+    const size_t row_bytes = sizeof(float) * PVE_OBS_W;
+    int64_t bad = 0;
+    for (int32_t b = b0; b < b1; ++b) {
+        const int64_t o0 = off[b], o1 = off[b + 1];
+        if (o0 < 0 || o1 < o0) { ++bad; continue; }
+        if (o1 > out_cap) continue;                             /* rows the step did not write */
+        for (int64_t r = o0; r < o1; ++r) {
+            float *dst = obs + (size_t)r * PVE_OBS_H * PVE_OBS_W;
+            for (int q = 0; q < PVE_OBS_H; ++q) {
+                int64_t idx = 0;
+                const int k = pve_obs_src_decode(src[(size_t)r * 8 + q], o1 - o0, &idx);
+                float *d = dst + q * PVE_OBS_W;
+                if (k > 0) memcpy(d, (k == 1 ? r0 : pr) + (size_t)(o0 + idx) * PVE_OBS_W, row_bytes);
+                else if (k == 0) memset(d, 0, row_bytes);
+                else {
+                    ++bad;
+                    const uint32_t w = PVE_NAN_BITS;
+                    for (int i = 0; i < PVE_OBS_W; ++i) memcpy(d + i, &w, sizeof w);
+                }
+            }
+        }
+    }
+    return bad;
+}
+
+int32_t pve_expand_obs(const int32_t *off_dev, int32_t B, int64_t out_cap, const float *r0_dev, const float *pr_dev,
+                       const int16_t *src_dev, float *obs_dev, void *stream) {
+    if (!off_dev || !r0_dev || !pr_dev || !src_dev || !obs_dev || B < 0) return PVE_EINVAL;
+    if (B == 0) return PVE_OK;
+#ifndef PVE_HOST_EMULATION
+    pve_expand_obs_kernel<<<B, 128, 0, (pve_stream_t)stream>>>(off_dev, out_cap, (const pve_v4 *)r0_dev, (const pve_v4 *)pr_dev,
+                                                               src_dev, (pve_v4 *)obs_dev);
+    return cudaGetLastError() == cudaSuccess ? PVE_OK : PVE_ECUDA;
+#else
+    (void)stream;
+    return pve_expand_obs_host(off_dev, 0, B, out_cap, r0_dev, pr_dev, src_dev, obs_dev) >= 0 ? PVE_OK : PVE_EINVAL;
+#endif
 }
 
 /* ---- actor (N1) ---------------------------------------------------------------------------- */

@@ -33,6 +33,9 @@
 #include <math.h>
 #include <stdint.h>
 #include <string.h>
+#ifndef __CUDACC__
+#include <assert.h>
+#endif
 
 #include "pve_mcc.h"
 
@@ -483,6 +486,57 @@ PVE_DEV void pve_move_rows(const PveRowJob &J, int first_warp) {
         memcpy(J.oblk + (size_t)it * 7, src, PVE_OBS_W * sizeof(float));
     }
 #endif
+}
+
+/* ---------------------------------------------------------------------------------------------
+ * Factored observation (pve_outputs.row0_out / prev_row0 / obs_src; SRC instantiation only): per agent its
+ * row 0 of this tick, the row stored for its vehicle when the tick started, and the 7 row codes of its
+ * observation translated to agent indices.  A neighbour is always an agent of the same tick (virtual
+ * lanes hold agents only, phase E), so a "last tick's row" code (PVE_SRC_PREV | slot * 7) becomes
+ * 0x4000 | the neighbour's agent index.  Everything read here is final after phase G1 and no later
+ * phase writes it, so either half of a split CTA can do it: the mover warps right after G1 when there
+ * are no observation rows to move, the team after phase K otherwise.
+ * ------------------------------------------------------------------------------------------- */
+struct PveFactJob {
+    int A, V, AC;
+    const uint16_t *srcc;         /* [A][7] gather codes */
+    const uint16_t *acnt;         /* [V + 1] agent index of each vehicle slot (exclusive scan of the control flags) */
+    const uint16_t *vidx;         /* [A] vehicle slot of each agent */
+    const float *rows_smem;       /* [AC + 1][28] this tick's row 0 of every agent */
+    const float *rows_prev;       /* last tick's stored rows of this intersection */
+    pve_v4 *row0_out, *prev_out;  /* this intersection's first row of pve_outputs.row0_out / prev_row0, or null */
+    pve_v4 *src_out;              /* ... of pve_outputs.obs_src */
+};
+
+PVE_DEV void pve_write_factored(const PveFactJob &J, int t, int nthreads) {
+    if (J.src_out == nullptr) return;
+#pragma unroll 1
+    for (int it = t; it < J.A * 8; it += nthreads) {
+        const int g = it >> 3, q = it & 7;
+        if (q < 7) {                       /* 16-byte piece q of both rows: a warp stores 4 rows x 7 pieces contiguously */
+            J.row0_out[g * 7 + q] = ((const pve_v4 *)(J.rows_smem + (size_t)g * PVE_OBS_W))[q];
+            J.prev_out[g * 7 + q] = ((const pve_v4 *)(J.rows_prev + (size_t)J.vidx[g] * PVE_OBS_W))[q];
+        } else {
+            uint32_t w4[4];
+#pragma unroll
+            for (int r = 0; r < 8; ++r) {
+                const uint32_t c = r < PVE_OBS_H ? J.srcc[g * 7 + r] : (uint32_t)(J.AC * 7);
+                uint32_t v;
+                if (c == (uint32_t)(J.AC * 7)) v = 0xFFFFu;                                 /* the zero row */
+                else if (c & PVE_SRC_PREV) {
+                    const int kn = (int)((c & 0x7FFFu) / 7u);
+#ifndef __CUDACC__
+                    /* the premise of the contract: the neighbour is an agent of this tick */
+                    assert(kn < J.V && J.acnt[kn + 1] == J.acnt[kn] + 1 && J.acnt[kn] < J.A);
+#endif
+                    v = 0x4000u | J.acnt[kn];
+                } else v = c / 7u;
+                if (r & 1) w4[r >> 1] |= v << 16; else w4[r >> 1] = v;
+            }
+            pve_v4 s; s.x = w4[0]; s.y = w4[1]; s.z = w4[2]; s.w = w4[3];
+            J.src_out[g] = s;
+        }
+    }
 }
 
 /* ---------------------------------------------------------------------------------------------
@@ -1059,9 +1113,19 @@ PVE_DEV void pve_step_block(const PveParams &P, const PveState &S, const pve_out
      *      final after G1) while the lower half ("team") finishes the tick ------------------------ */
     PveRowJob RJ;
     RJ.A = A; RJ.srcc = srcc; RJ.rows_smem = row0; RJ.rows_prev = row0_prev_base; RJ.oblk = oblk; RJ.zero_row = AC;
+    PveFactJob FJ;
+    if (SRC) {
+        const bool fact = O.obs_src != nullptr && out_ok;
+        FJ.A = A; FJ.V = V; FJ.AC = AC; FJ.srcc = srcc; FJ.acnt = acnt; FJ.vidx = vidx; FJ.rows_smem = row0;
+        FJ.rows_prev = row0_prev_base;
+        FJ.row0_out = fact ? (pve_v4 *)O.row0_out + obase * (PVE_OBS_W / 4) : nullptr;
+        FJ.prev_out = fact ? (pve_v4 *)O.prev_row0 + obase * (PVE_OBS_W / 4) : nullptr;
+        FJ.src_out = fact ? (pve_v4 *)O.obs_src + obase : nullptr;
+    }
 #ifdef __CUDACC__
     if (NS < NT && (int)threadIdx.x >= NS) {
         pve_move_rows<NT, (NT > NS ? (NT - NS) / 32 : 1)>(RJ, NS / 32);
+        if (SRC && oblk == nullptr) pve_write_factored(FJ, (int)threadIdx.x - NS, NT - NS);
 #ifdef PVE_PHASE_TIMING
         if ((int)threadIdx.x == NS && S.stats) ((long long *)S.dbg)[(size_t)b * 48 + 47] = clock64();
 #endif
@@ -1381,6 +1445,13 @@ PVE_DEV void pve_step_block(const PveParams &P, const PveState &S, const pve_out
                 pve_v4 nb; nb.x = w4[0]; nb.y = w4[1]; nb.z = w4[2]; nb.w = w4[3];
                 ((pve_v4 *)O.nbr_src)[obase + g] = nb;
             }
+        PVE_END_TID_NOSYNC
+    }
+    /* ---- optional output: the factored observation, on the half of the CTA that has no observation rows to move (the
+     *      mover warps took it after G1 when pve_outputs.obs is null) */
+    if (SRC && (NS == NT || oblk != nullptr)) {
+        PVE_FOR_TEAM(tid)
+            pve_write_factored(FJ, tid, NS);
         PVE_END_TID_NOSYNC
     }
 

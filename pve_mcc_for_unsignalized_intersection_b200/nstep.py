@@ -174,6 +174,9 @@ class NStepFolder:
         """main.py:243-266 for the tick that produced ``outputs`` (a ``StepOutputs``).  Asynchronous.
         ``distinct_rows``: None = use the scene's neighbour sources when it exports them; False = always evaluate the
         target actor on all 7 rows of every observation."""
+        if outputs.obs is None:
+            raise ValueError("NStepFolder.push reads the observations, and these outputs carry none (BatchedScene("
+                             "full_obs=False)): call bind_outputs() before the step so that it writes them into the frame log")
         o = outputs.native()
         if distinct_rows is None:
             distinct_rows = getattr(outputs, "nbr_src", None) is not None and outputs is self.scene.out

@@ -7,6 +7,7 @@ compute happens in the hand-written sm_100a kernels of ``csrc/`` behind the C AB
 ``include/pve_mcc.h``; torch tensors are used only as device buffers and for streams.
 """
 import ctypes as C
+from concurrent.futures import ThreadPoolExecutor
 
 import numpy as np
 import torch
@@ -24,14 +25,17 @@ class StepOutputs:
     reused by the next ``step`` call.
     """
 
-    def __init__(self, B, out_cap, device, neighbour_sources=False, records_only=False):
+    def __init__(self, B, out_cap, device, neighbour_sources=False, records_only=False, factored=False, full_obs=True,
+                 lib=None):
         z = lambda *s, dt: torch.zeros(*s, dtype=dt, device=device)
         e = lambda *s, dt: None
         per_agent = e if records_only else z                       # records_only: the 16-byte records replace them
+        self.B, self.out_cap, self._lib = B, out_cap, lib
         # agent_offset and the three per-intersection counters share one allocation (one DMA on the host path)
         self._small = z(4 * B + 1, dt=torch.int32)
         self.agent_offset = self._small[:B + 1]
-        self.obs = z(out_cap, OBS_H, OBS_W, dt=torch.float32)       # re_state
+        # re_state; None with full_obs=False: the step does not write the 7 x 28 block at all
+        self.obs = z(out_cap, OBS_H, OBS_W, dt=torch.float32) if full_obs else None
         self.reward = per_agent(out_cap, dt=torch.float32)
         self.ids = per_agent(out_cap, 4, dt=torch.int32)           # env, lane, j, uid
         self.cpv = per_agent(out_cap, dt=torch.int32)              # collisions_per_veh[:, 0]
@@ -45,6 +49,12 @@ class StepOutputs:
         # optional: where each of the 7 observation rows was copied from (include/pve_mcc.h, pve_outputs.nbr_src):
         # -1 zero row; g' = row 0 of agent g' of the same intersection this tick; 0x4000 | k = last tick's row of slot k
         self.nbr_src = z(out_cap, 8, dt=torch.int16) if neighbour_sources else None
+        # optional: the factored observation (include/pve_mcc.h, pve_outputs.row0_out / prev_row0 / obs_src): this tick's
+        # row 0 of every agent, the row stored for its vehicle when the tick started, and per observation row a code:
+        # -1 zero row, g' = row0_out of agent g' of the same intersection, 0x4000 | g' = prev_row0 of agent g'
+        self.row0_out = z(out_cap, OBS_W, dt=torch.float32) if factored else None
+        self.prev_row0 = z(out_cap, OBS_W, dt=torch.float32) if factored else None
+        self.obs_src = z(out_cap, 8, dt=torch.int16) if factored else None
         self._n = None
 
     FIELDS = ("agent_offset", "obs", "reward", "ids", "cpv", "status", "jerk_sum",
@@ -58,7 +68,7 @@ class StepOutputs:
         self.env_collisions = self._small[B + 1:2 * B + 1]
         self.env_lock = self._small[2 * B + 1:3 * B + 1]
         self.env_removed = self._small[3 * B + 1:4 * B + 1]
-        for f in ("obs", "reward", "ids", "cpv", "status", "jerk_sum", "packed"):
+        for f in ("obs", "reward", "ids", "cpv", "status", "jerk_sum", "packed", "row0_out", "prev_row0", "obs_src"):
             if getattr(self, f) is not None:
                 setattr(self, f, getattr(self, f).pin_memory())
         return self
@@ -70,7 +80,53 @@ class StepOutputs:
             setattr(o, f, t.data_ptr() if t is not None else None)
         o.nbr_src = self.nbr_src.data_ptr() if self.nbr_src is not None else None
         o.packed = self.packed.data_ptr() if self.packed is not None else None
+        for f in ("row0_out", "prev_row0", "obs_src"):
+            t = getattr(self, f)
+            setattr(o, f, t.data_ptr() if t is not None else None)
         return o
+
+    def expand_obs(self, n=None, out=None, threads=1):
+        """The observations ``[n, 7, 28]`` rebuilt bit for bit from the factored block (``row0_out``, ``prev_row0``,
+        ``obs_src``), into ``out`` (float32 ``[>= n, 7, 28]`` on the buffers' device, allocated if None); returns
+        ``out[:n]``.  ``n`` defaults to this tick's row count.  Device buffers: one kernel on the current stream
+        (``pve_expand_obs``).  Host buffers: the C expander (``pve_expand_obs_host``) over ``threads`` ranges of
+        intersections in parallel (the calls release the GIL).  Raises ``ValueError`` if a code is out of range."""
+        if self.obs_src is None:
+            raise ValueError("these outputs carry no factored observation (BatchedScene(factored_obs=True), "
+                             "make_async_buffers(factored=True))")
+        lib = self._lib or N.load_library()
+        dev = self.obs_src.device
+        n = self.n_agents if n is None else int(n)
+        if out is None:
+            out = torch.empty(max(n, 1), OBS_H, OBS_W, dtype=torch.float32, device=dev)
+        if (out.dtype != torch.float32 or out.device != dev or not out.is_contiguous() or out.dim() != 3
+                or tuple(out.shape[1:]) != (OBS_H, OBS_W) or out.shape[0] < n):
+            raise ValueError("out must be a contiguous float32 [>= %d, 7, 28] tensor on %s" % (n, dev))
+        # rows past n (and past the buffers) are never touched: the expanders skip intersections beyond the cap
+        cap = min(n, self.row0_out.shape[0], self.prev_row0.shape[0], self.obs_src.shape[0])
+        ptrs = (self.row0_out.data_ptr(), self.prev_row0.data_ptr(), self.obs_src.data_ptr(), out.data_ptr())
+        if dev.type == "cuda":
+            stream = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            rc = lib.pve_expand_obs(self.agent_offset.data_ptr(), self.B, cap, *ptrs, stream)
+            if rc != 0:
+                raise N.NativeError("pve_expand_obs failed with %d" % rc)
+            return out[:n]
+        off = self.agent_offset.numpy()
+        bounds = [0, self.B]
+        if threads > 1 and self.B > 1:      # ranges of about equal row counts
+            cuts = np.searchsorted(off[:self.B + 1], np.arange(1, threads) * (n / threads), side="left")
+            bounds = sorted(set([0, self.B] + [int(min(max(c, 0), self.B)) for c in cuts]))
+        ranges = list(zip(bounds[:-1], bounds[1:]))
+        call = lambda r: int(lib.pve_expand_obs_host(self.agent_offset.data_ptr(), r[0], r[1], cap, *ptrs))
+        if len(ranges) == 1:
+            bad = [call(ranges[0])]
+        else:
+            bad = list(_pool(threads).map(call, ranges))
+        if any(b < 0 for b in bad):
+            raise N.NativeError("pve_expand_obs_host failed with %d" % min(bad))
+        if sum(bad):
+            raise ValueError("the factored observation holds %d invalid row codes" % sum(bad))
+        return out[:n]
 
     def records(self, n=None):
         """Host buffers only: the agent records as a numpy structured array (``_native.RECORD_DTYPE``: reward, uid,
@@ -95,11 +151,20 @@ class StepOutputs:
         return (self.status & N.ST_DONE) != 0
 
 
+_POOLS = {}
+
+
+def _pool(threads):
+    if threads not in _POOLS:
+        _POOLS[threads] = ThreadPoolExecutor(max_workers=threads, thread_name_prefix="pve_expand")
+    return _POOLS[threads]
+
+
 class BatchedScene:
     """B independent 12-lane intersections resident on one GPU."""
 
     def __init__(self, n_envs, config=None, veh_cap=128, agent_cap=96, out_cap=None, device="cuda:0",
-                 threads=0, _library=None, neighbour_sources=False):
+                 threads=0, _library=None, neighbour_sources=False, factored_obs=False, full_obs=True):
         self.cfg = config or SceneConfig()
         self.B, self.veh_cap, self.agent_cap = int(n_envs), int(veh_cap), int(agent_cap)
         self.out_cap = int(out_cap) if out_cap is not None else self.B * self.agent_cap
@@ -124,7 +189,12 @@ class BatchedScene:
         # capacities are rounded up to a compiled capacity class; the class value is the array stride
         self.veh_cap = int(self.lib.pve_veh_cap(self._h))
         self.agent_cap = int(self.lib.pve_agent_cap(self._h))
-        self.out = StepOutputs(self.B, self.out_cap, self.device, neighbour_sources=neighbour_sources)
+        # factored_obs: the step also writes the factored observation (StepOutputs.row0_out / prev_row0 / obs_src;
+        # 12-lane intersections only); full_obs=False: it does not write the 784-byte observation of every agent
+        if factored_obs and self.cfg.lane_num != NLANE:
+            raise ValueError("factored_obs exists for the 12-lane intersection only (lane_num=%d)" % self.cfg.lane_num)
+        self.out = StepOutputs(self.B, self.out_cap, self.device, neighbour_sources=neighbour_sources,
+                               factored=factored_obs, full_obs=full_obs, lib=self.lib)
         self._out_native = self.out.native()
         self._spawn = None
         self._counters = torch.zeros(16, dtype=torch.float64, device=self.device)
@@ -221,7 +291,7 @@ class BatchedScene:
 
     def make_host_outputs(self, pinned=True):
         """Pinned host mirrors of the output arrays for ``step_host``."""
-        host = StepOutputs(self.B, self.out_cap, "cpu")
+        host = StepOutputs(self.B, self.out_cap, "cpu", lib=self.lib)
         if pinned and self.device.type == "cuda":
             host.pin()
         return host
@@ -243,25 +313,31 @@ class BatchedScene:
         self.out._n = n
         return n
 
-    def make_async_buffers(self):
-        """Three (device, pinned host) output pairs for ``step_host_async``: consecutive ticks take them in turn."""
+    def make_async_buffers(self, factored=False, full_obs=None):
+        """Three (device, pinned host) output pairs for ``step_host_async``: consecutive ticks take them in turn.
+        ``factored``: with the factored observation (``copy_factored``); the device buffers then hold no ``obs`` unless
+        ``full_obs`` is set, so the step does not write the 784-byte block of every agent."""
+        full_obs = (not factored) if full_obs is None else bool(full_obs)
         pairs = []
         for _ in range(3):
-            dev = StepOutputs(self.B, self.out_cap, self.device, records_only=True)
-            host = StepOutputs(self.B, self.out_cap, "cpu", records_only=True).pin()
+            kw = dict(records_only=True, factored=factored, full_obs=full_obs, lib=self.lib)
+            dev = StepOutputs(self.B, self.out_cap, self.device, **kw)
+            host = StepOutputs(self.B, self.out_cap, "cpu", **kw).pin()
             pairs.append((dev, host, dev.native(), host.native()))      # the ctypes views are built once
         return pairs
 
-    def step_host_async(self, actions_host, pair, copy_obs=False):
+    def step_host_async(self, actions_host, pair, copy_obs=False, copy_factored=False):
         """Enqueue one tick through host buffers without waiting (``pve_step_host_async``): actions by DMA from the
         pinned ``actions_host``, agent records / offsets / per-intersection counters (and the observations with
-        ``copy_obs``) by DMA into ``pair[1]`` while later ticks already run.  At most three ticks may be in flight;
-        ``host_wait()`` returns the row count of the oldest one once its host buffers are complete."""
+        ``copy_obs``, the factored observation with ``copy_factored``: 240 instead of 784 bytes per agent, rebuilt with
+        ``host.expand_obs()``) by DMA into ``pair[1]`` while later ticks already run.  At most three ticks may be in
+        flight; ``host_wait()`` returns the row count of the oldest one once its host buffers are complete."""
         assert actions_host.dtype == torch.float32 and actions_host.is_contiguous() and actions_host.is_pinned()
         assert actions_host.shape == (self.B, self.veh_cap)
         dev, host, dev_native, host_native = pair
         self._check(self.lib.pve_step_host_async(self._h, actions_host.data_ptr(), C.byref(dev_native),
-                                                 C.byref(host_native), 2 if copy_obs else 0, self._stream()))
+                                                 C.byref(host_native), (2 if copy_obs else 0) | (4 if copy_factored else 0),
+                                                 self._stream()))
         self._async_q = getattr(self, "_async_q", []) + [host]
 
     def host_wait(self):
