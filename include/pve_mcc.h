@@ -326,7 +326,8 @@ typedef struct pve_critic pve_critic;
 int32_t pve_critic_create(const float *weights_host, int32_t n_floats, int32_t device, pve_critic **out);
 void pve_critic_destroy(pve_critic *c);
 /* q_dev[i] = Q(obs_dev[i][0][0..27], act7_dev[i][0..6]) for i < min(max_rows, n_rows_dev[0]) (n_rows_dev may be
- * null: all max_rows rows).  obs_dev: [max_rows][7][28] observations, only row 0 is read (main.py:257). */
+ * null: all max_rows rows).  obs_dev: [max_rows][7][28] observations, only row 0 is read (main.py:257).  (A factored
+ * folder's push runs the same network on pve_outputs.row0_out, rows 28 floats apart.) */
 int32_t pve_critic_forward(pve_critic *c, const float *obs_dev, const float *act7_dev, int64_t max_rows,
                            const int32_t *n_rows_dev, float *q_dev, void *stream);
 
@@ -348,9 +349,17 @@ typedef struct pve_nstep pve_nstep;
  * buffer_size = ReplayBuffer(buffer_size, ...) (main.py:212), buffer_size - 1 >= out_cap */
 int32_t pve_nstep_create(int32_t n_envs, int32_t uid_slots, int32_t seq_max_step, int64_t out_cap,
                          int64_t buffer_size, int32_t device, pve_nstep **out);
+/* The same folder with a FACTORED frame log: per push slot the factored observation (row0_out f32[out_cap][28],
+ * prev_row0 f32[out_cap][28], obs_src i16[out_cap][8], see pve_outputs) and that push's agent_offset[B + 1] -- 240 B per
+ * output row instead of the 784 B block (the log is about 0.31 x as large).  Same arguments and checks.  Push it with
+ * pve_nstep_push_factored only; the replay memory, counters and bootstrap values are those of a full-frame folder fed
+ * the same ticks, bit for bit. */
+int32_t pve_nstep_create_factored(int32_t n_envs, int32_t uid_slots, int32_t seq_max_step, int64_t out_cap,
+                                  int64_t buffer_size, int32_t device, pve_nstep **out);
 void pve_nstep_destroy(pve_nstep *f);
 /* main.py:243-266 for the tick whose outputs are in `out_dev` (agent_offset, ids, status, obs, reward are read).
- * The bootstrap term uses the two target networks on this tick's observations.  Asynchronous on `stream`. */
+ * The bootstrap term uses the two target networks on this tick's observations.  Asynchronous on `stream`.
+ * Full-frame folders only (a factored folder: PVE_EINVAL, see pve_nstep_last_error). */
 int32_t pve_nstep_push(pve_nstep *f, const pve_outputs *out_dev, double gamma, pve_actor *target_actor,
                        pve_critic *target_critic, void *stream);
 /* The same tick with the scene at hand and out_dev->nbr_src filled in by the step: the target actor is evaluated once
@@ -359,13 +368,33 @@ int32_t pve_nstep_push(pve_nstep *f, const pve_outputs *out_dev, double gamma, p
  * sees the same row contents).  Must be called before the scene's next step (last tick's rows are still in place). */
 int32_t pve_nstep_push_scene(pve_nstep *f, pve_scene *s, const pve_outputs *out_dev, double gamma,
                              pve_actor *target_actor, pve_critic *target_critic, void *stream);
+/* main.py:243-266 for one tick from its FACTORED observation (factored folders only; otherwise, or when one of
+ * row0_out / prev_row0 / obs_src is missing, PVE_EINVAL).  Reads agent_offset, ids, status, reward, row0_out, prev_row0
+ * and obs_src; out_dev->obs may be null and is never read.  The target actor runs once per distinct row: on row0_out, on
+ * the prev_row0 rows some 0x4000 code refers to, and the 7 actions are gathered through obs_src; the target critic runs on
+ * row0_out.  Asynchronous; pushes must come in tick order, but since the outputs carry every row the push needs, it
+ * does not have to run before the scene's next step (give that step other output buffers). */
+int32_t pve_nstep_push_factored(pve_nstep *f, const pve_outputs *out_dev, double gamma, pve_actor *target_actor,
+                                pve_critic *target_critic, void *stream);
 /* a new episode (main.py:230 builds a new TrafficInteraction every epoch): every vehicle's buffered transitions are
  * dropped, the replay memory and num_experiences are kept (agent1_memory_seq lives across epochs, main.py:212) */
 /* Where the NEXT push expects its observations: a block of the folder's frame log ([out_cap][7][28] floats, device).
  * Hand it to the step as pve_outputs.obs and the push finds the frames in place; any other pve_outputs.obs is copied
  * into the log by the push (one out_cap x 784 B device copy).  The log holds the last seq_max_step + 2 pushes: the
  * per-vehicle buffers of main.py:243-246 keep references into it instead of private copies of veh["state"]. */
-int32_t pve_nstep_obs_slot(const pve_nstep *f, float **obs_dev);
+int32_t pve_nstep_obs_slot(const pve_nstep *f, float **obs_dev);      /* a factored folder: PVE_ESTATE */
+/* The factored folder's counterpart: where the NEXT push expects row0_out / prev_row0 / obs_src (device blocks of the
+ * log).  Hand them to the step as pve_outputs fields and the push finds them in place; outputs elsewhere are copied in
+ * (one device copy of each, sized by out_cap).  The push always copies agent_offset into the slot.  A full-frame folder:
+ * PVE_ESTATE. */
+int32_t pve_nstep_factored_slot(const pve_nstep *f, float **row0_dev, float **prev_row0_dev, int16_t **obs_src_dev);
+/* bytes of the frame log (either format) */
+int64_t pve_nstep_log_bytes(const pve_nstep *f);
+/* the message of the last refused push */
+const char *pve_nstep_last_error(const pve_nstep *f);
+/* measurement aids: CUDA events around the fold kernel of every push while on; pve_nstep_fold_ms waits for the last one */
+int32_t pve_nstep_set_profiling(pve_nstep *f, int32_t on);
+int32_t pve_nstep_fold_ms(pve_nstep *f, float *ms);
 int32_t pve_nstep_reset(pve_nstep *f, void *stream);
 int32_t pve_nstep_replay(const pve_nstep *f, pve_replay_view *view);
 /* out_host[0] = num_experiences (replay_buffer.py:47), [1] = records added by the last push, [2] = history slots

@@ -109,6 +109,15 @@ def load_library(path=None):
     lib.pve_nstep_destroy.restype = None
     lib.pve_nstep_push.argtypes = [vp, C.POINTER(PveOutputs), C.c_double, vp, vp, vp]
     lib.pve_nstep_push_scene.argtypes = [vp, vp, C.POINTER(PveOutputs), C.c_double, vp, vp, vp]
+    lib.pve_nstep_create_factored.argtypes = [i32, i32, i32, i64, i64, i32, C.POINTER(vp)]
+    lib.pve_nstep_push_factored.argtypes = [vp, C.POINTER(PveOutputs), C.c_double, vp, vp, vp]
+    lib.pve_nstep_factored_slot.argtypes = [vp, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp)]
+    lib.pve_nstep_log_bytes.argtypes = [vp]
+    lib.pve_nstep_log_bytes.restype = i64
+    lib.pve_nstep_last_error.argtypes = [vp]
+    lib.pve_nstep_last_error.restype = C.c_char_p
+    lib.pve_nstep_set_profiling.argtypes = [vp, i32]
+    lib.pve_nstep_fold_ms.argtypes = [vp, C.POINTER(C.c_float)]
     lib.pve_nstep_reset.argtypes = [vp, vp]
     lib.pve_nstep_obs_slot.argtypes = [vp, C.POINTER(vp)]
     lib.pve_nstep_replay.argtypes = [vp, C.POINTER(PveReplayView)]

@@ -59,7 +59,8 @@ static inline void pvq_pack(const float *W, uint32_t *out) {
 #define PVQ_TILE 128
 #define PVQ_SMEM_BYTES (PVQ_WORDS * 4 + PVQ_TILE * PVM_AS * 4)
 
-/* 16 agents of this warp: rows row0 + 16 warp .. + 15 */
+/* 16 agents of this warp: rows row0 + 16 warp .. + 15; STRIDE as in pvc_round */
+template <int STRIDE>
 __device__ __forceinline__ void pvq_warp_round(const uint32_t *__restrict__ pw, float *__restrict__ a, const long long row0,
                                                const int n_valid, const float *__restrict__ obs,
                                                const float *__restrict__ act7, float *__restrict__ q) {
@@ -70,7 +71,7 @@ __device__ __forceinline__ void pvq_warp_round(const uint32_t *__restrict__ pw, 
     {
         const int r = lane & 15, half = lane >> 4, row = warp * 16 + r;
         const bool valid = row < n_valid;
-        const float4 *src = reinterpret_cast<const float4 *>(obs + (row0 + (valid ? row : 0)) * PVN_OBS) + half * 4;
+        const float4 *src = reinterpret_cast<const float4 *>(obs + (row0 + (valid ? row : 0)) * STRIDE) + half * 4;
         float4 x[4];
 #pragma unroll
         for (int p = 0; p < 4; ++p)
@@ -165,6 +166,7 @@ __device__ __forceinline__ void pvq_warp_round(const uint32_t *__restrict__ pw, 
 }
 
 /* same contract as pve_critic_kernel (nstep.cuh); PW = the packed block of pvq_pack */
+template <int STRIDE>
 __global__ void __launch_bounds__(PVQ_THREADS, 2)
 pve_critic_mma_kernel(const uint32_t *__restrict__ PW, const float *__restrict__ obs, const float *__restrict__ act7,
                       float *__restrict__ q, const long long n_rows_max, const int32_t *__restrict__ n_rows_dev) {
@@ -178,7 +180,7 @@ pve_critic_mma_kernel(const uint32_t *__restrict__ PW, const float *__restrict__
     __syncthreads();
     for (long long t0 = (long long)blockIdx.x * PVQ_TILE; t0 < n_rows; t0 += (long long)gridDim.x * PVQ_TILE) {
         const int n_valid = (int)min((long long)PVQ_TILE, n_rows - t0);
-        if ((int)(threadIdx.x >> 5) * 16 < n_valid) pvq_warp_round(pw, a, t0, n_valid, obs, act7, q);
+        if ((int)(threadIdx.x >> 5) * 16 < n_valid) pvq_warp_round<STRIDE>(pw, a, t0, n_valid, obs, act7, q);
     }
 }
 #endif  /* __CUDACC__ */

@@ -534,6 +534,7 @@ pve_actor_tc_kernel(const __grid_constant__ PvtVecs V, const uint16_t *__restric
 }
 
 /* ---- critic: same contract as pve_critic_kernel (nstep.cuh) ------------------------------------------ */
+template <int STRIDE>
 __global__ void __launch_bounds__(PVT_THREADS_CRITIC, 1)
 pve_critic_tc_kernel(const __grid_constant__ PvtVecs V, const uint16_t *__restrict__ PW, const float *__restrict__ obs,
                      const float *__restrict__ act7, float *__restrict__ q, const long long n_rows_max,
@@ -549,7 +550,7 @@ pve_critic_tc_kernel(const __grid_constant__ PvtVecs V, const uint16_t *__restri
     for (long long t0 = ((long long)blockIdx.x * PVT_GROUPS + g) * PVT_TILE; t0 < n_rows; t0 += (long long)gridDim.x * PVT_GROUPS * PVT_TILE) {
         const long long row = t0 + G.gt;
         const bool valid = row < n_rows;
-        const float o = pvt_round<true>(V, G, valid ? obs + row * PVN_OBS : nullptr, valid ? act7 + row * 7 : nullptr);
+        const float o = pvt_round<true>(V, G, valid ? obs + row * STRIDE : nullptr, valid ? act7 + row * 7 : nullptr);
         if (valid) q[row] = o;                                                   /* NET:73 */
     }
     pvt_teardown(tmem);

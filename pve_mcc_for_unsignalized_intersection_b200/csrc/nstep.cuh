@@ -39,6 +39,12 @@
  * HBM-bound: per record 2 x 784 B frames in, 2 x 784 + 36 B out = 3.2 KB per agent-tick in steady state (round 1, with
  * the per-slot frame rings: 4.7 KB).
  *
+ * FACTORED frame log (pve_nstep_create_factored): the log keeps each push's factored observation instead of its blocks,
+ * per slot row0 f32[out_cap][28], prev f32[out_cap][28], src i16[out_cap][8] (pve_outputs.row0_out / prev_row0 /
+ * obs_src) and that push's agent_offset[B + 1]: 240 B per row instead of 784.  A frame reference is the same 32-bit
+ * log row slot * out_cap + r; its codes are relative to the vehicle's intersection `env`, so the fold resolves code g'
+ * as log row slot * out_cap + off_slot[env] + g' and expands the 49 float4 pieces of the frame into the record.
+ *
  * The critic (model_agent_maddpg.py:52-76: LN(28) -> Dense 64 -> LN -> ReLU -> concat 7 actions -> Dense 64 ->
  * LN -> ReLU -> Dense 1) reuses the register-tiled fp32 GEMM chain of actor.cuh; fp32 FFMA for the same
  * conditioning reason.  Device only (numpy restatement for tests: oracle/nstep_oracle.py).
@@ -75,6 +81,22 @@ struct PvnTable {
     int U, M, S, B;
 };
 
+struct PvnFactored {                 /* the factored frame log; all null for a full-frame folder (T.log is used) */
+    float *row0, *prev;              /* [M][out_cap][28] */
+    int16_t *src;                    /* [M][out_cap][8] */
+    int32_t *off;                    /* [M][B + 1] agent_offset of the push that wrote the slot */
+};
+
+/* the source of one observation row under its factored code (pve_outputs.obs_src) in an intersection of A rows:
+ * 0 = the zero row, 1 = row0_out row `idx`, 2 = prev_row0 row `idx` (relative to the intersection), -1 = invalid */
+PVE_HD int pve_obs_src_decode(int16_t c, int64_t A, int64_t *idx) {
+    if (c == -1) return 0;
+    if (c < 0 || (int64_t)(c & 0x3FFF) >= A) return -1;
+    *idx = c & 0x3FFF;
+    return (c & 0x4000) ? 2 : 1;
+}
+#define PVE_NAN_BITS 0x7FC00000u      /* an observation row behind an invalid code */
+
 struct PvnReplay {                   /* replay_buffer.py:8-9 as a ring of cap = buffer_size - 1 records */
     float *state, *action, *reward, *next_state;
     uint8_t *done;
@@ -88,8 +110,9 @@ struct PvnReplay {                   /* replay_buffer.py:8-9 as a ring of cap = 
 #define PVC_WPAD ((PVC_S_COUNT + 3) & ~3)
 #define PVC_SMEM_BYTES ((PVC_WPAD + PVC_TILE * PVC_AS) * 4)
 
-/* one tile of <= 16 R agents starting at row0: q[row] = Q'(obs[row][0][:], act7[row][:]) */
-template <int R>
+/* one tile of <= 16 R agents starting at row0: q[row] = Q'(obs[row][0][:], act7[row][:]); STRIDE = floats from one
+ * agent's row 0 to the next (PVN_OBS: observation blocks, PVE_OBS_W: pve_outputs.row0_out) */
+template <int R, int STRIDE>
 __device__ __forceinline__ void pvc_round(const float *__restrict__ w, float *__restrict__ a, const long long row0,
                                           const int n_valid, const float *__restrict__ obs, const float *__restrict__ act7,
                                           float *__restrict__ q) {
@@ -98,7 +121,7 @@ __device__ __forceinline__ void pvc_round(const float *__restrict__ w, float *__
         float x[28];
         const bool valid = tid < n_valid;
         const long long r = row0 + (valid ? tid : 0);
-        const float4 *src = reinterpret_cast<const float4 *>(obs + r * PVN_OBS);
+        const float4 *src = reinterpret_cast<const float4 *>(obs + r * STRIDE);
 #pragma unroll
         for (int i = 0; i < 7; ++i) {
             const float4 v = valid ? src[i] : make_float4(0.f, 0.f, 0.f, 0.f);
@@ -168,6 +191,7 @@ __device__ __forceinline__ void pvc_round(const float *__restrict__ w, float *__
 }
 
 /* q[r] for r < min(n_rows_max, n_rows_dev[0]); persistent CTAs stride over tiles of 128 agents */
+template <int STRIDE>
 __global__ void __launch_bounds__(PVC_THREADS, 3)
 pve_critic_kernel(const float *__restrict__ W, const float *__restrict__ obs, const float *__restrict__ act7,
                   float *__restrict__ q, const long long n_rows_max, const int32_t *__restrict__ n_rows_dev) {
@@ -187,9 +211,9 @@ pve_critic_kernel(const float *__restrict__ W, const float *__restrict__ obs, co
     __syncthreads();
     for (long long t0 = (long long)blockIdx.x * PVC_TILE; t0 < n_rows; t0 += (long long)gridDim.x * PVC_TILE) {
         const int n_valid = (int)min((long long)PVC_TILE, n_rows - t0);
-        if (n_valid > 64) pvc_round<8>(w, a, t0, n_valid, obs, act7, q);
-        else if (n_valid > 32) pvc_round<4>(w, a, t0, n_valid, obs, act7, q);
-        else pvc_round<2>(w, a, t0, n_valid, obs, act7, q);
+        if (n_valid > 64) pvc_round<8, STRIDE>(w, a, t0, n_valid, obs, act7, q);
+        else if (n_valid > 32) pvc_round<4, STRIDE>(w, a, t0, n_valid, obs, act7, q);
+        else pvc_round<2, STRIDE>(w, a, t0, n_valid, obs, act7, q);
     }
 }
 
@@ -222,6 +246,50 @@ pvn_gather_kernel(const int16_t *__restrict__ nbr_src, const int32_t *__restrict
     if (v < 0) a = mu_zero[0];                                                       /* TIS:1334: the all-zero row */
     else if (v & 0x4000) a = mu_prev[(size_t)env * VC + (v & 0x3FFF)];               /* stored last tick */
     else a = act7[((long long)agent_offset[env] + v) * PVE_OBS_H];                  /* this tick's row 0 of agent v */
+    act7[r * PVE_OBS_H + k] = a;
+}
+
+/* ---- the same from the factored observation (pve_nstep_push_factored) -------------------------------------------
+ * obs_src names every row: mark the prev_row0 rows that some observation refers to; gather act7[r][k], k = 0..6, from
+ * mu0 (the actor on row0_out), mu_prev (on the marked prev_row0 rows) and the zero row's action.  A code is checked
+ * against its intersection's row count as pve_expand_obs does; an invalid one gathers NaN. */
+__device__ __forceinline__ long long pvn_src_row(const int v, const int32_t *__restrict__ agent_offset, const int env,
+                                                 const long long out_cap) {
+    const long long o0 = agent_offset[env], o1 = min((long long)agent_offset[env + 1], out_cap);
+    const long long g = v & 0x3FFF;
+    return (o0 >= 0 && o0 + g < o1) ? o0 + g : -1;
+}
+__global__ void __launch_bounds__(256)
+pvn_mark_factored_kernel(const int16_t *__restrict__ obs_src, const int32_t *__restrict__ ids,
+                         const int32_t *__restrict__ agent_offset, const int B, const long long out_cap,
+                         uint8_t *__restrict__ need) {
+    const long long n_rows = min((long long)agent_offset[B], out_cap);
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long r = i >> 3;
+    const int k = (int)(i & 7);
+    if (r >= n_rows || k == 0 || k >= PVE_OBS_H) return;
+    const int v = obs_src[r * 8 + k];
+    if (v < 0 || !(v & 0x4000)) return;
+    const long long s = pvn_src_row(v, agent_offset, ids[r * 4], out_cap);
+    if (s >= 0) need[s] = 1;
+}
+__global__ void __launch_bounds__(256)
+pvn_gather_factored_kernel(const int16_t *__restrict__ obs_src, const int32_t *__restrict__ ids,
+                           const int32_t *__restrict__ agent_offset, const int B, const long long out_cap,
+                           const float *__restrict__ mu0, const float *__restrict__ mu_prev,
+                           const float *__restrict__ mu_zero, float *__restrict__ act7) {
+    const long long n_rows = min((long long)agent_offset[B], out_cap);
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const long long r = i >> 3;
+    const int k = (int)(i & 7);
+    if (r >= n_rows || k >= PVE_OBS_H) return;
+    const int v = obs_src[r * 8 + k];
+    float a;
+    if (v == -1) a = mu_zero[0];                                                     /* TIS:1334: the all-zero row */
+    else {
+        const long long s = v < 0 ? -1 : pvn_src_row(v, agent_offset, ids[r * 4], out_cap);
+        a = s < 0 ? __int_as_float((int)PVE_NAN_BITS) : (v & 0x4000) ? mu_prev[s] : mu0[s];
+    }
     act7[r * PVE_OBS_H + k] = a;
 }
 
@@ -308,11 +376,41 @@ __device__ __forceinline__ void pvn_zero_frame(float *__restrict__ dst, const in
     if (lane < 49 - 32) d4[32 + lane] = make_float4(0.f, 0.f, 0.f, 0.f);
 }
 
+/* frame f (a log row, >= 0) of the factored log, expanded into dst as pve_expand_obs does: lane l stores the float4
+ * pieces l and l + 32 of the 49.  `env` is the vehicle's intersection; the frame's codes are relative to it in the
+ * offsets of the push that wrote the slot.  action != null: also the action column (TIS:290) of the 7 rows. */
+__device__ __forceinline__ void pvn_expand_frame(float *__restrict__ dst, const PvnFactored F, const long long out_cap,
+                                                 const int B, const long long f, const int env, const int lane,
+                                                 float *__restrict__ action) {
+    const long long slot = f / out_cap;
+    const int32_t *const off = F.off + slot * (B + 1);
+    const long long o0 = off[env], o1 = off[env + 1];
+    const long long A = (o0 >= 0 && o1 >= o0 && o1 <= out_cap) ? o1 - o0 : 0;   /* rows the step did not write: NaN */
+    const int16_t *const src = F.src + f * 8;
+    const float4 *const r0 = reinterpret_cast<const float4 *>(F.row0 + (slot * out_cap + o0) * PVE_OBS_W);
+    const float4 *const pr = reinterpret_cast<const float4 *>(F.prev + (slot * out_cap + o0) * PVE_OBS_W);
+    float4 *const d4 = reinterpret_cast<float4 *>(dst);
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+        const int p = lane + 32 * h;
+        if (h == 1 && p >= 49) break;
+        const int row = p / 7, piece = p - 7 * row;
+        int64_t idx = 0;
+        const int k = pve_obs_src_decode(src[row], A, &idx);
+        float4 v;
+        if (k > 0) v = (k == 1 ? r0 : pr)[idx * 7 + piece];
+        else { const float w = k == 0 ? 0.f : __int_as_float((int)PVE_NAN_BITS); v = make_float4(w, w, w, w); }
+        d4[p] = v;
+        if (action && piece == 0) action[row] = v.z;                                /* column 2 of the row */
+    }
+}
+
+template <bool FACT>
 __global__ void __launch_bounds__(256)
 pvn_fold_kernel(const PvnTable T, const PvnReplay R, const int32_t *__restrict__ ids, const uint8_t *__restrict__ status,
                 const float *__restrict__ reward, const float *__restrict__ q,
                 const int32_t *__restrict__ agent_offset, const long long out_cap, const unsigned stamp, const double gamma,
-                const uint32_t *__restrict__ plan, const long long *__restrict__ blk_base) {
+                const uint32_t *__restrict__ plan, const long long *__restrict__ blk_base, const PvnFactored F) {
     const long long n_rows = min((long long)agent_offset[T.B], out_cap);
     const int lane = threadIdx.x & 31;
     const long long warp0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -350,11 +448,18 @@ pvn_fold_kernel(const PvnTable T, const PvnReplay R, const int32_t *__restrict__
             int nx = head + 1; nx -= nx >= M ? M : 0;
             /* both references were stored by earlier pushes (n == 1: the next state is this tick's own row) */
             const int f_state = is_new ? -1 : fidx[head];
-            const float *const src_next = n == 1 ? obs_r : T.log + (size_t)fidx[nx] * PVN_OBS;
-            if (f_state < 0) pvn_zero_frame(R.state + pos * PVN_OBS, lane);
-            else pvn_copy_frame(R.state + pos * PVN_OBS, T.log + (size_t)f_state * PVN_OBS, lane);
-            pvn_copy_frame(R.next_state + pos * PVN_OBS, src_next, lane);
-            if (lane < PVE_OBS_H) R.action[pos * PVE_OBS_H + lane] = src_next[lane * PVE_OBS_W + 2];   /* TIS:290 */
+            if constexpr (FACT) {
+                if (f_state < 0) pvn_zero_frame(R.state + pos * PVN_OBS, lane);
+                else pvn_expand_frame(R.state + pos * PVN_OBS, F, T.out_cap, T.B, f_state, id.x, lane, nullptr);
+                pvn_expand_frame(R.next_state + pos * PVN_OBS, F, T.out_cap, T.B, n == 1 ? my_row : (long long)fidx[nx],
+                                 id.x, lane, R.action + pos * PVE_OBS_H);                      /* TIS:290 */
+            } else {
+                const float *const src_next = n == 1 ? obs_r : T.log + (size_t)fidx[nx] * PVN_OBS;
+                if (f_state < 0) pvn_zero_frame(R.state + pos * PVN_OBS, lane);
+                else pvn_copy_frame(R.state + pos * PVN_OBS, T.log + (size_t)f_state * PVN_OBS, lane);
+                pvn_copy_frame(R.next_state + pos * PVN_OBS, src_next, lane);
+                if (lane < PVE_OBS_H) R.action[pos * PVE_OBS_H + lane] = src_next[lane * PVE_OBS_W + 2];   /* TIS:290 */
+            }
             if (lane == 0) { R.reward[pos] = (float)tgt; R.done[pos] = 0; }          /* main.py:263-264 */
             head = nx;                                                               /* main.py:265-266 */
             n -= 1;

@@ -138,16 +138,6 @@ static int rt_host_alloc(void **p, size_t n) { return rt_alloc(p, n); }
 static void rt_host_free(void *p) { free(p); }
 #endif
 
-/* the source of one observation row under its factored code (pve_outputs.obs_src) in an intersection of A rows:
- * 0 = the zero row, 1 = row0_out row `idx`, 2 = prev_row0 row `idx` (relative to the intersection), -1 = invalid */
-PVE_HD int pve_obs_src_decode(int16_t c, int64_t A, int64_t *idx) {
-    if (c == -1) return 0;
-    if (c < 0 || (int64_t)(c & 0x3FFF) >= A) return -1;
-    *idx = c & 0x3FFF;
-    return (c & 0x4000) ? 2 : 1;
-}
-#define PVE_NAN_BITS 0x7FC00000u      /* an observation row behind an invalid code */
-
 /* =============================================================================================
  * kernels
  * =========================================================================================== */
@@ -1578,13 +1568,17 @@ int32_t pve_critic_create(const float *weights_host, int32_t n_floats, int32_t d
     if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || sms <= 0) sms = 148;
     c->use_mma = 3;
     if (const char *impl = getenv("PVE_CRITIC_IMPL")) c->use_mma = strcmp(impl, "ffma") == 0 ? 0 : strcmp(impl, "mma") == 0 ? 1 : strcmp(impl, "tc5") == 0 ? 2 : 3;
-    bool ok = cudaFuncSetAttribute(pve_critic_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PVC_SMEM_BYTES) == cudaSuccess
-              && cudaFuncSetAttribute(pve_critic_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PVQ_SMEM_BYTES) == cudaSuccess
-              && cudaFuncSetAttribute(pve_critic_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PVT_CRITIC_SMEM) == cudaSuccess;
+    /* both row-0 strides: observation blocks (pve_critic_forward) and the factored log's rows (pve_nstep_push_factored) */
+    bool ok = cudaFuncSetAttribute(pve_critic_kernel<PVN_OBS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PVC_SMEM_BYTES) == cudaSuccess
+              && cudaFuncSetAttribute(pve_critic_mma_kernel<PVN_OBS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PVQ_SMEM_BYTES) == cudaSuccess
+              && cudaFuncSetAttribute(pve_critic_tc_kernel<PVN_OBS>, cudaFuncAttributeMaxDynamicSharedMemorySize, PVT_CRITIC_SMEM) == cudaSuccess
+              && cudaFuncSetAttribute(pve_critic_kernel<PVE_OBS_W>, cudaFuncAttributeMaxDynamicSharedMemorySize, PVC_SMEM_BYTES) == cudaSuccess
+              && cudaFuncSetAttribute(pve_critic_mma_kernel<PVE_OBS_W>, cudaFuncAttributeMaxDynamicSharedMemorySize, PVQ_SMEM_BYTES) == cudaSuccess
+              && cudaFuncSetAttribute(pve_critic_tc_kernel<PVE_OBS_W>, cudaFuncAttributeMaxDynamicSharedMemorySize, PVT_CRITIC_SMEM) == cudaSuccess;
     c->blocks_tc = sms;                      /* one persistent CTA per SM */
-    if (ok && (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pve_critic_kernel, PVC_THREADS, PVC_SMEM_BYTES) != cudaSuccess || per_sm < 1)) per_sm = 1;
+    if (ok && (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pve_critic_kernel<PVN_OBS>, PVC_THREADS, PVC_SMEM_BYTES) != cudaSuccess || per_sm < 1)) per_sm = 1;
     c->blocks = per_sm * sms;
-    if (ok && (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pve_critic_mma_kernel, PVQ_THREADS, PVQ_SMEM_BYTES) != cudaSuccess || per_sm < 1)) per_sm = 1;
+    if (ok && (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, pve_critic_mma_kernel<PVN_OBS>, PVQ_THREADS, PVQ_SMEM_BYTES) != cudaSuccess || per_sm < 1)) per_sm = 1;
     c->blocks_mma = per_sm * sms;
     uint32_t *packed = ok ? (uint32_t *)malloc(sizeof(uint32_t) * PVQ_WORDS) : nullptr;
     ok = ok && packed;
@@ -1619,6 +1613,34 @@ void pve_critic_destroy(pve_critic *c) {
     free(c);
 }
 
+#ifndef PVE_HOST_EMULATION
+}  /* extern "C" */
+/* q_dev[i] = Q(obs_dev + i * STRIDE, act7_dev[i]) for i < min(max_rows, n_rows_dev[0]) */
+template <int STRIDE>
+static int32_t critic_forward(pve_critic *c, const float *obs_dev, const float *act7_dev, int64_t max_rows,
+                              const int32_t *n_rows_dev, float *q_dev, pve_stream_t stream) {
+    if (max_rows == 0) return PVE_OK;
+    const long long tiles = (max_rows + PVC_TILE - 1) / PVC_TILE;              /* both kernels: 128 agents per tile */
+    const int impl = c->use_mma == 3 ? (max_rows >= PVE_TC_MIN_ROWS ? 2 : 1) : c->use_mma;
+    if (impl == 2) {
+        const long long ctas = (tiles + PVT_GROUPS - 1) / PVT_GROUPS;
+        const int blocks = (int)(ctas < c->blocks_tc ? ctas : c->blocks_tc);
+        pve_critic_tc_kernel<STRIDE><<<blocks, PVT_THREADS_CRITIC, PVT_CRITIC_SMEM, stream>>>(c->vecs, c->tw_dev, obs_dev, act7_dev, q_dev,
+                                                                                           (long long)max_rows, n_rows_dev);
+    } else if (impl) {
+        const int blocks = (int)(tiles < c->blocks_mma ? tiles : c->blocks_mma);
+        pve_critic_mma_kernel<STRIDE><<<blocks, PVQ_THREADS, PVQ_SMEM_BYTES, stream>>>(c->pw_dev, obs_dev, act7_dev, q_dev,
+                                                                                      (long long)max_rows, n_rows_dev);
+    } else {
+        const int blocks = (int)(tiles < c->blocks ? tiles : c->blocks);
+        pve_critic_kernel<STRIDE><<<blocks, PVC_THREADS, PVC_SMEM_BYTES, stream>>>(c->w_dev, obs_dev, act7_dev, q_dev,
+                                                                                  (long long)max_rows, n_rows_dev);
+    }
+    return cudaGetLastError() == cudaSuccess ? PVE_OK : PVE_ECUDA;
+}
+extern "C" {
+#endif
+
 int32_t pve_critic_forward(pve_critic *c, const float *obs_dev, const float *act7_dev, int64_t max_rows,
                            const int32_t *n_rows_dev, float *q_dev, void *stream_) {
     if (!c || !obs_dev || !act7_dev || !q_dev || max_rows < 0) return PVE_EINVAL;
@@ -1626,24 +1648,7 @@ int32_t pve_critic_forward(pve_critic *c, const float *obs_dev, const float *act
     (void)n_rows_dev; (void)stream_;
     return PVE_ESTATE;
 #else
-    if (max_rows == 0) return PVE_OK;
-    const long long tiles = (max_rows + PVC_TILE - 1) / PVC_TILE;              /* both kernels: 128 agents per tile */
-    const int impl = c->use_mma == 3 ? (max_rows >= PVE_TC_MIN_ROWS ? 2 : 1) : c->use_mma;
-    if (impl == 2) {
-        const long long ctas = (tiles + PVT_GROUPS - 1) / PVT_GROUPS;
-        const int blocks = (int)(ctas < c->blocks_tc ? ctas : c->blocks_tc);
-        pve_critic_tc_kernel<<<blocks, PVT_THREADS_CRITIC, PVT_CRITIC_SMEM, (pve_stream_t)stream_>>>(c->vecs, c->tw_dev, obs_dev, act7_dev, q_dev,
-                                                                                                  (long long)max_rows, n_rows_dev);
-    } else if (impl) {
-        const int blocks = (int)(tiles < c->blocks_mma ? tiles : c->blocks_mma);
-        pve_critic_mma_kernel<<<blocks, PVQ_THREADS, PVQ_SMEM_BYTES, (pve_stream_t)stream_>>>(c->pw_dev, obs_dev, act7_dev, q_dev,
-                                                                                             (long long)max_rows, n_rows_dev);
-    } else {
-        const int blocks = (int)(tiles < c->blocks ? tiles : c->blocks);
-        pve_critic_kernel<<<blocks, PVC_THREADS, PVC_SMEM_BYTES, (pve_stream_t)stream_>>>(c->w_dev, obs_dev, act7_dev, q_dev,
-                                                                                         (long long)max_rows, n_rows_dev);
-    }
-    return cudaGetLastError() == cudaSuccess ? PVE_OK : PVE_ECUDA;
+    return critic_forward<PVN_OBS>(c, obs_dev, act7_dev, max_rows, n_rows_dev, q_dev, (pve_stream_t)stream_);
 #endif
 }
 
@@ -1657,30 +1662,45 @@ struct pve_nstep {
     long long *counters;         /* [4] device */
     long long out_cap, pushes;
     int n_blk, device, fold_blocks;
-    /* pve_nstep_push_scene only (allocated on first use): referenced-row marks and actions of last tick's stored rows */
-    uint8_t *need;               /* [B][veh_cap] */
-    float *mu_prev;              /* [B][veh_cap] */
+    /* pve_nstep_push_scene (allocated on first use): referenced-row marks and actions of last tick's stored rows,
+     * [B][veh_cap]; a factored folder: the same for the referenced prev_row0 rows, [out_cap] */
+    uint8_t *need;
+    float *mu_prev;
     size_t scene_slots;
+    PvnFactored F;               /* the factored frame log (pve_nstep_create_factored; T.log is null then) */
+    float *mu0;                  /* factored: [out_cap] the target actor on this tick's row0_out */
+    char err[256];
+#ifndef PVE_HOST_EMULATION
+    cudaEvent_t fold_ev[2];      /* pve_nstep_set_profiling: around the fold kernel of the last push */
+#endif
+    int profiling;
 };
+
+static int32_t nstep_refuse(pve_nstep *f, const char *msg) {
+    snprintf(f->err, sizeof f->err, "%s", msg);
+    return PVE_EINVAL;
+}
 
 void pve_nstep_destroy(pve_nstep *f) {
     if (!f) return;
 #ifndef PVE_HOST_EMULATION
     cudaFree(f->T.key); cudaFree(f->T.fill); cudaFree(f->T.rew); cudaFree(f->T.fidx); cudaFree(f->T.log);
     cudaFree(f->R.state); cudaFree(f->R.action); cudaFree(f->R.reward); cudaFree(f->R.next_state); cudaFree(f->R.done);
-    cudaFree(f->need); cudaFree(f->mu_prev);
+    cudaFree(f->need); cudaFree(f->mu_prev); cudaFree(f->mu0);
+    cudaFree(f->F.row0); cudaFree(f->F.prev); cudaFree(f->F.src); cudaFree(f->F.off);
+    if (f->profiling) { cudaEventDestroy(f->fold_ev[0]); cudaEventDestroy(f->fold_ev[1]); }
     cudaFree(f->act7); cudaFree(f->q); cudaFree(f->plan); cudaFree(f->blk_count); cudaFree(f->blk_base); cudaFree(f->counters);
 #endif
     free(f);
 }
 
-int32_t pve_nstep_create(int32_t n_envs, int32_t uid_slots, int32_t seq_max_step, int64_t out_cap,
-                         int64_t buffer_size, int32_t device, pve_nstep **out) {
+static int32_t nstep_create(int32_t n_envs, int32_t uid_slots, int32_t seq_max_step, int64_t out_cap,
+                            int64_t buffer_size, int32_t device, bool factored, pve_nstep **out) {
     if (!out || n_envs < 1 || uid_slots < 16 || (uid_slots & (uid_slots - 1)) != 0 || seq_max_step < 0
         || seq_max_step + 2 > PVN_MAX_M || out_cap < 1 || buffer_size - 1 < out_cap)
         return PVE_EINVAL;
 #ifdef PVE_HOST_EMULATION
-    (void)device;
+    (void)device; (void)factored;
     return PVE_ESTATE;                       /* device only */
 #else
     if (cudaSetDevice(device) != cudaSuccess) return PVE_ECUDA;
@@ -1700,7 +1720,14 @@ int32_t pve_nstep_create(int32_t n_envs, int32_t uid_slots, int32_t seq_max_step
               && cudaMalloc((void **)&f->T.fill, slots * 2) == cudaSuccess
               && cudaMalloc((void **)&f->T.rew, slots * f->T.M * sizeof(float)) == cudaSuccess
               && cudaMalloc((void **)&f->T.fidx, slots * f->T.M * sizeof(int32_t)) == cudaSuccess
-              && cudaMalloc((void **)&f->T.log, (size_t)f->T.M * oc * PVN_OBS * sizeof(float)) == cudaSuccess
+              && (factored || cudaMalloc((void **)&f->T.log, (size_t)f->T.M * oc * PVN_OBS * sizeof(float)) == cudaSuccess)
+              && (!factored || (cudaMalloc((void **)&f->F.row0, (size_t)f->T.M * oc * PVE_OBS_W * sizeof(float)) == cudaSuccess
+                                && cudaMalloc((void **)&f->F.prev, (size_t)f->T.M * oc * PVE_OBS_W * sizeof(float)) == cudaSuccess
+                                && cudaMalloc((void **)&f->F.src, (size_t)f->T.M * oc * 8 * sizeof(int16_t)) == cudaSuccess
+                                && cudaMalloc((void **)&f->F.off, (size_t)f->T.M * (n_envs + 1) * sizeof(int32_t)) == cudaSuccess
+                                && cudaMalloc((void **)&f->need, oc) == cudaSuccess
+                                && cudaMalloc((void **)&f->mu_prev, oc * sizeof(float)) == cudaSuccess
+                                && cudaMalloc((void **)&f->mu0, oc * sizeof(float)) == cudaSuccess))
               && cudaMalloc((void **)&f->R.state, cap * PVN_OBS * sizeof(float)) == cudaSuccess
               && cudaMalloc((void **)&f->R.next_state, cap * PVN_OBS * sizeof(float)) == cudaSuccess
               && cudaMalloc((void **)&f->R.action, cap * PVE_OBS_H * sizeof(float)) == cudaSuccess
@@ -1722,12 +1749,23 @@ int32_t pve_nstep_create(int32_t n_envs, int32_t uid_slots, int32_t seq_max_step
 #endif
 }
 
+int32_t pve_nstep_create(int32_t n_envs, int32_t uid_slots, int32_t seq_max_step, int64_t out_cap,
+                         int64_t buffer_size, int32_t device, pve_nstep **out) {
+    return nstep_create(n_envs, uid_slots, seq_max_step, out_cap, buffer_size, device, false, out);
+}
+
+int32_t pve_nstep_create_factored(int32_t n_envs, int32_t uid_slots, int32_t seq_max_step, int64_t out_cap,
+                                  int64_t buffer_size, int32_t device, pve_nstep **out) {
+    return nstep_create(n_envs, uid_slots, seq_max_step, out_cap, buffer_size, device, true, out);
+}
+
 #ifndef PVE_HOST_EMULATION
 static int32_t nstep_fold(pve_nstep *f, const pve_outputs *O, double gamma, pve_critic *target_critic, void *stream_);
 #endif
 
 int32_t pve_nstep_push(pve_nstep *f, const pve_outputs *O, double gamma, pve_actor *target_actor,
                        pve_critic *target_critic, void *stream_) {
+    if (f && f->F.row0) return nstep_refuse(f, "pve_nstep_push: this folder keeps a factored frame log, push with pve_nstep_push_factored");
     if (!f || !O || !target_actor || !target_critic || !O->agent_offset || !O->ids || !O->status || !O->obs || !O->reward)
         return PVE_EINVAL;
 #ifdef PVE_HOST_EMULATION
@@ -1748,26 +1786,43 @@ int32_t pve_nstep_push(pve_nstep *f, const pve_outputs *O, double gamma, pve_act
 static int32_t nstep_fold(pve_nstep *f, const pve_outputs *O, double gamma, pve_critic *target_critic, void *stream_) {
     pve_stream_t stream = (pve_stream_t)stream_;
     const int32_t *n_rows_dev = O->agent_offset + f->T.B;
-    int32_t rc = pve_critic_forward(target_critic, O->obs, f->act7, f->out_cap, n_rows_dev, f->q, stream_);
+    const bool fact = f->F.row0 != nullptr;
+    int32_t rc = fact ? critic_forward<PVE_OBS_W>(target_critic, O->row0_out, f->act7, f->out_cap, n_rows_dev, f->q, stream)
+                      : critic_forward<PVN_OBS>(target_critic, O->obs, f->act7, f->out_cap, n_rows_dev, f->q, stream);
     if (rc != PVE_OK) return rc;
     const unsigned stamp = (unsigned)(++f->pushes);
-    /* this tick's observations belong in slot stamp % M of the frame log: already there if the step wrote them to
-     * pve_nstep_obs_slot(), copied otherwise (the whole block: the row count lives on the device) */
-    float *const slot = f->T.log + (size_t)(stamp % (unsigned)f->T.M) * (size_t)f->out_cap * PVN_OBS;
-    if (O->obs != slot
-        && cudaMemcpyAsync(slot, O->obs, (size_t)f->out_cap * PVN_OBS * sizeof(float), cudaMemcpyDeviceToDevice, stream) != cudaSuccess)
-        return PVE_ECUDA;
+    const size_t at = (size_t)(stamp % (unsigned)f->T.M) * (size_t)f->out_cap;
+    /* this tick's frames belong in slot stamp % M of the frame log: already there if the step wrote them to
+     * pve_nstep_obs_slot() / pve_nstep_factored_slot(), copied otherwise (whole blocks: the row count lives on the device) */
+    const auto put = [&](void *slot, const void *src, size_t bytes) {
+        return slot == src || cudaMemcpyAsync(slot, src, bytes, cudaMemcpyDeviceToDevice, stream) == cudaSuccess;
+    };
+    const size_t oc = (size_t)f->out_cap;
+    const bool ok = fact ? put(f->F.row0 + at * PVE_OBS_W, O->row0_out, oc * PVE_OBS_W * sizeof(float))
+                           && put(f->F.prev + at * PVE_OBS_W, O->prev_row0, oc * PVE_OBS_W * sizeof(float))
+                           && put(f->F.src + at * 8, O->obs_src, oc * 8 * sizeof(int16_t))
+                           && put(f->F.off + (size_t)(stamp % (unsigned)f->T.M) * (f->T.B + 1), O->agent_offset,
+                                  (size_t)(f->T.B + 1) * sizeof(int32_t))
+                         : put(f->T.log + at * PVN_OBS, O->obs, oc * PVN_OBS * sizeof(float));
+    if (!ok) return PVE_ECUDA;
     pvn_plan_kernel<<<f->n_blk, PVN_PLAN_THREADS, 0, stream>>>(f->T, O->ids, O->status, O->agent_offset, f->out_cap, stamp,
                                                               f->plan, f->blk_count, f->counters);
     pvn_scan_kernel<<<1, 1024, 0, stream>>>(f->blk_count, f->blk_base, f->n_blk, f->counters);
-    pvn_fold_kernel<<<f->fold_blocks, 256, 0, stream>>>(f->T, f->R, O->ids, O->status, O->reward, f->q, O->agent_offset,
-                                                        f->out_cap, stamp, gamma, f->plan, f->blk_base);
+    if (f->profiling) cudaEventRecord(f->fold_ev[0], stream);
+    if (fact)
+        pvn_fold_kernel<true><<<f->fold_blocks, 256, 0, stream>>>(f->T, f->R, O->ids, O->status, O->reward, f->q, O->agent_offset,
+                                                                 f->out_cap, stamp, gamma, f->plan, f->blk_base, f->F);
+    else
+        pvn_fold_kernel<false><<<f->fold_blocks, 256, 0, stream>>>(f->T, f->R, O->ids, O->status, O->reward, f->q, O->agent_offset,
+                                                                  f->out_cap, stamp, gamma, f->plan, f->blk_base, f->F);
+    if (f->profiling) cudaEventRecord(f->fold_ev[1], stream);
     return cudaGetLastError() == cudaSuccess ? PVE_OK : PVE_ECUDA;
 }
 #endif
 
 int32_t pve_nstep_push_scene(pve_nstep *f, pve_scene *s, const pve_outputs *O, double gamma, pve_actor *target_actor,
                              pve_critic *target_critic, void *stream_) {
+    if (f && f->F.row0) return nstep_refuse(f, "pve_nstep_push_scene: this folder keeps a factored frame log, push with pve_nstep_push_factored");
     if (!f || !s || !O || !target_actor || !target_critic || !O->agent_offset || !O->ids || !O->status || !O->obs
         || !O->reward || !O->nbr_src)
         return PVE_EINVAL;
@@ -1814,10 +1869,99 @@ int32_t pve_nstep_push_scene(pve_nstep *f, pve_scene *s, const pve_outputs *O, d
 #endif
 }
 
+int32_t pve_nstep_push_factored(pve_nstep *f, const pve_outputs *O, double gamma, pve_actor *target_actor,
+                                pve_critic *target_critic, void *stream_) {
+    if (f && !f->F.row0) return nstep_refuse(f, "pve_nstep_push_factored: this folder keeps a full-frame log (pve_nstep_create); "
+                                                "create it with pve_nstep_create_factored");
+    if (f && O && (!O->row0_out || !O->prev_row0 || !O->obs_src))
+        return nstep_refuse(f, "pve_nstep_push_factored: the outputs need row0_out, prev_row0 and obs_src");
+    if (!f || !O || !target_actor || !target_critic || !O->agent_offset || !O->ids || !O->status || !O->reward)
+        return PVE_EINVAL;
+#ifdef PVE_HOST_EMULATION
+    (void)gamma; (void)stream_;
+    return PVE_ESTATE;
+#else
+    if (target_actor->device != f->device || target_critic->device != f->device) return PVE_EINVAL;
+    if (!target_actor->zero_dev) return PVE_ESTATE;      /* computed by pve_actor_create */
+    pve_stream_t stream = (pve_stream_t)stream_;
+    const int B = f->T.B;
+    const int32_t *n_rows_dev = O->agent_offset + B;
+    const long long oc = f->out_cap;
+    const int groups = (int)((oc + PVA_TILE - 1) / PVA_TILE);
+    /* 1. this tick's agent rows (row0_out) */
+    if (launch_actor(target_actor, O->row0_out, nullptr, nullptr, nullptr, 0.f, f->mu0, PVA_TILE, groups, oc, stream,
+                     n_rows_dev, 1, nullptr, 1) != cudaSuccess)
+        return PVE_ECUDA;
+    /* 2. the prev_row0 rows that some observation refers to */
+    if (cudaMemsetAsync(f->need, 0, (size_t)oc, stream) != cudaSuccess) return PVE_ECUDA;
+    const int grid = (int)((oc * 8 + 255) / 256);
+    pvn_mark_factored_kernel<<<grid, 256, 0, stream>>>(O->obs_src, O->ids, O->agent_offset, B, oc, f->need);
+    if (launch_actor(target_actor, O->prev_row0, nullptr, nullptr, nullptr, 0.f, f->mu_prev, PVA_TILE, groups, oc, stream,
+                     n_rows_dev, 1, f->need, 1) != cudaSuccess)
+        return PVE_ECUDA;
+    /* 3. act7[r][0..6] through obs_src */
+    pvn_gather_factored_kernel<<<grid, 256, 0, stream>>>(O->obs_src, O->ids, O->agent_offset, B, oc, f->mu0, f->mu_prev,
+                                                         target_actor->zero_dev + 28, f->act7);
+    if (cudaGetLastError() != cudaSuccess) return PVE_ECUDA;
+    return nstep_fold(f, O, gamma, target_critic, stream_);
+#endif
+}
+
 int32_t pve_nstep_obs_slot(const pve_nstep *f, float **obs_dev) {
     if (!f || !obs_dev) return PVE_EINVAL;
     *obs_dev = f->T.log ? f->T.log + (size_t)((unsigned)(f->pushes + 1) % (unsigned)f->T.M) * (size_t)f->out_cap * PVN_OBS : nullptr;
     return f->T.log ? PVE_OK : PVE_ESTATE;
+}
+
+int32_t pve_nstep_factored_slot(const pve_nstep *f, float **row0_dev, float **prev_dev, int16_t **src_dev) {
+    if (!f || !row0_dev || !prev_dev || !src_dev) return PVE_EINVAL;
+    if (!f->F.row0) return PVE_ESTATE;
+    const size_t at = (size_t)((unsigned)(f->pushes + 1) % (unsigned)f->T.M) * (size_t)f->out_cap;
+    *row0_dev = f->F.row0 + at * PVE_OBS_W;
+    *prev_dev = f->F.prev + at * PVE_OBS_W;
+    *src_dev = f->F.src + at * 8;
+    return PVE_OK;
+}
+
+int64_t pve_nstep_log_bytes(const pve_nstep *f) {
+    if (!f) return PVE_EINVAL;
+    const long long M = f->T.M, oc = f->out_cap;
+    if (f->F.row0) return M * (oc * (2 * PVE_OBS_W * (long long)sizeof(float) + 8 * (long long)sizeof(int16_t))
+                               + (f->T.B + 1) * (long long)sizeof(int32_t));
+    return M * oc * PVN_OBS * (long long)sizeof(float);
+}
+
+const char *pve_nstep_last_error(const pve_nstep *f) { return f ? f->err : "null folder"; }
+
+int32_t pve_nstep_set_profiling(pve_nstep *f, int32_t on) {
+    if (!f) return PVE_EINVAL;
+#ifdef PVE_HOST_EMULATION
+    (void)on;
+    return PVE_ESTATE;
+#else
+    if (on && !f->profiling) {
+        if (cudaEventCreate(&f->fold_ev[0]) != cudaSuccess) return PVE_ECUDA;
+        if (cudaEventCreate(&f->fold_ev[1]) != cudaSuccess) { cudaEventDestroy(f->fold_ev[0]); return PVE_ECUDA; }
+        f->profiling = 1;
+    } else if (!on && f->profiling) {
+        cudaEventDestroy(f->fold_ev[0]);
+        cudaEventDestroy(f->fold_ev[1]);
+        f->profiling = 0;
+    }
+    return PVE_OK;
+#endif
+}
+
+int32_t pve_nstep_fold_ms(pve_nstep *f, float *ms) {
+    if (!f || !ms) return PVE_EINVAL;
+#ifdef PVE_HOST_EMULATION
+    return PVE_ESTATE;
+#else
+    if (!f->profiling || f->pushes == 0) return PVE_ESTATE;
+    if (cudaEventSynchronize(f->fold_ev[1]) != cudaSuccess || cudaEventElapsedTime(ms, f->fold_ev[0], f->fold_ev[1]) != cudaSuccess)
+        return PVE_ECUDA;
+    return PVE_OK;
+#endif
 }
 
 int32_t pve_nstep_reset(pve_nstep *f, void *stream_) {

@@ -134,21 +134,35 @@ class NStepFolder:
 
     ``seq_max_step`` = ``args.seq_max_step`` (main.py:91); ``buffer_size`` = first argument of ``ReplayBuffer``
     (main.py:212).  ``uid_slots``: history slots per intersection (power of two; default twice the vehicle capacity).
+
+    ``factored``: keep the frame log in the factored form (``pve_nstep_create_factored``: row 0, previous row 0 and 8 row
+    codes per agent, 240 instead of 784 bytes; ``log_bytes`` tells the size) and push from the factored observation.  The
+    scene must export it (``BatchedScene(factored_obs=True)``, with or without ``full_obs``; 12-lane intersections only).
+    The replay memory, counters and bootstrap values are those of a full-frame folder fed the same ticks, bit for bit.
     """
 
-    def __init__(self, scene, target_actor, target_critic, seq_max_step=12, buffer_size=500000, uid_slots=None):
+    factored = False
+
+    def __init__(self, scene, target_actor, target_critic, seq_max_step=12, buffer_size=500000, uid_slots=None,
+                 factored=False):
         self.device = _cuda_device(scene.device)
         self.lib = scene.lib
         self.scene, self.target_actor, self.target_critic = scene, target_actor, target_critic
+        self.factored = bool(factored)
+        if self.factored and getattr(scene.out, "obs_src", None) is None:
+            raise ValueError("NStepFolder(factored=True) pushes the factored observation, and this scene does not export it: "
+                             "create the scene with BatchedScene(factored_obs=True) (12-lane intersections only)")
         if uid_slots is None:
             uid_slots = 1 << int(np.ceil(np.log2(max(16, 2 * scene.veh_cap))))
         self.seq_max_step, self.buffer_size, self.uid_slots = int(seq_max_step), int(buffer_size), int(uid_slots)
         self._h = C.c_void_p()
-        rc = self.lib.pve_nstep_create(scene.B, self.uid_slots, self.seq_max_step, scene.out_cap, self.buffer_size,
-                                       self.device.index or 0, C.byref(self._h))
+        create = self.lib.pve_nstep_create_factored if self.factored else self.lib.pve_nstep_create
+        rc = create(scene.B, self.uid_slots, self.seq_max_step, scene.out_cap, self.buffer_size,
+                    self.device.index or 0, C.byref(self._h))
         if rc != 0:
             raise N.NativeError("pve_nstep_create failed with %d (seq_max_step <= 14, uid_slots a power of two >= 16, "
                                 "buffer_size - 1 >= out_cap = %d)" % (rc, scene.out_cap))
+        self.log_bytes = int(self.lib.pve_nstep_log_bytes(self._h))     # the frame log of the last seq_max_step + 2 pushes
         view = N.PveReplayView()
         self.lib.pve_nstep_replay(self._h, C.byref(view))
         self.capacity = int(view.capacity)                        # buffer_size - 1 (replay_buffer.py:47-53)
@@ -173,7 +187,22 @@ class NStepFolder:
     def push(self, outputs, gamma, distinct_rows=None):
         """main.py:243-266 for the tick that produced ``outputs`` (a ``StepOutputs``).  Asynchronous.
         ``distinct_rows``: None = use the scene's neighbour sources when it exports them; False = always evaluate the
-        target actor on all 7 rows of every observation."""
+        target actor on all 7 rows of every observation.
+
+        A factored folder reads the factored observation of ``outputs`` (any ``StepOutputs`` with ``row0_out``,
+        ``prev_row0`` and ``obs_src``, not only ``scene.out``; ``obs`` is never read) and evaluates the target actor once
+        per distinct row.  Its outputs carry every row the push needs, so the push may come after the scene's next step
+        (give that step other outputs); pushes must still come in tick order."""
+        if self.factored:
+            if any(getattr(outputs, f, None) is None for f in ("row0_out", "prev_row0", "obs_src")):
+                raise ValueError("a factored NStepFolder pushes the factored observation, and these outputs carry none "
+                                 "(BatchedScene(factored_obs=True))")
+            rc = self.lib.pve_nstep_push_factored(self._h, C.byref(outputs.native()), float(gamma), self.target_actor._h,
+                                                  self.target_critic._h, self._stream())
+            if rc != 0:
+                raise N.NativeError("pve_nstep_push_factored failed with %d: %s"
+                                    % (rc, self.lib.pve_nstep_last_error(self._h).decode()))
+            return
         if outputs.obs is None:
             raise ValueError("NStepFolder.push reads the observations, and these outputs carry none (BatchedScene("
                              "full_obs=False)): call bind_outputs() before the step so that it writes them into the frame log")
@@ -195,8 +224,21 @@ class NStepFolder:
         """Zero-copy: make the next ``scene.step`` write its observations straight into the folder's frame log.  Call it
         before every step whose outputs will be pushed (``outputs`` defaults to ``scene.out``; its ``obs`` tensor is
         replaced by a view of the log block the next push expects, so read ``outputs.obs`` before the next call).
-        Without it ``push`` copies the observation block into the log (same results, one more device copy per tick)."""
+        Without it ``push`` copies the observation block into the log (same results, one more device copy per tick).
+        A factored folder replaces ``row0_out``, ``prev_row0`` and ``obs_src`` instead (``pve_nstep_factored_slot``)."""
         outputs = self.scene.out if outputs is None else outputs
+        if self.factored:
+            ptrs = [C.c_void_p() for _ in range(3)]
+            rc = self.lib.pve_nstep_factored_slot(self._h, *[C.byref(p) for p in ptrs])
+            if rc != 0:
+                raise N.NativeError("pve_nstep_factored_slot failed with %d" % rc)
+            oc = self.scene.out_cap
+            shapes = ((oc, OBS_W, torch.float32), (oc, OBS_W, torch.float32), (oc, 8, torch.int16))
+            for name, p, (n, w, dt) in zip(("row0_out", "prev_row0", "obs_src"), ptrs, shapes):
+                setattr(outputs, name, self._wrap(p.value, (n, w), dt))
+                if outputs is self.scene.out:
+                    setattr(self.scene._out_native, name, p.value)     # the struct the scene hands to pve_step
+            return outputs
         ptr = C.c_void_p()
         rc = self.lib.pve_nstep_obs_slot(self._h, C.byref(ptr))
         if rc != 0:
@@ -244,7 +286,7 @@ class NStepFolder:
         class _Mem:
             pass
         m = _Mem()
-        m.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": {torch.float32: "<f4", torch.uint8: "|u1"}[dtype],
+        m.__cuda_array_interface__ = {"shape": tuple(shape), "typestr": {torch.float32: "<f4", torch.uint8: "|u1", torch.int16: "<i2"}[dtype],
                                       "data": (int(ptr), False), "version": 2}
         return torch.as_tensor(m, device=self.device)
 
