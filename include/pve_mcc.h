@@ -191,6 +191,30 @@ const char *pve_last_error(const pve_scene *s);
  * warmup != 0 advances every intersection to its first arrival like TIS:214-220. */
 int32_t pve_reset(pve_scene *s, const int32_t *spawn_tick_dev, int32_t K, int32_t warmup, void *stream);
 
+/* A new episode whose traffic the step kernels generate themselves: a Poisson arrival stream per lane, so that no spawn
+ * table is built, uploaded or kept (an episode of any length costs O(B) device memory: 96 B per intersection, plus one
+ * 32 MB clock table per handle allocated by its first Poisson reset).  For global intersection e = first_env + b, lane i
+ * and arrival record r = 0, 1, ...: one Philox4x32-10 block with key (seed & 0xffffffff, seed >> 32) and counter
+ * (e, i, r, 0) gives w0..w3; u = (((w0 << 21) | (w1 >> 11)) + 1) * 2^-53; the headway is
+ * h_r = max(min_headway, -mean * ln(u)) with mean = 3600 / rate_veh_per_hour and ln evaluated by the library's own
+ * +-x/ series (bit-identical on every build); T_r = T_{r-1} + h_r in float64 (T_{-1} = 0); the spawn tick is the first
+ * n whose accumulated 0.1 s clock (SURVEY.md Q8) is >= T_r, PVE_NEVER past 4 000 000 ticks and from record 65 535 on.
+ * lane_num = 8: the intention draw of record r is w2 & 1 (no pve_set_intention_draws needed).  The Python
+ * arrivals.poisson_arrivals is the numpy mirror of the stream.
+ * Intersections see the same traffic however a batch is sharded: a handle holding intersections [lo, hi) of a larger
+ * batch passes first_env = lo. */
+typedef struct pve_poisson {
+    uint64_t seed;
+    double rate_veh_per_hour;   /* finite, > 0 */
+    double min_headway;         /* seconds; finite, > 0 (an arrival at 0 s would read as table padding) */
+    int64_t first_env;          /* >= 0, first_env + n_envs <= 2^32 */
+} pve_poisson;
+/* Like pve_reset (state zeroed, warmup != 0 jumps to the first arrival and runs the tick that brings it in), with the
+ * arrivals of `p`; nothing is borrowed.  The handle stays in Poisson mode until a pve_reset with a table.  PVE_EINVAL
+ * (see pve_last_error) for a rate or min_headway that is not finite and > 0, a negative first_env, first_env + n_envs
+ * > 2^32, or pve_config.dt != 0.1. */
+int32_t pve_reset_poisson(pve_scene *s, const pve_poisson *p, int32_t warmup, void *stream);
+
 /* lane_num = 8 only, before pve_reset: draws_dev uint8 [B][K][12], draws_dev[b][k][i] in {0, 1} = what the reference's
  * `random.randint(0, 1)` returns for the k-th arrival of lane i (TIS:390: intention = self.intention[i][draw]); K and the
  * layout are those of the spawn table handed to the next pve_reset.  Borrowed, must outlive the rollout. */
@@ -241,6 +265,10 @@ int64_t pve_host_wait(pve_scene *s);
 /* rows the NEXT pve_step will emit (device scan result; synchronises `stream`) */
 int64_t pve_next_agent_total(pve_scene *s, void *stream);
 
+/* Teacher forcing: the state of every intersection from `in`.  hdr.next_spawn is not read: it is recomputed from
+ * hdr.veh_rec, from the spawn table in table mode and, in Poisson mode, by summing the headways of records
+ * 0 .. veh_rec[i] again in record order -- the additions the spawns made, so the pending arrival time and next_spawn are
+ * exact and the rollout continues bit for bit. */
 int32_t pve_set_state(pve_scene *s, const pve_state_view *in, void *stream);
 int32_t pve_get_state(pve_scene *s, const pve_state_view *out, void *stream);
 

@@ -42,6 +42,11 @@ class PveOutputs(C.Structure):
                  "env_collisions", "env_lock", "env_removed", "nbr_src", "packed", "row0_out", "prev_row0", "obs_src")]
 
 
+class PvePoisson(C.Structure):
+    """pve_poisson: the arrival stream of pve_reset_poisson"""
+    _fields_ = [("seed", C.c_uint64), ("rate_veh_per_hour", C.c_double), ("min_headway", C.c_double), ("first_env", C.c_int64)]
+
+
 class PveReplayView(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ("state", "action", "reward", "next_state", "done")] + [("capacity", C.c_int64)]
 
@@ -68,6 +73,7 @@ def load_library(path=None):
     lib.pve_last_error.argtypes = [vp]
     lib.pve_last_error.restype = C.c_char_p
     lib.pve_reset.argtypes = [vp, vp, i32, i32, vp]
+    lib.pve_reset_poisson.argtypes = [vp, C.POINTER(PvePoisson), i32, vp]
     lib.pve_set_intention_draws.argtypes = [vp, vp]
     lib.pve_step.argtypes = [vp, vp, C.POINTER(PveOutputs), vp]
     lib.pve_step_host.argtypes = [vp, vp, C.POINTER(PveOutputs), C.POINTER(PveOutputs), i32, vp]

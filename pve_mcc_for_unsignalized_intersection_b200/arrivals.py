@@ -79,6 +79,72 @@ def synthetic_arrivals(n_envs, rate_veh_per_hour, horizon_s, seed=0, min_headway
         rows = int(rows * 1.3) + 8
 
 
+# ---- the Poisson arrival stream of BatchedScene.reset_poisson (csrc/arrivals.cuh), mirrored in numpy -------------------
+_PHILOX_M0, _PHILOX_M1 = np.uint64(0xD2511F53), np.uint64(0xCD9E8D57)
+_PHILOX_W0, _PHILOX_W1 = np.uint64(0x9E3779B9), np.uint64(0xBB67AE85)
+_U32 = np.uint64(0xFFFFFFFF)
+# 2 / (2k + 1), k = 11 .. 1: the odd series of 2 atanh(s) (the same literals as csrc/arrivals.cuh)
+_LOG_SERIES = (0.08695652173913043, 0.09523809523809523, 0.10526315789473684, 0.11764705882352941, 0.13333333333333333,
+               0.15384615384615385, 0.18181818181818182, 0.2222222222222222, 0.2857142857142857, 0.4, 0.6666666666666666)
+_LN2_HI, _LN2_LO = 6.93147180369123816490e-01, 1.90821492927058770002e-10
+MAX_REC = 65535               # records from here on never spawn (veh_rec is 16 bits)
+
+
+def philox4x32(c0, c1, c2, c3, k0, k1):
+    """Philox4x32-10 on broadcastable arrays of 32-bit words (any integer dtype); returns four uint64 arrays of 32-bit
+    words.  Counter 0, key 0 gives 6627e8d5 e169c58d bc57ac4c 9b00dbd8 (Random123's known-answer vector)."""
+    c = [np.asarray(x).astype(np.uint64) & _U32 for x in (c0, c1, c2, c3)]
+    k0, k1 = np.uint64(int(k0) & 0xFFFFFFFF), np.uint64(int(k1) & 0xFFFFFFFF)
+    s32 = np.uint64(32)
+    for _ in range(10):
+        p0, p1 = _PHILOX_M0 * c[0], _PHILOX_M1 * c[2]
+        c = [(p1 >> s32) ^ c[1] ^ k0, p1 & _U32, (p0 >> s32) ^ c[3] ^ k1, p0 & _U32]
+        k0, k1 = (k0 + _PHILOX_W0) & _U32, (k1 + _PHILOX_W1) & _U32
+    return c
+
+
+def stream_log(u):
+    """ln(u) for float64 u in [2^-53, 1] by the stream's own scheme (exact scaling to m in [sqrt(1/2), sqrt(2)),
+    s = (m - 1) / (m + 1), odd series in s up to s^23, e * ln2 in two parts): + - * / only, so the device, the kernel
+    emulation and numpy agree bit for bit.  Within 1 ulp of a correctly rounded log."""
+    m, e = np.frexp(np.asarray(u, dtype=np.float64))
+    low = m < 0.70710678118654752440
+    m = np.where(low, m + m, m)
+    dk = np.where(low, e - 1, e).astype(np.float64)
+    f = m - 1.0
+    s = f / (2.0 + f)
+    z = s * s
+    R = _LOG_SERIES[0]
+    for c in _LOG_SERIES[1:]:
+        R = c + z * R
+    R = z * R
+    hfsq = 0.5 * f * f
+    return dk * _LN2_HI - ((hfsq - (s * (hfsq + R) + dk * _LN2_LO)) - f)
+
+
+def poisson_arrivals(n_envs, rate_veh_per_hour, rows, seed, min_headway=1.0, first_env=0, lanes=NLANE):
+    """The first ``rows`` records of every lane of the stream that ``BatchedScene.reset_poisson`` generates on the device,
+    for global intersections ``first_env .. first_env + n_envs - 1``.  Returns ``(seconds, draws)``: float64 arrival
+    times ``[n_envs, rows, lanes]`` and the lane_num = 8 intention draws (uint8 in {0, 1}) of the same records.
+
+    Per record ``r`` of lane ``i`` of intersection ``e``: Philox4x32-10 with counter ``(e, i, r, 0)`` and key
+    ``(seed & 0xffffffff, seed >> 32)`` gives ``w0..w3``; ``u = (((w0 << 21) | (w1 >> 11)) + 1) * 2**-53``; the headway is
+    ``max(min_headway, -mean * stream_log(u))`` with ``mean = 3600 / rate``; times are the running sums in record order;
+    the draw is ``w2 & 1``.  ``to_spawn_ticks(seconds)`` gives the spawn ticks the device uses (which also never spawns
+    a record past ``MAX_TICK`` or from record ``MAX_REC`` on).  The distribution is that of ``synthetic_arrivals``, the
+    random stream is not."""
+    seed = int(seed)
+    e = (int(first_env) + np.arange(n_envs, dtype=np.uint64))[:, None, None]
+    r = np.arange(rows, dtype=np.uint64)[None, :, None]
+    i = np.arange(lanes, dtype=np.uint64)[None, None, :]
+    w0, w1, w2, _ = philox4x32(e, i, r, np.uint64(0), seed & 0xFFFFFFFF, seed >> 32)
+    x = (w0 << np.uint64(21)) | (w1 >> np.uint64(11))
+    u = (x + np.uint64(1)).astype(np.float64) * 2.0 ** -53
+    mean = 3600.0 / float(rate_veh_per_hour)
+    head = np.maximum(-mean * stream_log(u), float(min_headway))
+    return np.add.accumulate(head, axis=1), (w2 & np.uint64(1)).astype(np.uint8)
+
+
 def stress_arrivals(n_envs, horizon_s, headway=1.0):
     """Worst-case occupancy: every lane receives a vehicle every ``headway`` seconds."""
     rows = int(horizon_s / headway) + 4

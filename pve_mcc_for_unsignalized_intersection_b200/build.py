@@ -8,7 +8,8 @@ CSRC = os.path.join(PKG_DIR, "csrc")
 INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include")
 LIB = os.path.join(CSRC, "libpve_mcc.so")
 SOURCES = [os.path.join(CSRC, "pve_mcc.cu"), os.path.join(CSRC, "scene_step.cuh"), os.path.join(CSRC, "scene_step4.cuh"), os.path.join(CSRC, "actor.cuh"),
-           os.path.join(CSRC, "actor_mma.cuh"), os.path.join(CSRC, "nstep.cuh"), os.path.join(CSRC, "critic_mma.cuh"), os.path.join(CSRC, "mlp_tc5.cuh"), os.path.join(INCLUDE, "pve_mcc.h")]
+           os.path.join(CSRC, "actor_mma.cuh"), os.path.join(CSRC, "nstep.cuh"), os.path.join(CSRC, "critic_mma.cuh"), os.path.join(CSRC, "mlp_tc5.cuh"), os.path.join(CSRC, "arrivals.cuh"),
+           os.path.join(INCLUDE, "pve_mcc.h")]
 
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               # float64 state must follow the reference's two-rounding a*b+c (no FMA contraction)

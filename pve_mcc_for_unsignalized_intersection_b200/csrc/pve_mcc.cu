@@ -84,6 +84,12 @@ struct pve_scene {
 #endif
     int order_age;               /* ticks since the order was refreshed (-1: never) */
     const int32_t *spawn_tick;   /* borrowed */
+    /* Poisson mode (pve_reset_poisson): the step kernels generate the arrivals (arrivals.cuh) instead of reading
+     * spawn_tick; pend_dev / clock_dev are allocated by the first Poisson reset and kept for the handle's lifetime */
+    int poisson;
+    PvePoisson poi;
+    double *pend_dev;            /* [B][12] */
+    double *clock_dev;           /* [PVE_MAX_TICK + 1] */
     float *actions_dev;          /* staging for pve_step_host */
     double *counters_dev;
     int32_t *pinned_i32;         /* host-visible scratch */
@@ -158,9 +164,9 @@ struct PveResident {
         return nt == 96 ? BY_SMEM : nt == 512 ? (BY_SMEM < 2 ? BY_SMEM : 2) : (CTAS128 * 128 / nt > 0 ? CTAS128 * 128 / nt : 1);
     }
 };
-template <int NT, int VC, int AC, bool SRC>
+template <int NT, int VC, int AC, bool SRC, bool POI>
 __global__ void __launch_bounds__(NT, PveResident<VC, AC>::blocks(NT))
-pve_step_kernel(const PveParams P, const PveState S, const pve_outputs O, const int32_t *spawn_tick,
+pve_step_kernel(const PveParams P, const PveState S, const pve_outputs O, const typename PveArrivalsT<POI>::type spawn_tick,
                 const float *actions, const int phase) {
     extern __shared__ __align__(16) unsigned char pve_smem[];
     /* CTAs are dispatched in index order; starting the busiest intersections first shortens the tail
@@ -168,22 +174,22 @@ pve_step_kernel(const PveParams P, const PveState S, const pve_outputs O, const 
     const int b = S.order ? S.order[blockIdx.x] : (int)blockIdx.x;
     /* dual mode: intersections of the big kernel are skipped (pve_step_block tests klass[b] after it has issued its
      * first loads, so the test costs no extra memory round trip) */
-    pve_step_block<NT, VC, AC, SRC>(P, S, O, spawn_tick, actions, phase, b, pve_smem, S.klass);
+    pve_step_block<NT, VC, AC, SRC, POI>(P, S, O, spawn_tick, actions, phase, b, pve_smem, S.klass);
     /* dual mode launches this grid as the programmatic dependent of the big kernel (same stream, started while the
      * big kernel runs): it may not complete before that one has (no-op for an ordinary launch) */
     asm volatile("griddepcontrol.wait;" ::: "memory");
 }
 
 /* dual mode: the intersections that do not fit the small class, a few per tick */
-template <int NT, int VC, int AC, bool SRC>
+template <int NT, int VC, int AC, bool SRC, bool POI>
 __global__ void __launch_bounds__(NT, PveResident<VC, AC>::blocks(NT))
-pve_step_big_kernel(const PveParams P, const PveState S, const pve_outputs O, const int32_t *spawn_tick,
+pve_step_big_kernel(const PveParams P, const PveState S, const pve_outputs O, const typename PveArrivalsT<POI>::type spawn_tick,
                     const float *actions, const int phase) {
     extern __shared__ __align__(16) unsigned char pve_smem[];
     asm volatile("griddepcontrol.launch_dependents;");      /* the small kernel shares nothing with this one: start it now */
     const int n = *S.big_cnt;
     for (int i = (int)blockIdx.x; i < n; i += (int)gridDim.x) {
-        pve_step_block<NT, VC, AC, SRC>(P, S, O, spawn_tick, actions, phase, S.big_list[i], pve_smem, nullptr);
+        pve_step_block<NT, VC, AC, SRC, POI>(P, S, O, spawn_tick, actions, phase, S.big_list[i], pve_smem, nullptr);
         __syncthreads();                                   /* shared memory is reused by the next one */
     }
 }
@@ -211,15 +217,15 @@ __global__ void pve_classify_kernel(PveState S, int B) {
 
 /* ---- lane_num = 4 / 8 (scene_step4.cuh): one warp per intersection, PVE4_WARPS intersections per CTA -------------- */
 #define PVE4_WARPS 4
-template <int NLN, int LC>
+template <int NLN, int LC, bool POI>
 __global__ void __launch_bounds__(32 * PVE4_WARPS)
-pve4_step_kernel(const Pve4Params P, const PveState S, const pve_outputs O, const int32_t *spawn_tick, const uint8_t *draws,
-                 const float *actions, const int64_t *off4) {
+pve4_step_kernel(const Pve4Params P, const PveState S, const pve_outputs O, const typename PveArrivalsT<POI>::type spawn_tick,
+                 const uint8_t *draws, const float *actions, const int64_t *off4) {
     extern __shared__ __align__(16) unsigned char pve_smem[];
     const int b = (int)blockIdx.x * PVE4_WARPS + (int)(threadIdx.x >> 5);
     if (b >= P.B) return;
     Pve4SmemT<LC> &M = ((Pve4SmemT<LC> *)pve_smem)[threadIdx.x >> 5];
-    pve4_step_block<NLN>(P, S, O, spawn_tick, draws, actions, b, M, off4[b]);
+    pve4_step_block<NLN, POI>(P, S, O, spawn_tick, draws, actions, b, M, off4[b]);
 }
 
 /* exclusive prefix of the agent counts -> first output row of every intersection (one CTA; B is small on this path) */
@@ -265,14 +271,17 @@ __global__ void pve_gsum_kernel(const int32_t *__restrict__ n_ctrl, int32_t *__r
     gs_now[g] = s; gs_a[g] = 0; gs_b[g] = 0;
 }
 
-__global__ void pve_reset_kernel(PveState S, const int32_t *__restrict__ spawn_tick, int B, int K, int warmup) {
+template <bool POI>
+__global__ void pve_reset_kernel(PveState S, const typename PveArrivalsT<POI>::type spawn_tick, int B, int K, int warmup) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
     pve_env_header h;
     memset(&h, 0, sizeof h);
     int first = PVE_NEVER;
     for (int i = 0; i < PVE_NLANE; ++i) {
-        const int t = (K > 0) ? spawn_tick[(size_t)b * K * PVE_NLANE + i] : PVE_NEVER;
+        int t;
+        if constexpr (POI) t = pve_reset_lane(spawn_tick, b, i);
+        else t = (K > 0) ? spawn_tick[(size_t)b * K * PVE_NLANE + i] : PVE_NEVER;
         h.next_spawn[i] = t;
         h.head_lane[i] = -1;
         first = min(first, t);
@@ -287,7 +296,8 @@ __global__ void pve_reset_kernel(PveState S, const int32_t *__restrict__ spawn_t
 }
 
 /* after pve_set_state: recompute the derived header fields */
-__global__ void pve_recount_kernel(PveState S, const int32_t *__restrict__ spawn_tick, int B, int VC, int K) {
+template <bool POI>
+__global__ void pve_recount_kernel(PveState S, const typename PveArrivalsT<POI>::type spawn_tick, int B, int VC, int K) {
     const int b = blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
     pve_env_header *h = S.hdr + b;
@@ -299,7 +309,8 @@ __global__ void pve_recount_kernel(PveState S, const int32_t *__restrict__ spawn
     h->n_ctrl = nc;
     for (int i = 0; i < PVE_NLANE; ++i) {
         const int rec = h->veh_rec[i];
-        h->next_spawn[i] = (spawn_tick && rec < K) ? spawn_tick[((size_t)b * K + rec) * PVE_NLANE + i] : PVE_NEVER;
+        if constexpr (POI) h->next_spawn[i] = pve_recount_lane(spawn_tick, b, i, rec);
+        else h->next_spawn[i] = (spawn_tick && rec < K) ? spawn_tick[((size_t)b * K + rec) * PVE_NLANE + i] : PVE_NEVER;
     }
     S.n_ctrl[b] = nc;
     S.n_veh[b] = nv;
@@ -361,13 +372,16 @@ static void emul_gsum(const int32_t *n_ctrl, int32_t *gs_now, int32_t *gs_a, int
         gs_now[g] = s; gs_a[g] = 0; gs_b[g] = 0;
     }
 }
-static void emul_reset(PveState S, const int32_t *spawn_tick, int B, int K, int warmup) {
+template <bool POI>
+static void emul_reset(PveState S, const typename PveArrivalsT<POI>::type spawn_tick, int B, int K, int warmup) {
     for (int b = 0; b < B; ++b) {
         pve_env_header h;
         memset(&h, 0, sizeof h);
         int first = PVE_NEVER;
         for (int i = 0; i < PVE_NLANE; ++i) {
-            const int t = (K > 0) ? spawn_tick[(size_t)b * K * PVE_NLANE + i] : PVE_NEVER;
+            int t;
+            if constexpr (POI) t = pve_reset_lane(spawn_tick, b, i);
+            else t = (K > 0) ? spawn_tick[(size_t)b * K * PVE_NLANE + i] : PVE_NEVER;
             h.next_spawn[i] = t; h.head_lane[i] = -1;
             first = t < first ? t : first;
         }
@@ -376,7 +390,8 @@ static void emul_reset(PveState S, const int32_t *spawn_tick, int B, int K, int 
         for (int q = 0; q < PVE_NSTAT; ++q) S.stats[(size_t)b * PVE_NSTAT + q] = 0.0;
     }
 }
-static void emul_recount(PveState S, const int32_t *spawn_tick, int B, int VC, int K) {
+template <bool POI>
+static void emul_recount(PveState S, const typename PveArrivalsT<POI>::type spawn_tick, int B, int VC, int K) {
     for (int b = 0; b < B; ++b) {
         pve_env_header *h = S.hdr + b;
         int nv = 0, nc = 0;
@@ -386,7 +401,8 @@ static void emul_recount(PveState S, const int32_t *spawn_tick, int B, int VC, i
         h->n_veh = nv; h->n_ctrl = nc;
         for (int i = 0; i < PVE_NLANE; ++i) {
             const int rec = h->veh_rec[i];
-            h->next_spawn[i] = (spawn_tick && rec < K) ? spawn_tick[((size_t)b * K + rec) * PVE_NLANE + i] : PVE_NEVER;
+            if constexpr (POI) h->next_spawn[i] = pve_recount_lane(spawn_tick, b, i, rec);
+            else h->next_spawn[i] = (spawn_tick && rec < K) ? spawn_tick[((size_t)b * K + rec) * PVE_NLANE + i] : PVE_NEVER;
         }
         S.n_ctrl[b] = nc; S.n_veh[b] = nv;
     }
@@ -457,19 +473,26 @@ static bool pick_class(int veh_cap, int agent_cap, int *VC, int *AC, size_t *sme
     return false;
 }
 
+/* the arrivals argument of the step kernels: the spawn table, or the Poisson generator */
+template <bool POI>
+static typename PveArrivalsT<POI>::type arrivals_arg(const pve_scene *s) {
+    if constexpr (POI) return s->poi;
+    else return s->spawn_tick;
+}
+
 #ifndef PVE_HOST_EMULATION
-template <int NT, int VC, int AC, bool SRC>
+template <int NT, int VC, int AC, bool SRC, bool POI>
 static cudaError_t launch_variant(pve_scene *s, const float *actions, const pve_outputs &O, pve_stream_t stream) {
     static bool attr_set[16] = {false};
     int dev = s->device & 15;
     if (!attr_set[dev]) {
-        cudaError_t e = cudaFuncSetAttribute(pve_step_kernel<NT, VC, AC, SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        cudaError_t e = cudaFuncSetAttribute(pve_step_kernel<NT, VC, AC, SRC, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                              (int)(PveLayout<VC, AC>::BYTES + s->smem_pad));
         if (e != cudaSuccess) return e;
         attr_set[dev] = true;
     }
-    pve_step_kernel<NT, VC, AC, SRC><<<s->cfg.n_envs, NT, PveLayout<VC, AC>::BYTES + s->smem_pad, stream>>>(
-        s->prm, s->st, O, s->spawn_tick, actions, s->phase);
+    pve_step_kernel<NT, VC, AC, SRC, POI><<<s->cfg.n_envs, NT, PveLayout<VC, AC>::BYTES + s->smem_pad, stream>>>(
+        s->prm, s->st, O, arrivals_arg<POI>(s), actions, s->phase);
     return cudaGetLastError();
 }
 /* dual mode: the small kernel (96 threads, class PVE_SMALL_VC / PVE_SMALL_AC: more intersections resident per SM) on
@@ -481,17 +504,17 @@ static cudaError_t launch_variant(pve_scene *s, const float *actions, const pve_
 #ifndef PVE_SMALL_NT
 #define PVE_SMALL_NT 96
 #endif
-template <int VC, int AC, bool SRC>
+template <int VC, int AC, bool SRC, bool POI>
 static cudaError_t launch_dual(pve_scene *s, const float *actions, const pve_outputs &O, pve_stream_t stream) {
     static bool attr_set[16] = {false};
     int dev = s->device & 15;
     const size_t smem_small = PveLayout<PVE_SMALL_VC, PVE_SMALL_AC>::BYTES, smem_big = PveLayout<VC, AC>::BYTES;
     cudaError_t e;
     if (!attr_set[dev]) {
-        e = cudaFuncSetAttribute(pve_step_kernel<PVE_SMALL_NT, PVE_SMALL_VC, PVE_SMALL_AC, SRC>,
+        e = cudaFuncSetAttribute(pve_step_kernel<PVE_SMALL_NT, PVE_SMALL_VC, PVE_SMALL_AC, SRC, POI>,
                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem_small + s->smem_pad));
         if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(pve_step_big_kernel<128, VC, AC, SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_big);
+        e = cudaFuncSetAttribute(pve_step_big_kernel<128, VC, AC, SRC, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_big);
         if (e != cudaSuccess) return e;
         attr_set[dev] = true;
     }
@@ -502,7 +525,7 @@ static cudaError_t launch_dual(pve_scene *s, const float *actions, const pve_out
          * starts when every CTA of the big kernel has executed griddepcontrol.launch_dependents and waits for the big
          * kernel's completion only at its own end (griddepcontrol.wait), so the stream's next kernel is ordered after
          * both. */
-        pve_step_big_kernel<128, VC, AC, SRC><<<big_grid, 128, smem_big, stream>>>(s->prm, s->st, O, s->spawn_tick, actions, s->phase);
+        pve_step_big_kernel<128, VC, AC, SRC, POI><<<big_grid, 128, smem_big, stream>>>(s->prm, s->st, O, arrivals_arg<POI>(s), actions, s->phase);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
         cudaLaunchConfig_t cfg;
         memset(&cfg, 0, sizeof cfg);
@@ -512,27 +535,66 @@ static cudaError_t launch_dual(pve_scene *s, const float *actions, const pve_out
         at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
         at[0].val.programmaticStreamSerializationAllowed = 1;
         cfg.attrs = at; cfg.numAttrs = 1;
-        const int32_t *sp_arg = s->spawn_tick;
-        return cudaLaunchKernelEx(&cfg, pve_step_kernel<PVE_SMALL_NT, PVE_SMALL_VC, PVE_SMALL_AC, SRC>, s->prm, s->st, O, sp_arg, actions, (int)s->phase);
+        const typename PveArrivalsT<POI>::type sp_arg = arrivals_arg<POI>(s);
+        return cudaLaunchKernelEx(&cfg, pve_step_kernel<PVE_SMALL_NT, PVE_SMALL_VC, PVE_SMALL_AC, SRC, POI>, s->prm, s->st, O, sp_arg, actions, (int)s->phase);
     }
     if ((e = cudaEventRecord(s->ev_fork, stream)) != cudaSuccess) return e;
     if ((e = cudaStreamWaitEvent(s->side, s->ev_fork, 0)) != cudaSuccess) return e;
-    pve_step_big_kernel<128, VC, AC, SRC><<<big_grid, 128, smem_big, s->side>>>(s->prm, s->st, O, s->spawn_tick, actions, s->phase);
+    pve_step_big_kernel<128, VC, AC, SRC, POI><<<big_grid, 128, smem_big, s->side>>>(s->prm, s->st, O, arrivals_arg<POI>(s), actions, s->phase);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     if ((e = cudaEventRecord(s->ev_join, s->side)) != cudaSuccess) return e;
-    pve_step_kernel<PVE_SMALL_NT, PVE_SMALL_VC, PVE_SMALL_AC, SRC><<<s->cfg.n_envs, PVE_SMALL_NT, smem_small + s->smem_pad, stream>>>(
-        s->prm, s->st, O, s->spawn_tick, actions, s->phase);
+    pve_step_kernel<PVE_SMALL_NT, PVE_SMALL_VC, PVE_SMALL_AC, SRC, POI><<<s->cfg.n_envs, PVE_SMALL_NT, smem_small + s->smem_pad, stream>>>(
+        s->prm, s->st, O, arrivals_arg<POI>(s), actions, s->phase);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
     return cudaStreamWaitEvent(stream, s->ev_join, 0);
 }
 
 /* the instantiation that also writes pve_outputs.nbr_src and the factored observation only when the caller asks for
- * one of them */
+ * one of them; the Poisson instantiation only in Poisson mode */
 static bool wants_src(const pve_outputs &O) { return O.nbr_src != nullptr || O.obs_src != nullptr; }
 template <int NT, int VC, int AC>
 static cudaError_t launch_one(pve_scene *s, const float *actions, const pve_outputs &O, pve_stream_t stream) {
-    return wants_src(O) ? launch_variant<NT, VC, AC, true>(s, actions, O, stream)
-                     : launch_variant<NT, VC, AC, false>(s, actions, O, stream);
+    if (s->poisson)
+        return wants_src(O) ? launch_variant<NT, VC, AC, true, true>(s, actions, O, stream)
+                            : launch_variant<NT, VC, AC, false, true>(s, actions, O, stream);
+    return wants_src(O) ? launch_variant<NT, VC, AC, true, false>(s, actions, O, stream)
+                     : launch_variant<NT, VC, AC, false, false>(s, actions, O, stream);
+}
+template <int VC, int AC>
+static cudaError_t launch_dual_any(pve_scene *s, const float *actions, const pve_outputs &O, pve_stream_t stream) {
+    if (s->poisson)
+        return wants_src(O) ? launch_dual<VC, AC, true, true>(s, actions, O, stream) : launch_dual<VC, AC, false, true>(s, actions, O, stream);
+    return wants_src(O) ? launch_dual<VC, AC, true, false>(s, actions, O, stream) : launch_dual<VC, AC, false, false>(s, actions, O, stream);
+}
+#endif
+
+#ifndef PVE_HOST_EMULATION
+/* lane_num = 4 / 8: the step kernel of one arrival source */
+template <bool POI>
+static cudaError_t launch_kernel4(pve_scene *s, const float *actions, const pve_outputs &O, pve_stream_t stream) {
+    static bool attr_set[16] = {false};
+    /* capacity class 64 (lists and vehicle slots of <= 64 entries): half the shared memory, twice the resident warps */
+    const bool small = s->prm.VC <= 64;
+    const size_t smem = (small ? sizeof(Pve4SmemT<64>) : sizeof(Pve4SmemT<128>)) * PVE4_WARPS;
+    cudaError_t e;
+    if (!attr_set[s->device & 15]) {
+        if ((e = cudaFuncSetAttribute(pve4_step_kernel<4, 128, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<128>) * PVE4_WARPS))) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(pve4_step_kernel<8, 128, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<128>) * PVE4_WARPS))) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(pve4_step_kernel<4, 64, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<64>) * PVE4_WARPS))) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(pve4_step_kernel<8, 64, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<64>) * PVE4_WARPS))) != cudaSuccess) return e;
+        attr_set[s->device & 15] = true;
+    }
+    const int grid = (s->cfg.n_envs + PVE4_WARPS - 1) / PVE4_WARPS;
+    const typename PveArrivalsT<POI>::type arr = arrivals_arg<POI>(s);
+    if (s->lane_num == 4 && small)
+        pve4_step_kernel<4, 64, POI><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, arr, nullptr, actions, s->off4);
+    else if (s->lane_num == 4)
+        pve4_step_kernel<4, 128, POI><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, arr, nullptr, actions, s->off4);
+    else if (small)
+        pve4_step_kernel<8, 64, POI><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, arr, s->draws, actions, s->off4);
+    else
+        pve4_step_kernel<8, 128, POI><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, arr, s->draws, actions, s->off4);
+    return cudaGetLastError();
 }
 #endif
 
@@ -540,30 +602,10 @@ static cudaError_t launch_one(pve_scene *s, const float *actions, const pve_outp
 static int32_t launch_step4(pve_scene *s, const float *actions, const pve_outputs &O, pve_stream_t stream) {
     const int B = s->cfg.n_envs;
 #ifndef PVE_HOST_EMULATION
-    static bool attr_set[16] = {false};
-    /* capacity class 64 (lists and vehicle slots of <= 64 entries): half the shared memory, twice the resident warps */
-    const bool small = s->prm.VC <= 64;
-    const size_t smem = (small ? sizeof(Pve4SmemT<64>) : sizeof(Pve4SmemT<128>)) * PVE4_WARPS;
-    if (!attr_set[s->device & 15]) {
-        RT_CHECK(s, cudaFuncSetAttribute(pve4_step_kernel<4, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<128>) * PVE4_WARPS)));
-        RT_CHECK(s, cudaFuncSetAttribute(pve4_step_kernel<8, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<128>) * PVE4_WARPS)));
-        RT_CHECK(s, cudaFuncSetAttribute(pve4_step_kernel<4, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<64>) * PVE4_WARPS)));
-        RT_CHECK(s, cudaFuncSetAttribute(pve4_step_kernel<8, 64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<64>) * PVE4_WARPS)));
-        attr_set[s->device & 15] = true;
-    }
     if (s->profiling) RT_CHECK(s, cudaEventRecord(s->ev[0], stream));
     pve4_offsets_kernel<<<1, 1024, 0, stream>>>(s->st.n_ctrl, s->off4, B);
     RT_CHECK(s, cudaGetLastError());
-    const int grid = (B + PVE4_WARPS - 1) / PVE4_WARPS;
-    if (s->lane_num == 4 && small)
-        pve4_step_kernel<4, 64><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, s->spawn_tick, nullptr, actions, s->off4);
-    else if (s->lane_num == 4)
-        pve4_step_kernel<4, 128><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, s->spawn_tick, nullptr, actions, s->off4);
-    else if (small)
-        pve4_step_kernel<8, 64><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, s->spawn_tick, s->draws, actions, s->off4);
-    else
-        pve4_step_kernel<8, 128><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, s->spawn_tick, s->draws, actions, s->off4);
-    RT_CHECK(s, cudaGetLastError());
+    RT_CHECK(s, (s->poisson ? launch_kernel4<true>(s, actions, O, stream) : launch_kernel4<false>(s, actions, O, stream)));
     if (s->profiling) RT_CHECK(s, cudaEventRecord(s->ev[1], stream));
     const int G = s->n_groups;
     pve_gsum_kernel<<<(G + 127) / 128, 128, 0, stream>>>(s->st.n_ctrl, s->gsum, s->gsum + G, s->gsum + 2 * (size_t)G, B, G);
@@ -577,8 +619,10 @@ static int32_t launch_step4(pve_scene *s, const float *actions, const pve_output
     if (!M) return PVE_ENOMEM;
     for (int b = 0; b < B; ++b) {
         memset(M, 0xA5, sizeof *M);           /* poison: catches reads of unwritten shared memory */
-        if (s->lane_num == 4) pve4_step_block<4>(s->prm4, s->st, O, s->spawn_tick, nullptr, actions, b, *M, s->off4[b]);
-        else pve4_step_block<8>(s->prm4, s->st, O, s->spawn_tick, s->draws, actions, b, *M, s->off4[b]);
+        if (s->poisson && s->lane_num == 4) pve4_step_block<4, true>(s->prm4, s->st, O, s->poi, nullptr, actions, b, *M, s->off4[b]);
+        else if (s->poisson) pve4_step_block<8, true>(s->prm4, s->st, O, s->poi, nullptr, actions, b, *M, s->off4[b]);
+        else if (s->lane_num == 4) pve4_step_block<4, false>(s->prm4, s->st, O, s->spawn_tick, nullptr, actions, b, *M, s->off4[b]);
+        else pve4_step_block<8, false>(s->prm4, s->st, O, s->spawn_tick, s->draws, actions, b, *M, s->off4[b]);
     }
     delete M;
     emul_gsum(s->st.n_ctrl, s->gsum, s->gsum + s->n_groups, s->gsum + 2 * (size_t)s->n_groups, B, s->n_groups);
@@ -624,9 +668,9 @@ static int32_t launch_step(pve_scene *s, const float *actions, const pve_outputs
     bool done = false;
     if (s->dual) {
         done = true;
-        if (VCc == 192) RT_CHECK(s, (wants_src(O) ? launch_dual<192, 128, true>(s, actions, O, stream) : launch_dual<192, 128, false>(s, actions, O, stream)));
-        else if (ACc == 96) RT_CHECK(s, (wants_src(O) ? launch_dual<128, 96, true>(s, actions, O, stream) : launch_dual<128, 96, false>(s, actions, O, stream)));
-        else RT_CHECK(s, (wants_src(O) ? launch_dual<128, 80, true>(s, actions, O, stream) : launch_dual<128, 80, false>(s, actions, O, stream)));
+        if (VCc == 192) RT_CHECK(s, (launch_dual_any<192, 128>(s, actions, O, stream)));
+        else if (ACc == 96) RT_CHECK(s, (launch_dual_any<128, 96>(s, actions, O, stream)));
+        else RT_CHECK(s, (launch_dual_any<128, 80>(s, actions, O, stream)));
     }
 #define X(vc, ac)                                                                              \
     if (!done && VCc == vc && ACc == ac) {                                                     \
@@ -652,7 +696,8 @@ static int32_t launch_step(pve_scene *s, const float *actions, const pve_outputs
         done = true;                                                                           \
         for (int b = 0; b < B; ++b) {                                                          \
             memset(smem, 0xA5, s->smem_bytes); /* poison: catches reads of unwritten shared memory */ \
-            pve_step_block<64, vc, ac, true>(s->prm, s->st, O, s->spawn_tick, actions, s->phase, b, smem, nullptr); \
+            if (s->poisson) pve_step_block<64, vc, ac, true, true>(s->prm, s->st, O, s->poi, actions, s->phase, b, smem, nullptr); \
+            else pve_step_block<64, vc, ac, true, false>(s->prm, s->st, O, s->spawn_tick, actions, s->phase, b, smem, nullptr); \
         }                                                                                      \
     }
     PVE_CLASSES(X)
@@ -726,6 +771,7 @@ void pve_destroy(pve_scene *s) {
     rt_host_free(s->pinned_i32); rt_host_free(s->pinned_gs);
     rt_free(s->klass_buf[0]); rt_free(s->klass_buf[1]); rt_free(s->big_list_buf[0]); rt_free(s->big_list_buf[1]);
     rt_free(s->big_cnt3);
+    rt_free(s->clock_dev); rt_free(s->pend_dev);
 #ifndef PVE_HOST_EMULATION
     for (int i = 0; i < 3; ++i) if (s->ev[i]) cudaEventDestroy(s->ev[i]);
     if (s->side) cudaStreamDestroy(s->side);
@@ -915,19 +961,11 @@ int32_t pve_set_intention_draws(pve_scene *s, const uint8_t *draws_dev) {
     return PVE_OK;
 }
 
-int32_t pve_reset(pve_scene *s, const int32_t *spawn_tick_dev, int32_t K, int32_t warmup, void *stream_) {
-    if (!s) return PVE_EINVAL;
-    if (s->lane_num == 8 && spawn_tick_dev && K > 0 && !s->draws) {
-        snprintf(s->err, sizeof s->err, "lane_num = 8: call pve_set_intention_draws before pve_reset (TIS:390 draws every new "
-                                        "vehicle's intention at random; the draws are an input here)");
-        return PVE_EINVAL;
-    }
-    pve_stream_t stream = (pve_stream_t)stream_;
+/* the state of a new episode from the handle's arrival source (pve_reset / pve_reset_poisson); warm_step: run the tick
+ * that brings the first vehicle(s) in */
+static int32_t reset_state(pve_scene *s, int32_t warmup, bool warm_step, pve_stream_t stream) {
     const int B = s->cfg.n_envs;
     const size_t nv = (size_t)B * s->cfg.veh_cap;
-    s->spawn_tick = spawn_tick_dev;
-    s->prm.K = spawn_tick_dev ? K : 0;
-    s->prm4.K = s->prm.K;
     s->phase = 0;
     s->rot = 0;
     s->order_age = -1;
@@ -941,19 +979,86 @@ int32_t pve_reset(pve_scene *s, const int32_t *spawn_tick_dev, int32_t K, int32_
     RT_CHECK(s, rt_memset(s->st.row0[0], 0, sizeof(float) * nv * PVE_OBS_W, stream));
     RT_CHECK(s, rt_memset(s->st.row0[1], 0, sizeof(float) * nv * PVE_OBS_W, stream));
 #ifndef PVE_HOST_EMULATION
-    pve_reset_kernel<<<(B + 127) / 128, 128, 0, stream>>>(s->st, s->spawn_tick, B, s->prm.K, warmup);
+    if (s->poisson) pve_reset_kernel<true><<<(B + 127) / 128, 128, 0, stream>>>(s->st, s->poi, B, 0, warmup);
+    else pve_reset_kernel<false><<<(B + 127) / 128, 128, 0, stream>>>(s->st, s->spawn_tick, B, s->prm.K, warmup);
     RT_CHECK(s, cudaGetLastError());
 #else
-    emul_reset(s->st, s->spawn_tick, B, s->prm.K, warmup);
+    if (s->poisson) emul_reset<true>(s->st, s->poi, B, 0, warmup);
+    else emul_reset<false>(s->st, s->spawn_tick, B, s->prm.K, warmup);
 #endif
     int32_t rc = launch_gsum(s, stream);
     if (rc != PVE_OK) return rc;
-    if (warmup && spawn_tick_dev && K > 0) {
+    if (warm_step) {
         /* the tick that brings the first vehicle(s) in: nothing to step, nothing to emit */
         if (!s->actions_dev) RT_CHECK(s, rt_alloc((void **)&s->actions_dev, sizeof(float) * nv));
         rc = launch_step(s, s->actions_dev, null_outputs(), stream);
     }
     return rc;
+}
+
+int32_t pve_reset(pve_scene *s, const int32_t *spawn_tick_dev, int32_t K, int32_t warmup, void *stream_) {
+    if (!s) return PVE_EINVAL;
+    if (s->lane_num == 8 && spawn_tick_dev && K > 0 && !s->draws) {
+        snprintf(s->err, sizeof s->err, "lane_num = 8: call pve_set_intention_draws before pve_reset (TIS:390 draws every new "
+                                        "vehicle's intention at random; the draws are an input here)");
+        return PVE_EINVAL;
+    }
+    s->poisson = 0;
+    s->spawn_tick = spawn_tick_dev;
+    s->prm.K = spawn_tick_dev ? K : 0;
+    s->prm4.K = s->prm.K;
+    return reset_state(s, warmup, warmup && spawn_tick_dev && K > 0, (pve_stream_t)stream_);
+}
+
+int32_t pve_reset_poisson(pve_scene *s, const pve_poisson *p, int32_t warmup, void *stream_) {
+    if (!s) return PVE_EINVAL;
+    if (!p) { snprintf(s->err, sizeof s->err, "pve_reset_poisson: null parameters"); return PVE_EINVAL; }
+    const int B = s->cfg.n_envs;
+    const char *bad = nullptr;
+    if (!(isfinite(p->rate_veh_per_hour) && p->rate_veh_per_hour > 0)) bad = "rate_veh_per_hour must be finite and > 0";
+    else if (!(isfinite(p->min_headway) && p->min_headway > 0))
+        bad = "min_headway must be finite and > 0 (an arrival at 0 s would read as table padding)";
+    else if (p->first_env < 0) bad = "first_env must be >= 0";
+    else if (p->first_env + (int64_t)B > ((int64_t)1 << 32)) bad = "first_env + n_envs must be <= 2^32 (the counter word of e)";
+    else if (s->cfg.dt != 0.1) bad = "Poisson arrivals use the reference's 0.1 s clock (pve_config.dt must be 0.1)";
+    if (bad) {
+        snprintf(s->err, sizeof s->err, "pve_reset_poisson: %s", bad);
+        return PVE_EINVAL;
+    }
+    pve_stream_t stream = (pve_stream_t)stream_;
+    if (!s->clock_dev) {       /* the reference's clock, the same sequential additions as arrivals.reference_clock */
+        const size_t n = (size_t)PVE_MAX_TICK + 1;
+        double *clock = (double *)malloc(sizeof(double) * n);
+        if (!clock) return PVE_ENOMEM;
+        clock[0] = 0.0;
+        for (size_t k = 1; k < n; ++k) clock[k] = clock[k - 1] + s->cfg.dt;
+        s->poi.clock_last = clock[n - 1];
+        int32_t rc = PVE_OK;
+        if (rt_alloc((void **)&s->clock_dev, sizeof(double) * n) != 0 ||
+            rt_alloc((void **)&s->pend_dev, sizeof(double) * PVE_NLANE * (size_t)B) != 0 ||
+            rt_copy(s->clock_dev, clock, sizeof(double) * n, stream) != 0 || rt_sync(stream) != 0) {
+            snprintf(s->err, sizeof s->err, "pve_reset_poisson: could not set up the %zu-byte clock table", sizeof(double) * n);
+            rt_free(s->clock_dev); rt_free(s->pend_dev);
+            s->clock_dev = nullptr; s->pend_dev = nullptr;
+            rc = PVE_ECUDA;
+        }
+        free(clock);
+        if (rc != PVE_OK) return rc;
+    }
+    PvePoisson &A = s->poi;
+    A.clock = s->clock_dev;
+    A.pend = s->pend_dev;
+    A.mean = 3600.0 / p->rate_veh_per_hour;
+    A.min_headway = p->min_headway;
+    A.key0 = (uint32_t)(p->seed & 0xFFFFFFFFu);
+    A.key1 = (uint32_t)(p->seed >> 32);
+    A.first_env = (uint32_t)p->first_env;
+    A.nlane = s->lane_num;
+    s->poisson = 1;
+    s->spawn_tick = nullptr;
+    s->prm.K = 0;
+    s->prm4.K = 0;
+    return reset_state(s, warmup, warmup != 0, stream);
 }
 
 int32_t pve_step(pve_scene *s, const float *actions_dev, const pve_outputs *out_dev, void *stream_) {
@@ -1250,10 +1355,12 @@ int32_t pve_set_state(pve_scene *s, const pve_state_view *in, void *stream_) {
     RT_CHECK(s, rt_copy(s->st.meta, in->meta, sizeof(pve_veh_meta) * nv, stream));
     RT_CHECK(s, rt_copy(s->st.row0[s->phase], in->row0, sizeof(float) * nv * PVE_OBS_W, stream));
 #ifndef PVE_HOST_EMULATION
-    pve_recount_kernel<<<(B + 127) / 128, 128, 0, stream>>>(s->st, s->spawn_tick, B, s->cfg.veh_cap, s->prm.K);
+    if (s->poisson) pve_recount_kernel<true><<<(B + 127) / 128, 128, 0, stream>>>(s->st, s->poi, B, s->cfg.veh_cap, 0);
+    else pve_recount_kernel<false><<<(B + 127) / 128, 128, 0, stream>>>(s->st, s->spawn_tick, B, s->cfg.veh_cap, s->prm.K);
     RT_CHECK(s, cudaGetLastError());
 #else
-    emul_recount(s->st, s->spawn_tick, B, s->cfg.veh_cap, s->prm.K);
+    if (s->poisson) emul_recount<true>(s->st, s->poi, B, s->cfg.veh_cap, 0);
+    else emul_recount<false>(s->st, s->spawn_tick, B, s->cfg.veh_cap, s->prm.K);
 #endif
     s->next_total = -1;
     s->order_age = -1;

@@ -76,6 +76,8 @@ static inline int pve_emul_atomic_add(int *p, int v) { int o = *p; *p = o + v; r
 #define PVE_RESTRICT __restrict__
 #endif
 
+#include "arrivals.cuh"
+
 struct alignas(16) pve_v4 { uint32_t x, y, z, w; };
 struct alignas(16) pve_d2 { double x, y; };
 
@@ -650,10 +652,12 @@ PVE_DEV float pve_reward(double vm, double aspan, double p, double v, double jr,
  * one tick of intersection b
  * ------------------------------------------------------------------------------------------- */
 /* SRC: also write pve_outputs.nbr_src.  A template flag, not a run-time test: with the code present but switched off
- * the default kernel measured 2-4 % slower (different register allocation), so it exists in its own instantiation. */
-template <int NT, int VC, int AC, bool SRC = false>
+ * the default kernel measured 2-4 % slower (different register allocation), so it exists in its own instantiation.
+ * POI: the arrivals come from the Poisson stream (arrivals.cuh, `arr` is a PvePoisson) instead of the spawn table
+ * (`arr` is the table); a template flag for the same reason. */
+template <int NT, int VC, int AC, bool SRC = false, bool POI = false>
 PVE_DEV void pve_step_block(const PveParams &P, const PveState &S, const pve_outputs &O,
-                            const int32_t *PVE_RESTRICT spawn_tick, const float *PVE_RESTRICT actions,
+                            const typename PveArrivalsT<POI>::type arr, const float *PVE_RESTRICT actions,
                             const int phase, const int b, unsigned char *smem, const uint8_t *skip_class) {
     typedef PveLayout<VC, AC> L;
     /* after phase G1 threads [0, NS) ("team") finish the tick, threads [NS, NT) ("movers") evaluate the rewards and
@@ -1336,8 +1340,14 @@ PVE_DEV void pve_step_block(const PveParams &P, const PveState &S, const pve_out
                 if (sp_i) {
                     const int rec = (int)hdr->veh_rec[i] + 1;                    /* TIS:430 */
                     hdr->veh_rec[i] = (uint16_t)rec;
-                    hdr->next_spawn[i] = (rec < P.K) ? spawn_tick[((size_t)b * P.K + rec) * PVE_NLANE + i]
-                                                     : PVE_NEVER;
+                    if constexpr (POI) {
+                        double *const pend = arr.pend + (size_t)b * PVE_NLANE + i;
+                        double T = *pend;
+                        hdr->next_spawn[i] = pve_next_arrival(arr, b, i, rec, T, &T);
+                        *pend = T;
+                    } else {
+                        hdr->next_spawn[i] = (rec < P.K) ? arr[((size_t)b * P.K + rec) * PVE_NLANE + i] : PVE_NEVER;
+                    }
                 }
                 hdr->lane_n[i] = (uint8_t)(surv_i + sp_i);
                 if (i == PVE_NLANE - 1) {            /* last in serial order: nobody reads hdr->tick after it */

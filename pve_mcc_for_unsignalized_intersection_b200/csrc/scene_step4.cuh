@@ -204,9 +204,9 @@ PVE_DEV void pve8_world_xy(const Pve4Params &P, double p, int i, int m, double *
 
 /* one tick of intersection b.  rows_cur: the stored rows (indexed by the vehicle slots of the tick's start, rewritten at
  * the end for the next tick); rows_new: scratch for the rows computed this tick (same indexing). */
-template <int NLN, class SMEM>      /* lane_num: 4 or 8; SMEM: Pve4SmemT<64> or <128> */
+template <int NLN, bool POI, class SMEM>      /* lane_num: 4 or 8; POI: Poisson arrivals (see pve_step_block); SMEM: Pve4SmemT<64> or <128> */
 PVE_DEV void pve4_step_block(const Pve4Params &P, const PveState &S, const pve_outputs &O,
-                             const int32_t *PVE_RESTRICT spawn_tick, const uint8_t *PVE_RESTRICT draws,
+                             const typename PveArrivalsT<POI>::type arr, const uint8_t *PVE_RESTRICT draws,
                              const float *PVE_RESTRICT actions, const int b, SMEM &M, const int64_t obase) {
     constexpr int PVE4_NLX = NLN;
     const size_t vbase = (size_t)b * (size_t)P.VC;
@@ -466,6 +466,10 @@ PVE_DEV void pve4_step_block(const Pve4Params &P, const PveState &S, const pve_o
                     if (NLN == 4) {
                         M.spawn_int[i] = M.h.pad_[0] % 3;         /* TIS:387: intention_re % 3 */
                         M.h.pad_[0] = (uint8_t)((M.h.pad_[0] + 1) % 3);
+                    } else if constexpr (POI) {                   /* TIS:390: the draw of the record is w2 & 1 of its block */
+                        uint32_t w[4];
+                        pve_arrival_block(arr, b, i, M.h.veh_rec[i], w);
+                        M.spawn_int[i] = P.int8[i][w[2] & 1];
                     } else {                                      /* TIS:390: intention[i][random.randint(0, 1)], the draw is an input */
                         const int dr = draws ? (int)(draws[((size_t)b * P.K + M.h.veh_rec[i]) * PVE_NLANE + i] & 1) : 0;
                         M.spawn_int[i] = P.int8[i][dr];
@@ -474,7 +478,14 @@ PVE_DEV void pve4_step_block(const Pve4Params &P, const PveState &S, const pve_o
                     ++pos; ++cnt; ++granted;
                     const int rec = (int)M.h.veh_rec[i] + 1;      /* TIS:430 */
                     M.h.veh_rec[i] = (uint16_t)rec;
-                    M.h.next_spawn[i] = (rec < P.K) ? spawn_tick[((size_t)b * P.K + rec) * PVE_NLANE + i] : PVE_NEVER;
+                    if constexpr (POI) {
+                        double *const pend = arr.pend + (size_t)b * PVE_NLANE + i;
+                        double T = *pend;
+                        M.h.next_spawn[i] = pve_next_arrival(arr, b, i, rec, T, &T);
+                        *pend = T;
+                    } else {
+                        M.h.next_spawn[i] = (rec < P.K) ? arr[((size_t)b * P.K + rec) * PVE_NLANE + i] : PVE_NEVER;
+                    }
                 } else M.h.overflow += 1;
             }
             M.h.lane_n[i] = (uint8_t)cnt;

@@ -7,7 +7,10 @@ import torch.distributed as dist
 
 
 def shard_range(n_total, rank, world):
-    """Contiguous block [lo, hi) of intersections owned by ``rank`` (sizes differ by at most one)."""
+    """Contiguous block [lo, hi) of intersections owned by ``rank`` (sizes differ by at most one).
+
+    With device-generated arrivals a rank passes ``first_env=lo`` to ``BatchedScene.reset_poisson``: the stream is keyed
+    by the global intersection index, so every intersection sees the same traffic however the batch is sharded."""
     base, rem = divmod(int(n_total), int(world))
     lo = rank * base + min(rank, rem)
     return lo, lo + base + (1 if rank < rem else 0)

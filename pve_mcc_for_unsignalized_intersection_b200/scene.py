@@ -279,6 +279,30 @@ class BatchedScene:
         self._check(self.lib.pve_reset(self._h, self._spawn.data_ptr(), ticks.shape[1], int(bool(warmup)),
                                        self._stream()))
 
+    def reset_poisson(self, rate_veh_per_hour, seed, min_headway=1.0, warmup=True, first_env=0):
+        """A new episode whose arrivals the step kernels generate on the device (``pve_reset_poisson``): per lane a
+        Poisson stream with headways ``max(min_headway, Exp(mean = 3600 / rate_veh_per_hour))`` -- the distribution of
+        ``synthetic_arrivals`` -- drawn from Philox with ``seed`` and the global intersection index
+        ``first_env + b``.  No spawn table is built or kept, so an episode of any length costs O(B) memory, and a new
+        episode with fresh traffic is one call with another seed.  ``arrivals.poisson_arrivals`` returns the same
+        traffic as arrays.  With ``lane_num=8`` the intention draws come from the same stream.  A later ``reset`` with
+        a table goes back to table mode."""
+        rate, min_headway = float(rate_veh_per_hour), float(min_headway)
+        seed, first_env = int(seed), int(first_env)
+        if not (np.isfinite(rate) and rate > 0):
+            raise ValueError("rate_veh_per_hour must be finite and > 0, got %r" % rate_veh_per_hour)
+        if not (np.isfinite(min_headway) and min_headway > 0):
+            raise ValueError("min_headway must be finite and > 0, got %r" % min_headway)
+        if not 0 <= seed < 2**64:
+            raise ValueError("seed must be in [0, 2**64), got %r" % seed)
+        if first_env < 0 or first_env + self.B > 2**32:
+            raise ValueError("first_env must be >= 0 with first_env + n_envs <= 2**32, got %r" % first_env)
+        if self.cfg.deltaT != 0.1:
+            raise ValueError("Poisson arrivals use the reference's 0.1 s clock (deltaT=%r)" % self.cfg.deltaT)
+        p = N.PvePoisson(seed, rate, min_headway, first_env)
+        self._check(self.lib.pve_reset_poisson(self._h, C.byref(p), int(bool(warmup)), self._stream()))
+        self._spawn = None           # the handle no longer reads the table
+
     # ---- step x V + scene_update + delete_vehicle ------------------------------------------
     def step(self, actions):
         """``actions``: float32 ``[B, veh_cap]`` on the scene's device; slot order is (lane, j), the
