@@ -137,7 +137,9 @@ typedef struct pve_outputs {
      * (get_state copies whole stored rows, TIS:1330-1334, Q3): -1 = the all-zero row; 0 .. 0x3FFF = row 0 of agent
      * g' of the same intersection THIS tick (output row agent_offset[b] + g'; entry 0 is the agent itself);
      * 0x4000 | k = the row stored LAST tick for vehicle slot k of the same intersection (slot order before this
-     * tick's removals).  Entry 7 is padding (-1).  Lets a consumer evaluate a network once per distinct row. */
+     * tick's removals; pve_row0_prev_dev until the next step).  Entry 7 is padding (-1).  Lets a consumer evaluate a
+     * network once per distinct row.  Every lane_num (12, 8, 4) writes it, with the same codes; a 0x4000 code always
+     * names the slot of a vehicle that is an agent of this tick. */
     int16_t *nbr_src;
     /* optional (may be null): [out_cap] pve_agent_record, the per-agent scalars of a row in ONE 16-byte record --
      * what a host-side consumer needs of reward / ids / cpv / status / jerk_sum at 16 instead of 29 bytes per agent
@@ -274,6 +276,10 @@ int32_t pve_get_state(pve_scene *s, const pve_state_view *out, void *stream);
 
 /* device views for a device-side actor: stored row 0 of every slot, and the packed meta */
 const float *pve_row0_dev(const pve_scene *s);
+/* the other row buffer: after a step, the stored rows that step read (slot order of its start), which the 0x4000 codes of
+ * pve_outputs.nbr_src name.  12 lanes: after every step; lane_num 4 / 8: after a step that wrote nbr_src.  Valid until
+ * the next step, reset or set_state. */
+const float *pve_row0_prev_dev(const pve_scene *s);
 const pve_veh_meta *pve_meta_dev(const pve_scene *s);
 const pve_env_header *pve_hdr_dev(const pve_scene *s);
 
@@ -392,8 +398,11 @@ int32_t pve_nstep_push(pve_nstep *f, const pve_outputs *out_dev, double gamma, p
                        pve_critic *target_critic, void *stream);
 /* The same tick with the scene at hand and out_dev->nbr_src filled in by the step: the target actor is evaluated once
  * per distinct row (this tick's agent rows + the referenced rows stored last tick + the zero row) instead of on all
- * 7 rows of every observation, and the 7 actions are gathered through nbr_src.  Results are identical (the network
- * sees the same row contents).  Must be called before the scene's next step (last tick's rows are still in place). */
+ * 7 rows of every observation, and the 7 actions are gathered through nbr_src.  The network sees the same row
+ * contents, so results are bit-identical to pve_nstep_push when both run the same network kernels (PVE_ACTOR_IMPL /
+ * PVE_CRITIC_IMPL set); by default each call picks its kernel by its own row count, and the zero row's action is
+ * computed once on one row, so the two may differ within the networks' tolerance.  Every lane_num (12, 8, 4).  Must be called before the scene's next step (last tick's
+ * rows are still in place: pve_row0_prev_dev). */
 int32_t pve_nstep_push_scene(pve_nstep *f, pve_scene *s, const pve_outputs *out_dev, double gamma,
                              pve_actor *target_actor, pve_critic *target_critic, void *stream);
 /* main.py:243-266 for one tick from its FACTORED observation (factored folders only; otherwise, or when one of

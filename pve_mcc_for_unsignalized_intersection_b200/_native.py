@@ -87,7 +87,7 @@ def load_library(path=None):
     lib.pve_next_agent_total.restype = i64
     lib.pve_set_state.argtypes = [vp, C.POINTER(PveStateView), vp]
     lib.pve_get_state.argtypes = [vp, C.POINTER(PveStateView), vp]
-    for name in ("pve_row0_dev", "pve_meta_dev", "pve_hdr_dev", "pve_env_stats_dev"):
+    for name in ("pve_row0_dev", "pve_row0_prev_dev", "pve_meta_dev", "pve_hdr_dev", "pve_env_stats_dev"):
         getattr(lib, name).argtypes = [vp]
         getattr(lib, name).restype = vp
     lib.pve_smem_bytes.argtypes = [vp]

@@ -217,7 +217,7 @@ __global__ void pve_classify_kernel(PveState S, int B) {
 
 /* ---- lane_num = 4 / 8 (scene_step4.cuh): one warp per intersection, PVE4_WARPS intersections per CTA -------------- */
 #define PVE4_WARPS 4
-template <int NLN, int LC, bool POI>
+template <int NLN, int LC, bool POI, bool SRC>
 __global__ void __launch_bounds__(32 * PVE4_WARPS)
 pve4_step_kernel(const Pve4Params P, const PveState S, const pve_outputs O, const typename PveArrivalsT<POI>::type spawn_tick,
                  const uint8_t *draws, const float *actions, const int64_t *off4) {
@@ -225,7 +225,7 @@ pve4_step_kernel(const Pve4Params P, const PveState S, const pve_outputs O, cons
     const int b = (int)blockIdx.x * PVE4_WARPS + (int)(threadIdx.x >> 5);
     if (b >= P.B) return;
     Pve4SmemT<LC> &M = ((Pve4SmemT<LC> *)pve_smem)[threadIdx.x >> 5];
-    pve4_step_block<NLN, POI>(P, S, O, spawn_tick, draws, actions, b, M, off4[b]);
+    pve4_step_block<NLN, POI, SRC>(P, S, O, spawn_tick, draws, actions, b, M, off4[b]);
 }
 
 /* exclusive prefix of the agent counts -> first output row of every intersection (one CTA; B is small on this path) */
@@ -427,8 +427,9 @@ static void emul_stats(PveState S, int B, double *out) {
  * =========================================================================================== */
 static void set_rotation(pve_scene *s) {
     const int G = s->n_groups;
-    s->st.n_ctrl = s->n_ctrl_buf[s->phase];
-    s->st.n_ctrl_next = s->n_ctrl_buf[s->phase ^ 1];
+    const int nc = s->lane_num == 12 ? s->phase : 0;      /* lane_num 4 / 8: one buffer, see launch_step4 */
+    s->st.n_ctrl = s->n_ctrl_buf[nc];
+    s->st.n_ctrl_next = s->n_ctrl_buf[nc ^ 1];
     s->st.gs_read = s->gsum + (size_t)(s->rot % 3) * G;
     s->st.gs_acc = s->gsum + (size_t)((s->rot + 1) % 3) * G;
     s->st.gs_zero = s->gsum + (size_t)((s->rot + 2) % 3) * G;
@@ -569,43 +570,51 @@ static cudaError_t launch_dual_any(pve_scene *s, const float *actions, const pve
 #endif
 
 #ifndef PVE_HOST_EMULATION
-/* lane_num = 4 / 8: the step kernel of one arrival source */
-template <bool POI>
-static cudaError_t launch_kernel4(pve_scene *s, const float *actions, const pve_outputs &O, pve_stream_t stream) {
+/* lane_num = 4 / 8: the step kernel of one arrival source; SRC: the instantiation that writes pve_outputs.nbr_src.
+ * S holds the stored rows of the tick's start in row0[0] (see pve4_step_block). */
+template <bool POI, bool SRC>
+static cudaError_t launch_kernel4(pve_scene *s, const PveState &S, const float *actions, const pve_outputs &O, pve_stream_t stream) {
     static bool attr_set[16] = {false};
     /* capacity class 64 (lists and vehicle slots of <= 64 entries): half the shared memory, twice the resident warps */
     const bool small = s->prm.VC <= 64;
     const size_t smem = (small ? sizeof(Pve4SmemT<64>) : sizeof(Pve4SmemT<128>)) * PVE4_WARPS;
     cudaError_t e;
     if (!attr_set[s->device & 15]) {
-        if ((e = cudaFuncSetAttribute(pve4_step_kernel<4, 128, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<128>) * PVE4_WARPS))) != cudaSuccess) return e;
-        if ((e = cudaFuncSetAttribute(pve4_step_kernel<8, 128, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<128>) * PVE4_WARPS))) != cudaSuccess) return e;
-        if ((e = cudaFuncSetAttribute(pve4_step_kernel<4, 64, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<64>) * PVE4_WARPS))) != cudaSuccess) return e;
-        if ((e = cudaFuncSetAttribute(pve4_step_kernel<8, 64, POI>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<64>) * PVE4_WARPS))) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(pve4_step_kernel<4, 128, POI, SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<128>) * PVE4_WARPS))) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(pve4_step_kernel<8, 128, POI, SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<128>) * PVE4_WARPS))) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(pve4_step_kernel<4, 64, POI, SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<64>) * PVE4_WARPS))) != cudaSuccess) return e;
+        if ((e = cudaFuncSetAttribute(pve4_step_kernel<8, 64, POI, SRC>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(Pve4SmemT<64>) * PVE4_WARPS))) != cudaSuccess) return e;
         attr_set[s->device & 15] = true;
     }
     const int grid = (s->cfg.n_envs + PVE4_WARPS - 1) / PVE4_WARPS;
     const typename PveArrivalsT<POI>::type arr = arrivals_arg<POI>(s);
     if (s->lane_num == 4 && small)
-        pve4_step_kernel<4, 64, POI><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, arr, nullptr, actions, s->off4);
+        pve4_step_kernel<4, 64, POI, SRC><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, S, O, arr, nullptr, actions, s->off4);
     else if (s->lane_num == 4)
-        pve4_step_kernel<4, 128, POI><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, arr, nullptr, actions, s->off4);
+        pve4_step_kernel<4, 128, POI, SRC><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, S, O, arr, nullptr, actions, s->off4);
     else if (small)
-        pve4_step_kernel<8, 64, POI><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, arr, s->draws, actions, s->off4);
+        pve4_step_kernel<8, 64, POI, SRC><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, S, O, arr, s->draws, actions, s->off4);
     else
-        pve4_step_kernel<8, 128, POI><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, s->st, O, arr, s->draws, actions, s->off4);
+        pve4_step_kernel<8, 128, POI, SRC><<<grid, 32 * PVE4_WARPS, smem, stream>>>(s->prm4, S, O, arr, s->draws, actions, s->off4);
     return cudaGetLastError();
 }
 #endif
 
-/* lane_num = 4 / 8: offsets, the step, and the group sums that pve_next_agent_total reads */
+/* lane_num = 4 / 8: offsets, the step, and the group sums that pve_next_agent_total reads.  The stored rows are
+ * row0[phase].  A step that writes nbr_src leaves them untouched, writes the next tick's rows into row0[phase ^ 1] and
+ * flips the phase, so that row0[phase ^ 1] holds the rows it read until the next step (as on 12 lanes); a step without
+ * nbr_src rewrites row0[phase] in place.  n_ctrl is rewritten in place too: it does not follow the phase here. */
 static int32_t launch_step4(pve_scene *s, const float *actions, const pve_outputs &O, pve_stream_t stream) {
     const int B = s->cfg.n_envs;
+    const bool src = O.nbr_src != nullptr;      /* check_factored refuses the other SRC outputs on 4 / 8 lanes */
+    PveState S = s->st;
+    S.row0[0] = s->st.row0[s->phase]; S.row0[1] = s->st.row0[s->phase ^ 1];
 #ifndef PVE_HOST_EMULATION
     if (s->profiling) RT_CHECK(s, cudaEventRecord(s->ev[0], stream));
     pve4_offsets_kernel<<<1, 1024, 0, stream>>>(s->st.n_ctrl, s->off4, B);
     RT_CHECK(s, cudaGetLastError());
-    RT_CHECK(s, (s->poisson ? launch_kernel4<true>(s, actions, O, stream) : launch_kernel4<false>(s, actions, O, stream)));
+    if (s->poisson) RT_CHECK(s, (src ? launch_kernel4<true, true>(s, S, actions, O, stream) : launch_kernel4<true, false>(s, S, actions, O, stream)));
+    else RT_CHECK(s, (src ? launch_kernel4<false, true>(s, S, actions, O, stream) : launch_kernel4<false, false>(s, S, actions, O, stream)));
     if (s->profiling) RT_CHECK(s, cudaEventRecord(s->ev[1], stream));
     const int G = s->n_groups;
     pve_gsum_kernel<<<(G + 127) / 128, 128, 0, stream>>>(s->st.n_ctrl, s->gsum, s->gsum + G, s->gsum + 2 * (size_t)G, B, G);
@@ -617,16 +626,21 @@ static int32_t launch_step4(pve_scene *s, const float *actions, const pve_output
     s->off4[B] = run;
     Pve4Smem *M = new (std::nothrow) Pve4Smem;
     if (!M) return PVE_ENOMEM;
+#define STEP4(NLN, POI, ARR, DRAWS)                                                                              \
+    (src ? pve4_step_block<NLN, POI, true>(s->prm4, S, O, ARR, DRAWS, actions, b, *M, s->off4[b])               \
+         : pve4_step_block<NLN, POI, false>(s->prm4, S, O, ARR, DRAWS, actions, b, *M, s->off4[b]))
     for (int b = 0; b < B; ++b) {
         memset(M, 0xA5, sizeof *M);           /* poison: catches reads of unwritten shared memory */
-        if (s->poisson && s->lane_num == 4) pve4_step_block<4, true>(s->prm4, s->st, O, s->poi, nullptr, actions, b, *M, s->off4[b]);
-        else if (s->poisson) pve4_step_block<8, true>(s->prm4, s->st, O, s->poi, nullptr, actions, b, *M, s->off4[b]);
-        else if (s->lane_num == 4) pve4_step_block<4, false>(s->prm4, s->st, O, s->spawn_tick, nullptr, actions, b, *M, s->off4[b]);
-        else pve4_step_block<8, false>(s->prm4, s->st, O, s->spawn_tick, s->draws, actions, b, *M, s->off4[b]);
+        if (s->poisson && s->lane_num == 4) STEP4(4, true, s->poi, nullptr);
+        else if (s->poisson) STEP4(8, true, s->poi, nullptr);
+        else if (s->lane_num == 4) STEP4(4, false, s->spawn_tick, nullptr);
+        else STEP4(8, false, s->spawn_tick, s->draws);
     }
+#undef STEP4
     delete M;
     emul_gsum(s->st.n_ctrl, s->gsum, s->gsum + s->n_groups, s->gsum + 2 * (size_t)s->n_groups, B, s->n_groups);
 #endif
+    if (src) s->phase ^= 1;
     return PVE_OK;
 }
 
@@ -1384,6 +1398,7 @@ int32_t pve_get_state(pve_scene *s, const pve_state_view *out, void *stream_) {
 }
 
 const float *pve_row0_dev(const pve_scene *s) { return s ? s->st.row0[s->phase] : nullptr; }
+const float *pve_row0_prev_dev(const pve_scene *s) { return s ? s->st.row0[s->phase ^ 1] : nullptr; }
 const pve_veh_meta *pve_meta_dev(const pve_scene *s) { return s ? s->st.meta : nullptr; }
 const pve_env_header *pve_hdr_dev(const pve_scene *s) { return s ? s->st.hdr : nullptr; }
 const double *pve_env_stats_dev(const pve_scene *s) { return s ? s->st.stats : nullptr; }

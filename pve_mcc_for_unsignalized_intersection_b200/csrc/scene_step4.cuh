@@ -202,9 +202,33 @@ PVE_DEV void pve8_world_xy(const Pve4Params &P, double p, int i, int m, double *
     else if (a == 2) { *x = -3 * cw; *y = -1 * w; } else { *x = w; *y = -3 * cw; }
 }
 
-/* one tick of intersection b.  rows_cur: the stored rows (indexed by the vehicle slots of the tick's start, rewritten at
- * the end for the next tick); rows_new: scratch for the rows computed this tick (same indexing). */
-template <int NLN, bool POI, class SMEM>      /* lane_num: 4 or 8; POI: Poisson arrivals (see pve_step_block); SMEM: Pve4SmemT<64> or <128> */
+/* SRC: 8 slots of the in-place compaction of column c of the stored rows (pve4_step_block): DOWN = the vehicles that
+ * move down or stay, k = k0 .. k0 + 7; else the ones that move up, k = k0 .. k0 - 7.  The loads of the 8 slots are all
+ * issued before their stores. */
+template <bool DOWN, class SMEM>
+PVE_DEV void pve4_move_rows(const SMEM &M, float *rows_new, const float *rows_cur, const int c, const int k0, const int V) {
+    float val[8];
+    bool mv[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) {
+        const int k = DOWN ? k0 + u : k0 - u;
+        mv[u] = (DOWN ? k < V : k >= 0) && !M.del[k] && (DOWN ? M.newpos[k] <= k : M.newpos[k] > k);
+        if (mv[u]) val[u] = M.done_row[k] ? rows_new[(size_t)k * PVE_OBS_W + c] : rows_cur[(size_t)M.newpos[k] * PVE_OBS_W + c];
+    }
+#pragma unroll
+    for (int u = 0; u < 8; ++u)
+        if (mv[u]) rows_new[(size_t)M.newpos[DOWN ? k0 + u : k0 - u] * PVE_OBS_W + c] = val[u];
+}
+
+/* one tick of intersection b.  The caller passes the stored rows of the tick's start as S.row0[0] and the other buffer as
+ * S.row0[1].  rows_cur: the stored rows (indexed by the vehicle slots of the tick's start); rows_new: the rows computed
+ * this tick (same indexing).
+ *   SRC = false: rows_new is scratch; rows_cur is rewritten at the end for the next tick (slot order after removals).
+ *   SRC = true:  also writes pve_outputs.nbr_src.  rows_cur is only read, so it still holds the rows this tick read when
+ *                the tick ends (pve_nstep_push_scene needs them); rows_new is compacted in place into the stored rows of
+ *                the next tick, and the caller swaps the two buffers.  Both leave the same rows in every slot below the
+ *                new vehicle count. */
+template <int NLN, bool POI, bool SRC, class SMEM>      /* lane_num: 4 or 8; POI: Poisson arrivals (see pve_step_block); SMEM: Pve4SmemT<64> or <128> */
 PVE_DEV void pve4_step_block(const Pve4Params &P, const PveState &S, const pve_outputs &O,
                              const typename PveArrivalsT<POI>::type arr, const uint8_t *PVE_RESTRICT draws,
                              const float *PVE_RESTRICT actions, const int b, SMEM &M, const int64_t obase) {
@@ -402,6 +426,23 @@ PVE_DEV void pve4_step_block(const Pve4Params &P, const PveState &S, const pve_o
                     P4_SYNC;
                     /* ---- reward, collision, bookkeeping of the agent (TIS:293-340) ---- */
                     P4_ONE {
+                        if constexpr (SRC) {      /* pve_outputs.nbr_src: the source of each row copied above */
+                            if (out_ok && O.nbr_src) {
+                                uint32_t w4[4];
+                                w4[0] = (uint32_t)g_out;
+                                for (int q = 1; q < 8; ++q) {
+                                    const int s = q < PVE_OBS_H ? (int)M.nbr[q - 1] : -1;
+                                    uint32_t v = 0xFFFFu;
+                                    if (s >= 0) {
+                                        const int ks = M.lslot[s];
+                                        v = M.done_row[ks] ? (uint32_t)M.outrow[ks] : (0x4000u | (uint32_t)ks);
+                                    }
+                                    if (q & 1) w4[q >> 1] |= v << 16; else w4[q >> 1] = v;
+                                }
+                                pve_v4 nb; nb.x = w4[0]; nb.y = w4[1]; nb.z = w4[2]; nb.w = w4[3];
+                                ((pve_v4 *)O.nbr_src)[obase + g_out] = nb;
+                            }
+                        }
                         M.done_row[k] = 1;
                         const int s0 = M.nbr[0];
                         const int k0 = s0 >= 0 ? (int)M.lslot[s0] : 0;
@@ -580,10 +621,24 @@ PVE_DEV void pve4_step_block(const Pve4Params &P, const PveState &S, const pve_o
                                 | ((uint32_t)(M.lock_a[k] + 1) << 3) | ((uint32_t)M.intent[k] << 5);
             mt.packed = M.step[k] | (c8 << 16) | (fl << 24);
             S.meta[o] = mt;
-            if (M.done_row[k])
+            if (!SRC && M.done_row[k])
                 for (int c = 0; c < PVE_OBS_W; ++c) rows_cur[(size_t)M.newpos[k] * PVE_OBS_W + c] = rows_new[(size_t)k * PVE_OBS_W + c];
         }
     }
+    if constexpr (SRC) {
+        /* rows_new[newpos[k]] = this tick's row of k, or (a survivor that was no agent) what rows_cur holds there, as the
+         * SRC = false branch leaves it.  In place: newpos increases with k, but a vehicle moves down (removals before it)
+         * or up (arrivals on an earlier lane).  A slot a vehicle moves down to was held by a vehicle that moves down or
+         * stays, or by a removed one, and one it moves up to by a vehicle that moves up or by a removed one; so one pass
+         * over the first kind in increasing k and one over the second in decreasing k read every row before a store can
+         * reach it.  Each lane owns one column, so the lanes need no synchronisation. */
+        P4_PAR(c, PVE_OBS_W) {
+            for (int k0 = 0; k0 < V; k0 += 8) pve4_move_rows<true>(M, rows_new, rows_cur, c, k0, V);
+            for (int k0 = V - 1; k0 >= 0; k0 -= 8) pve4_move_rows<false>(M, rows_new, rows_cur, c, k0, V);
+        }
+        P4_SYNC;      /* a spawn slot below may be a slot read above */
+    }
+    float *const rows_next = SRC ? rows_new : rows_cur;
     P4_PAR(i, PVE4_NLX) {
         if (M.spawn[i]) {                                                                         /* TIS:395-427 */
             const int np = M.spawn[i] - 1, it = M.spawn_int[i];
@@ -593,7 +648,7 @@ PVE_DEV void pve4_step_block(const Pve4Params &P, const PveState &S, const pve_o
             mt.uid = M.spawn_uid[i];
             mt.packed = ((uint32_t)(PVE_F_CONTROL | (1u << 3) | ((uint32_t)it << 5))) << 24;
             S.meta[o] = mt;
-            for (int c = 0; c < PVE_OBS_W; ++c) rows_cur[(size_t)np * PVE_OBS_W + c] = 0.f;
+            for (int c = 0; c < PVE_OBS_W; ++c) rows_next[(size_t)np * PVE_OBS_W + c] = 0.f;
         }
     }
     P4_SYNC;

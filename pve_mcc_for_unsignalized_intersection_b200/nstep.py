@@ -186,8 +186,10 @@ class NStepFolder:
 
     def push(self, outputs, gamma, distinct_rows=None):
         """main.py:243-266 for the tick that produced ``outputs`` (a ``StepOutputs``).  Asynchronous.
-        ``distinct_rows``: None = use the scene's neighbour sources when it exports them; False = always evaluate the
-        target actor on all 7 rows of every observation.
+        ``distinct_rows``: None = use the scene's neighbour sources when it exports them (``BatchedScene(
+        neighbour_sources=True)``, any ``lane_num``); False = always evaluate the target actor on all 7 rows of every
+        observation.  With neighbour sources the push reads the rows the step read, so it must come before the scene's
+        next step.
 
         A factored folder reads the factored observation of ``outputs`` (any ``StepOutputs`` with ``row0_out``,
         ``prev_row0`` and ``obs_src``, not only ``scene.out``; ``obs`` is never read) and evaluates the target actor once

@@ -48,6 +48,7 @@ class StepOutputs:
         self.packed = z(out_cap, 4, dt=torch.int32) if records_only else None
         # optional: where each of the 7 observation rows was copied from (include/pve_mcc.h, pve_outputs.nbr_src):
         # -1 zero row; g' = row 0 of agent g' of the same intersection this tick; 0x4000 | k = last tick's row of slot k
+        # (BatchedScene.row0_prev).  Written by every lane_num (12, 8, 4).
         self.nbr_src = z(out_cap, 8, dt=torch.int16) if neighbour_sources else None
         # optional: the factored observation (include/pve_mcc.h, pve_outputs.row0_out / prev_row0 / obs_src): this tick's
         # row 0 of every agent, the row stored for its vehicle when the tick started, and per observation row a code:
@@ -161,7 +162,9 @@ def _pool(threads):
 
 
 class BatchedScene:
-    """B independent 12-lane intersections resident on one GPU."""
+    """B independent intersections resident on one GPU: the 12-lane one, or with ``SceneConfig(lane_num=4 / 8)`` the
+    4- or 8-lane one.  ``neighbour_sources``: the step also writes ``StepOutputs.nbr_src`` (every geometry), which lets
+    ``NStepFolder.push`` evaluate its target actor once per distinct row."""
 
     def __init__(self, n_envs, config=None, veh_cap=128, agent_cap=96, out_cap=None, device="cuda:0",
                  threads=0, _library=None, neighbour_sources=False, factored_obs=False, full_obs=True):
@@ -418,6 +421,12 @@ class BatchedScene:
         """Stored observation row 0 of every vehicle slot, ``[B, veh_cap, 28]`` float32: the actor's
         input for the next tick (``veh["state"][0]``, MAIN:234-240).  Valid until the next ``step``."""
         return self._wrap(self.lib.pve_row0_dev(self._h), (self.B, self.veh_cap, OBS_W), torch.float32, "<f4")
+
+    def row0_prev(self):
+        """The rows the last ``step`` read, ``[B, veh_cap, 28]`` float32 in the slot order of that step's start: what
+        a ``0x4000 | k`` code of ``StepOutputs.nbr_src`` names.  12 lanes: after every step; ``lane_num`` 4 / 8: after a
+        step with ``neighbour_sources``.  Valid until the next ``step``, ``reset`` or ``set_state``."""
+        return self._wrap(self.lib.pve_row0_prev_dev(self._h), (self.B, self.veh_cap, OBS_W), torch.float32, "<f4")
 
     def control_mask(self):
         """``veh["control"]`` of every slot, bool ``[B, veh_cap]`` (slots past the live count are False)."""
