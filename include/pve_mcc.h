@@ -194,11 +194,12 @@ const char *pve_last_error(const pve_scene *s);
 int32_t pve_reset(pve_scene *s, const int32_t *spawn_tick_dev, int32_t K, int32_t warmup, void *stream);
 
 /* A new episode whose traffic the step kernels generate themselves: a Poisson arrival stream per lane, so that no spawn
- * table is built, uploaded or kept (an episode of any length costs O(B) device memory: 96 B per intersection, plus one
+ * table is built, uploaded or kept (an episode of any length costs O(B) device memory: 192 B per intersection, plus one
  * 32 MB clock table per handle allocated by its first Poisson reset).  For global intersection e = first_env + b, lane i
  * and arrival record r = 0, 1, ...: one Philox4x32-10 block with key (seed & 0xffffffff, seed >> 32) and counter
  * (e, i, r, 0) gives w0..w3; u = (((w0 << 21) | (w1 >> 11)) + 1) * 2^-53; the headway is
- * h_r = max(min_headway, -mean * ln(u)) with mean = 3600 / rate_veh_per_hour and ln evaluated by the library's own
+ * h_r = max(min_headway, -mean[b][i] * ln(u)) with mean[b][i] = 3600 / rate[b][i] (float64, on the host; here every
+ * lane's rate is rate_veh_per_hour, pve_reset_poisson_rates takes one per lane) and ln evaluated by the library's own
  * +-x/ series (bit-identical on every build); T_r = T_{r-1} + h_r in float64 (T_{-1} = 0); the spawn tick is the first
  * n whose accumulated 0.1 s clock (SURVEY.md Q8) is >= T_r, PVE_NEVER past 4 000 000 ticks and from record 65 535 on.
  * lane_num = 8: the intention draw of record r is w2 & 1 (no pve_set_intention_draws needed).  The Python
@@ -216,6 +217,14 @@ typedef struct pve_poisson {
  * (see pve_last_error) for a rate or min_headway that is not finite and > 0, a negative first_env, first_env + n_envs
  * > 2^32, or pve_config.dt != 0.1. */
 int32_t pve_reset_poisson(pve_scene *s, const pve_poisson *p, int32_t warmup, void *stream);
+/* pve_reset_poisson with a rate per intersection and lane: rates_host is host memory float64 [n_envs][lane_num] in veh/h,
+ * read during the call; p->rate_veh_per_hour is not read.  Everything else of the stream is the same, so rates that are
+ * all equal give bit for bit the traffic of pve_reset_poisson at that rate.  A handle holding intersections [lo, hi) of
+ * a larger batch passes rates[lo:hi] and first_env = lo.  PVE_EINVAL for a null rates_host, for an entry that is not
+ * finite and > 0 (pve_last_error names its intersection and lane), and for the other arguments as pve_reset_poisson.
+ * A later pve_reset or pve_reset_poisson replaces the rates. */
+int32_t pve_reset_poisson_rates(pve_scene *s, const pve_poisson *p, const double *rates_host, int32_t warmup,
+                                void *stream);
 
 /* lane_num = 8 only, before pve_reset: draws_dev uint8 [B][K][12], draws_dev[b][k][i] in {0, 1} = what the reference's
  * `random.randint(0, 1)` returns for the k-th arrival of lane i (TIS:390: intention = self.intention[i][draw]); K and the

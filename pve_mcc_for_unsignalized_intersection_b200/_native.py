@@ -74,6 +74,7 @@ def load_library(path=None):
     lib.pve_last_error.restype = C.c_char_p
     lib.pve_reset.argtypes = [vp, vp, i32, i32, vp]
     lib.pve_reset_poisson.argtypes = [vp, C.POINTER(PvePoisson), i32, vp]
+    lib.pve_reset_poisson_rates.argtypes = [vp, C.POINTER(PvePoisson), vp, i32, vp]
     lib.pve_set_intention_draws.argtypes = [vp, vp]
     lib.pve_step.argtypes = [vp, vp, C.POINTER(PveOutputs), vp]
     lib.pve_step_host.argtypes = [vp, vp, C.POINTER(PveOutputs), C.POINTER(PveOutputs), i32, vp]

@@ -126,10 +126,12 @@ def poisson_arrivals(n_envs, rate_veh_per_hour, rows, seed, min_headway=1.0, fir
     """The first ``rows`` records of every lane of the stream that ``BatchedScene.reset_poisson`` generates on the device,
     for global intersections ``first_env .. first_env + n_envs - 1``.  Returns ``(seconds, draws)``: float64 arrival
     times ``[n_envs, rows, lanes]`` and the lane_num = 8 intention draws (uint8 in {0, 1}) of the same records.
+    ``rate_veh_per_hour`` is one rate for every lane (``reset_poisson(rate)``) or an array of rates read as
+    ``lane_rates`` reads it (``reset_poisson(rates)``).
 
     Per record ``r`` of lane ``i`` of intersection ``e``: Philox4x32-10 with counter ``(e, i, r, 0)`` and key
     ``(seed & 0xffffffff, seed >> 32)`` gives ``w0..w3``; ``u = (((w0 << 21) | (w1 >> 11)) + 1) * 2**-53``; the headway is
-    ``max(min_headway, -mean * stream_log(u))`` with ``mean = 3600 / rate``; times are the running sums in record order;
+    ``max(min_headway, -mean[b, i] * stream_log(u))`` with ``mean[b, i] = 3600 / rate[b, i]``; times are the running sums in record order;
     the draw is ``w2 & 1``.  ``to_spawn_ticks(seconds)`` gives the spawn ticks the device uses (which also never spawns
     a record past ``MAX_TICK`` or from record ``MAX_REC`` on).  The distribution is that of ``synthetic_arrivals``, the
     random stream is not."""
@@ -140,9 +142,35 @@ def poisson_arrivals(n_envs, rate_veh_per_hour, rows, seed, min_headway=1.0, fir
     w0, w1, w2, _ = philox4x32(e, i, r, np.uint64(0), seed & 0xFFFFFFFF, seed >> 32)
     x = (w0 << np.uint64(21)) | (w1 >> np.uint64(11))
     u = (x + np.uint64(1)).astype(np.float64) * 2.0 ** -53
-    mean = 3600.0 / float(rate_veh_per_hour)
+    if np.ndim(rate_veh_per_hour) == 0:
+        mean = 3600.0 / float(rate_veh_per_hour)
+    else:
+        mean = (3600.0 / lane_rates(rate_veh_per_hour, n_envs, lanes))[:, None, :]
     head = np.maximum(-mean * stream_log(u), float(min_headway))
     return np.add.accumulate(head, axis=1), (w2 & np.uint64(1)).astype(np.uint8)
+
+
+def lane_rates(rates, n_envs, lanes):
+    """Per-lane rates as ``reset_poisson`` and ``poisson_arrivals`` read them: ``[n_envs]`` (one per intersection),
+    ``[lanes]`` (one per lane) or anything else that broadcasts to ``[n_envs, lanes]``.  Returns a C-contiguous float64
+    ``[n_envs, lanes]`` array; raises ``ValueError`` for another shape, for a 1-D array when ``n_envs == lanes`` (one per
+    intersection or one per lane?) and for an entry that is not finite and > 0, naming its intersection and lane."""
+    a = np.asarray(rates, dtype=np.float64)
+    if a.ndim == 1 and a.shape[0] == n_envs:
+        if n_envs == lanes:
+            raise ValueError("%d rates could be one per intersection or one per lane (n_envs == lane_num == %d): pass "
+                             "them as [%d, 1] or [1, %d]" % (lanes, lanes, lanes, lanes))
+        a = a[:, None]                          # one rate per intersection
+    try:
+        a = np.ascontiguousarray(np.broadcast_to(a, (n_envs, lanes)))
+    except ValueError:
+        raise ValueError("rates of shape %s do not broadcast to [n_envs, lane_num] = [%d, %d]"
+                         % (np.shape(rates), n_envs, lanes)) from None
+    bad = ~(np.isfinite(a) & (a > 0))
+    if bad.any():
+        b, i = np.argwhere(bad)[0]
+        raise ValueError("every rate must be finite and > 0; intersection %d, lane %d has %r" % (b, i, a[b, i]))
+    return a
 
 
 def stress_arrivals(n_envs, horizon_s, headway=1.0):

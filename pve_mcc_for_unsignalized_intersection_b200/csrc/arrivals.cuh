@@ -4,7 +4,7 @@
  * For global intersection e = first_env + b, lane i and arrival record r = 0, 1, ...:
  *   w0..w3 = Philox4x32-10(counter (e, i, r, 0), key (seed & 0xffffffff, seed >> 32))
  *   u      = (((w0 << 21) | (w1 >> 11)) + 1) * 2^-53                      in (0, 1]
- *   h_r    = max(min_headway, -mean * pve_log_u(u)),  mean = 3600 / rate_veh_per_hour
+ *   h_r    = max(min_headway, -mean[b][i] * pve_log_u(u)),  mean[b][i] = 3600 / rate[b][i] (float64, on the host)
  *   T_r    = T_{r-1} + h_r (float64, record order, T_{-1} = 0)
  *   spawn tick = the first n with clock[n] >= T_r (clock = the reference's accumulated 0.1 s clock, arrivals.py
  *                reference_clock); PVE_NEVER past PVE_MAX_TICK and from record PVE_MAX_REC on (veh_rec is 16 bits)
@@ -24,7 +24,10 @@
 struct PvePoisson {
     const double *clock;      /* [PVE_MAX_TICK + 1] the reference's accumulated clock, built by the library */
     double *pend;             /* [B][12] arrival time T of record veh_rec[i] of lane i (the one next_spawn[i] is for) */
-    double mean, min_headway; /* 3600 / rate_veh_per_hour, pve_poisson.min_headway */
+    double *mean;             /* [B][12] 3600 / rate of lane i of intersection b (pve_reset_poisson_rates) */
+    double uniform_mean;      /* > 0: pve_reset_poisson's 3600 / rate, which the reset writes to every lane of `mean`;
+                                 0: `mean` holds per-lane values already */
+    double min_headway;       /* pve_poisson.min_headway */
     double clock_last;        /* clock[PVE_MAX_TICK] */
     uint32_t key0, key1;      /* seed & 0xffffffff, seed >> 32 */
     uint32_t first_env;       /* e = first_env + b */
@@ -97,11 +100,11 @@ PVE_HD void pve_arrival_block(const PvePoisson &A, int b, int i, int r, uint32_t
     pve_philox(A.first_env + (uint32_t)b, (uint32_t)i, (uint32_t)r, 0u, A.key0, A.key1, w);
 }
 
-/* the headway h_r of a block */
-PVE_HD double pve_headway(const PvePoisson &A, const uint32_t w[4]) {
+/* the headway h_r of a block of a lane whose mean headway is `mean` (A.mean[b][i]) */
+PVE_HD double pve_headway(const PvePoisson &A, double mean, const uint32_t w[4]) {
     const uint64_t x = ((uint64_t)w[0] << 21) | (uint64_t)(w[1] >> 11);
     const double u = (double)(x + 1) * 1.1102230246251565e-16;          /* 2^-53 */
-    const double h = -A.mean * pve_log_u(u);
+    const double h = -mean * pve_log_u(u);
     return h > A.min_headway ? h : A.min_headway;
 }
 
@@ -123,32 +126,37 @@ PVE_HD int pve_spawn_tick_of(const PvePoisson &A, double T) {
 /* arrival time T_r of record r (r < PVE_MAX_REC), summed from record 0 in record order: what pve_reset_poisson and
  * pve_set_state store as the pending time */
 PVE_HD double pve_arrival_time(const PvePoisson &A, int b, int i, int r) {
+    const double mean = A.mean[(size_t)b * PVE_NLANE + i];
     double T = 0.0;
     uint32_t w[4];
     for (int q = 0; q <= r; ++q) {
         pve_arrival_block(A, b, i, q, w);
-        T = T + pve_headway(A, w);
+        T = T + pve_headway(A, mean, w);
     }
     return T;
 }
 
-/* record `rec` of lane i has just become the next arrival (a spawn, or a reset / set_state): its pending time
- * (T_rec = T_{rec-1} + h_rec when `T_prev` is T_{rec-1}) and its spawn tick */
-PVE_HD int pve_next_arrival(const PvePoisson &A, int b, int i, int rec, double T_prev, double *T_out) {
+/* record `rec` of lane i has just become the next arrival (a spawn, or a reset): *pend goes from T_{rec-1} to
+ * T_rec = T_{rec-1} + h_rec; returns its spawn tick.  `mean` is A.mean[b][i], which the step kernels load before the
+ * call so that the load overlaps the Philox rounds; *pend is read after them (overlapping the log), which keeps the
+ * small 12-lane step kernel within its 64 registers */
+PVE_HD int pve_next_arrival(const PvePoisson &A, int b, int i, int rec, double *pend, double mean) {
     if (rec >= PVE_MAX_REC) return PVE_NEVER;
     uint32_t w[4];
     pve_arrival_block(A, b, i, rec, w);
-    const double T = T_prev + pve_headway(A, w);
-    *T_out = T;
+    const double h = pve_headway(A, mean, w);
+    const double T = *pend + h;
+    *pend = T;
     return pve_spawn_tick_of(A, T);
 }
 
-/* pve_reset_poisson: record 0 becomes lane i's next arrival; lanes past A.nlane never spawn */
+/* pve_reset_poisson(_rates): record 0 becomes lane i's next arrival; lanes past A.nlane never spawn.  A uniform
+ * reset writes the lane's mean here, so it needs neither an allocation nor a launch of its own. */
 PVE_HD int pve_reset_lane(const PvePoisson &A, int b, int i) {
-    double T = 0.0;
-    const int t = i < A.nlane ? pve_next_arrival(A, b, i, 0, 0.0, &T) : PVE_NEVER;
-    A.pend[(size_t)b * PVE_NLANE + i] = T;
-    return t;
+    const size_t q = (size_t)b * PVE_NLANE + i;
+    if (A.uniform_mean > 0) A.mean[q] = A.uniform_mean;
+    A.pend[q] = 0.0;
+    return i < A.nlane ? pve_next_arrival(A, b, i, 0, A.pend + q, A.mean[q]) : PVE_NEVER;
 }
 
 /* pve_set_state: the pending time of record `rec` summed again from record 0 (the same additions in the same order

@@ -84,11 +84,12 @@ struct pve_scene {
 #endif
     int order_age;               /* ticks since the order was refreshed (-1: never) */
     const int32_t *spawn_tick;   /* borrowed */
-    /* Poisson mode (pve_reset_poisson): the step kernels generate the arrivals (arrivals.cuh) instead of reading
-     * spawn_tick; pend_dev / clock_dev are allocated by the first Poisson reset and kept for the handle's lifetime */
+    /* Poisson mode (pve_reset_poisson / _rates): the step kernels generate the arrivals (arrivals.cuh) instead of
+     * reading spawn_tick; pend_dev / clock_dev are allocated by the first Poisson reset and kept for the handle's
+     * lifetime */
     int poisson;
     PvePoisson poi;
-    double *pend_dev;            /* [B][12] */
+    double *pend_dev;            /* [2][B][12]: PvePoisson::pend, then PvePoisson::mean */
     double *clock_dev;           /* [PVE_MAX_TICK + 1] */
     float *actions_dev;          /* staging for pve_step_host */
     double *counters_dev;
@@ -1024,19 +1025,29 @@ int32_t pve_reset(pve_scene *s, const int32_t *spawn_tick_dev, int32_t K, int32_
     return reset_state(s, warmup, warmup && spawn_tick_dev && K > 0, (pve_stream_t)stream_);
 }
 
-int32_t pve_reset_poisson(pve_scene *s, const pve_poisson *p, int32_t warmup, void *stream_) {
+/* pve_reset_poisson (rates == nullptr: every lane at p->rate_veh_per_hour) and pve_reset_poisson_rates (rates: host
+ * [n_envs][lane_num] veh/h); `fn` names the entry point in pve_last_error */
+static int32_t reset_poisson(pve_scene *s, const pve_poisson *p, const double *rates, int32_t warmup, void *stream_,
+                             const char *fn) {
     if (!s) return PVE_EINVAL;
-    if (!p) { snprintf(s->err, sizeof s->err, "pve_reset_poisson: null parameters"); return PVE_EINVAL; }
-    const int B = s->cfg.n_envs;
+    if (!p) { snprintf(s->err, sizeof s->err, "%s: null parameters", fn); return PVE_EINVAL; }
+    const int B = s->cfg.n_envs, nl = s->lane_num;
+    for (size_t q = 0; rates && q < (size_t)B * nl; ++q) {
+        if (!(isfinite(rates[q]) && rates[q] > 0)) {
+            snprintf(s->err, sizeof s->err, "%s: the rate of intersection %zu, lane %zu is %g; every rate must be finite "
+                     "and > 0", fn, q / nl, q % nl, rates[q]);
+            return PVE_EINVAL;
+        }
+    }
     const char *bad = nullptr;
-    if (!(isfinite(p->rate_veh_per_hour) && p->rate_veh_per_hour > 0)) bad = "rate_veh_per_hour must be finite and > 0";
+    if (!rates && !(isfinite(p->rate_veh_per_hour) && p->rate_veh_per_hour > 0)) bad = "rate_veh_per_hour must be finite and > 0";
     else if (!(isfinite(p->min_headway) && p->min_headway > 0))
         bad = "min_headway must be finite and > 0 (an arrival at 0 s would read as table padding)";
     else if (p->first_env < 0) bad = "first_env must be >= 0";
     else if (p->first_env + (int64_t)B > ((int64_t)1 << 32)) bad = "first_env + n_envs must be <= 2^32 (the counter word of e)";
     else if (s->cfg.dt != 0.1) bad = "Poisson arrivals use the reference's 0.1 s clock (pve_config.dt must be 0.1)";
     if (bad) {
-        snprintf(s->err, sizeof s->err, "pve_reset_poisson: %s", bad);
+        snprintf(s->err, sizeof s->err, "%s: %s", fn, bad);
         return PVE_EINVAL;
     }
     pve_stream_t stream = (pve_stream_t)stream_;
@@ -1049,9 +1060,9 @@ int32_t pve_reset_poisson(pve_scene *s, const pve_poisson *p, int32_t warmup, vo
         s->poi.clock_last = clock[n - 1];
         int32_t rc = PVE_OK;
         if (rt_alloc((void **)&s->clock_dev, sizeof(double) * n) != 0 ||
-            rt_alloc((void **)&s->pend_dev, sizeof(double) * PVE_NLANE * (size_t)B) != 0 ||
+            rt_alloc((void **)&s->pend_dev, sizeof(double) * 2 * PVE_NLANE * (size_t)B) != 0 ||
             rt_copy(s->clock_dev, clock, sizeof(double) * n, stream) != 0 || rt_sync(stream) != 0) {
-            snprintf(s->err, sizeof s->err, "pve_reset_poisson: could not set up the %zu-byte clock table", sizeof(double) * n);
+            snprintf(s->err, sizeof s->err, "%s: could not set up the %zu-byte clock table", fn, sizeof(double) * n);
             rt_free(s->clock_dev); rt_free(s->pend_dev);
             s->clock_dev = nullptr; s->pend_dev = nullptr;
             rc = PVE_ECUDA;
@@ -1062,7 +1073,20 @@ int32_t pve_reset_poisson(pve_scene *s, const pve_poisson *p, int32_t warmup, vo
     PvePoisson &A = s->poi;
     A.clock = s->clock_dev;
     A.pend = s->pend_dev;
-    A.mean = 3600.0 / p->rate_veh_per_hour;
+    A.mean = s->pend_dev + PVE_NLANE * (size_t)B;
+    if (rates) {
+        /* the means in float64 on the host, the same division as arrivals.poisson_arrivals; lanes past lane_num never
+         * spawn and keep 0 */
+        double *mean = (double *)calloc((size_t)B * PVE_NLANE, sizeof(double));
+        if (!mean) return PVE_ENOMEM;
+        for (size_t q = 0; q < (size_t)B * nl; ++q) mean[q / nl * PVE_NLANE + q % nl] = 3600.0 / rates[q];
+        const int rc = rt_copy(A.mean, mean, sizeof(double) * PVE_NLANE * (size_t)B, stream) != 0 || rt_sync(stream) != 0;
+        free(mean);
+        if (rc) { snprintf(s->err, sizeof s->err, "%s: could not copy the rates to the device", fn); return PVE_ECUDA; }
+        A.uniform_mean = 0.0;
+    } else {
+        A.uniform_mean = 3600.0 / p->rate_veh_per_hour;
+    }
     A.min_headway = p->min_headway;
     A.key0 = (uint32_t)(p->seed & 0xFFFFFFFFu);
     A.key1 = (uint32_t)(p->seed >> 32);
@@ -1073,6 +1097,18 @@ int32_t pve_reset_poisson(pve_scene *s, const pve_poisson *p, int32_t warmup, vo
     s->prm.K = 0;
     s->prm4.K = 0;
     return reset_state(s, warmup, warmup != 0, stream);
+}
+
+int32_t pve_reset_poisson(pve_scene *s, const pve_poisson *p, int32_t warmup, void *stream) {
+    return reset_poisson(s, p, nullptr, warmup, stream, "pve_reset_poisson");
+}
+
+int32_t pve_reset_poisson_rates(pve_scene *s, const pve_poisson *p, const double *rates_host, int32_t warmup, void *stream) {
+    if (s && !rates_host) {
+        snprintf(s->err, sizeof s->err, "pve_reset_poisson_rates: null rates_host");
+        return PVE_EINVAL;
+    }
+    return reset_poisson(s, p, rates_host, warmup, stream, "pve_reset_poisson_rates");
 }
 
 int32_t pve_step(pve_scene *s, const float *actions_dev, const pve_outputs *out_dev, void *stream_) {

@@ -1341,10 +1341,8 @@ PVE_DEV void pve_step_block(const PveParams &P, const PveState &S, const pve_out
                     const int rec = (int)hdr->veh_rec[i] + 1;                    /* TIS:430 */
                     hdr->veh_rec[i] = (uint16_t)rec;
                     if constexpr (POI) {
-                        double *const pend = arr.pend + (size_t)b * PVE_NLANE + i;
-                        double T = *pend;
-                        hdr->next_spawn[i] = pve_next_arrival(arr, b, i, rec, T, &T);
-                        *pend = T;
+                        const size_t q = (size_t)b * PVE_NLANE + i;
+                        hdr->next_spawn[i] = pve_next_arrival(arr, b, i, rec, arr.pend + q, arr.mean[q]);
                     } else {
                         hdr->next_spawn[i] = (rec < P.K) ? arr[((size_t)b * P.K + rec) * PVE_NLANE + i] : PVE_NEVER;
                     }

@@ -520,10 +520,8 @@ PVE_DEV void pve4_step_block(const Pve4Params &P, const PveState &S, const pve_o
                     const int rec = (int)M.h.veh_rec[i] + 1;      /* TIS:430 */
                     M.h.veh_rec[i] = (uint16_t)rec;
                     if constexpr (POI) {
-                        double *const pend = arr.pend + (size_t)b * PVE_NLANE + i;
-                        double T = *pend;
-                        M.h.next_spawn[i] = pve_next_arrival(arr, b, i, rec, T, &T);
-                        *pend = T;
+                        const size_t q = (size_t)b * PVE_NLANE + i;
+                        M.h.next_spawn[i] = pve_next_arrival(arr, b, i, rec, arr.pend + q, arr.mean[q]);
                     } else {
                         M.h.next_spawn[i] = (rec < P.K) ? arr[((size_t)b * P.K + rec) * PVE_NLANE + i] : PVE_NEVER;
                     }

@@ -10,7 +10,9 @@ def shard_range(n_total, rank, world):
     """Contiguous block [lo, hi) of intersections owned by ``rank`` (sizes differ by at most one).
 
     With device-generated arrivals a rank passes ``first_env=lo`` to ``BatchedScene.reset_poisson``: the stream is keyed
-    by the global intersection index, so every intersection sees the same traffic however the batch is sharded."""
+    by the global intersection index, so every intersection sees the same traffic however the batch is sharded.  With
+    per-intersection or per-lane rates it passes its slice ``rates[lo:hi]`` of the whole batch's ``[n_total, lane_num]``
+    rates as well (``pve_reset_poisson_rates``)."""
     base, rem = divmod(int(n_total), int(world))
     lo = rank * base + min(rank, rem)
     return lo, lo + base + (1 if rank < rem else 0)

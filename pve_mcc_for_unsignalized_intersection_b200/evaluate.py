@@ -48,15 +48,43 @@ def format_report(vehicles, collisions, passed, passed_step_total, jerk_total, l
                              float(passed_step_total) / (passed + 0.0001) * deltaT, jerk_total / passed, lock_total))
 
 
+_TALLIES = ("vehicles", "collisions", "passed", "passed_step_total", "jerk_total", "lock_total")   # format_report's
+
+
 def evaluate_tables(tables, weights, ticks=36000, vm=5, collision_thr=2, device="cuda:0", veh_cap=128,
                     agent_cap=96, progress=None):
     """Closed loop actor + scene on every table of ``tables`` (list of ``[K, 12]`` arrays) for ``ticks``
     ticks.  Returns one dict per table with the quantities of main.py:566-581."""
-    B = len(tables)
+    return _evaluate(len(tables), lambda scene: scene.reset(stack_tables(tables), warmup=True), weights, ticks, vm,
+                     collision_thr, device, veh_cap, agent_cap, progress)
+
+
+def evaluate_poisson(weights, densities=DENSITIES, envs_per_density=64, ticks=36000, seed=0, min_headway=1.0, vm=5,
+                     collision_thr=2, device="cuda:0", veh_cap=192, agent_cap=128, progress=None):
+    """The density sweep of ``batch_test`` on generated traffic: ``envs_per_density`` intersections per density (veh/h
+    and lane), all of one density contiguous, in one scene with one ``reset_poisson`` of per-intersection rates, the
+    closed loop of ``evaluate_tables`` for ``ticks`` ticks.  Returns one dict per density: ``"density"``,
+    ``"intersections"`` (the dicts ``evaluate_tables`` returns, one per intersection), ``"pooled"`` (their sums) and
+    ``"report"`` (``format_report`` of the pooled sums)."""
+    n = int(envs_per_density)
+    rates = np.repeat(np.asarray(densities, dtype=np.float64), n)[:, None]
+    res = _evaluate(len(rates), lambda scene: scene.reset_poisson(rates, seed, min_headway=min_headway, warmup=True),
+                    weights, ticks, vm, collision_thr, device, veh_cap, agent_cap, progress)
+    out = []
+    for k, d in enumerate(densities):
+        per = res[k * n:(k + 1) * n]
+        pooled = {q: sum(r[q] for r in per) for q in _TALLIES}
+        out.append({"density": d, "intersections": per, "pooled": pooled, "report": format_report(**pooled)})
+    return out
+
+
+def _evaluate(B, reset, weights, ticks, vm, collision_thr, device, veh_cap, agent_cap, progress):
+    """``reset(scene)`` on a new scene of ``B`` intersections, then the closed loop; one dict of tallies per
+    intersection."""
     scene = BatchedScene(B, SceneConfig(vm=vm, collision_thr=collision_thr), veh_cap=veh_cap, agent_cap=agent_cap,
                          device=device)
     actor = BatchedActor(weights, device=device)
-    scene.reset(stack_tables(tables), warmup=True)
+    reset(scene)
     dev = scene.device
     acts = torch.empty(B, scene.veh_cap, dtype=torch.float32, device=dev)
     # the tallies of main.py:567-571 (jerks of finished vehicles, lock events, agents with collision > 0) are kept per

@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from . import _native as N
-from .arrivals import to_spawn_ticks
+from .arrivals import lane_rates, to_spawn_ticks
 from .config import NLANE, OBS_H, OBS_W, SceneConfig
 
 
@@ -289,11 +289,21 @@ class BatchedScene:
         ``first_env + b``.  No spawn table is built or kept, so an episode of any length costs O(B) memory, and a new
         episode with fresh traffic is one call with another seed.  ``arrivals.poisson_arrivals`` returns the same
         traffic as arrays.  With ``lane_num=8`` the intention draws come from the same stream.  A later ``reset`` with
-        a table goes back to table mode."""
-        rate, min_headway = float(rate_veh_per_hour), float(min_headway)
-        seed, first_env = int(seed), int(first_env)
-        if not (np.isfinite(rate) and rate > 0):
-            raise ValueError("rate_veh_per_hour must be finite and > 0, got %r" % rate_veh_per_hour)
+        a table goes back to table mode.
+
+        ``rate_veh_per_hour`` is one rate for every lane, or an array-like of rates broadcastable to ``[B, lane_num]``
+        (``[B]``: one per intersection, ``[lane_num]``: one per lane, ``[B, lane_num]``) for ``pve_reset_poisson_rates``;
+        equal rates give the same traffic either way.  A rank holding intersections ``[lo, hi)`` of a larger batch passes
+        ``rates[lo:hi]`` with ``first_env=lo``."""
+        rates = None
+        if np.ndim(rate_veh_per_hour) == 0:
+            rate = float(rate_veh_per_hour)
+            if not (np.isfinite(rate) and rate > 0):
+                raise ValueError("rate_veh_per_hour must be finite and > 0, got %r" % rate_veh_per_hour)
+        else:
+            rates = lane_rates(rate_veh_per_hour, self.B, self.cfg.lane_num)
+            rate = 0.0                          # pve_reset_poisson_rates does not read it
+        min_headway, seed, first_env = float(min_headway), int(seed), int(first_env)
         if not (np.isfinite(min_headway) and min_headway > 0):
             raise ValueError("min_headway must be finite and > 0, got %r" % min_headway)
         if not 0 <= seed < 2**64:
@@ -303,7 +313,11 @@ class BatchedScene:
         if self.cfg.deltaT != 0.1:
             raise ValueError("Poisson arrivals use the reference's 0.1 s clock (deltaT=%r)" % self.cfg.deltaT)
         p = N.PvePoisson(seed, rate, min_headway, first_env)
-        self._check(self.lib.pve_reset_poisson(self._h, C.byref(p), int(bool(warmup)), self._stream()))
+        if rates is None:
+            self._check(self.lib.pve_reset_poisson(self._h, C.byref(p), int(bool(warmup)), self._stream()))
+        else:
+            self._check(self.lib.pve_reset_poisson_rates(self._h, C.byref(p), rates.ctypes.data, int(bool(warmup)),
+                                                         self._stream()))
         self._spawn = None           # the handle no longer reads the table
 
     # ---- step x V + scene_update + delete_vehicle ------------------------------------------
